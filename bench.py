@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
                     [--shape l4|l3|mbv3|vit|eurosat] [--R 1|2] [--dtype fp32|bf16] [--batch 256] [--no-sweep]
+                    [--dump-outputs DIR]
 
 One "step" = one forward + one backward of the NFP layer (cosine, pad = R, reflect) over one batch
 of synthetic feature maps.  Default workload: BASELINE.json configs[1], ResNet18 layer4 maps
@@ -14,9 +15,11 @@ of synthetic feature maps.  Default workload: BASELINE.json configs[1], ResNet18
                   HOST pinned buffers: H2D of x and grad_y and D2H of y and grad_x inside the timed region.
 * ``roofline`` -- the dominant kernel (backward): algorithmic bytes per launch / its average launch
                   duration (CUDA events around a graph of back-to-back launches on rotating buffers).
-* ``cpu_baseline`` -- the reference's own operator (staged unmodified under baseline/_ref by build()) on the host
-                  cores; the conv-form port (oracle/nfp_convform.py) only if those files are missing.
+* ``cpu_baseline`` -- the reference's own operator (NFP_REFERENCE_ROOT, or the copy build() staged unmodified under
+                  oracle/_ref) on the host cores; the conv-form port (oracle/nfp_convform.py) only if those files are missing.
 * ``--impl reference`` -- that CPU path as its own arm, same metric / config.
+* ``--dump-outputs DIR`` -- y and grad_x of the last timed step as DIR/*.npy (seeded inputs: two builds can be
+                  compared output for output).
 
 Multi-GPU (torchrun): the batch dimension is sharded, one process per GPU, no data-path collective;
 weak scaling (B maps per GPU per step); time = max over ranks.
@@ -70,6 +73,7 @@ def parse_args():
     ap.add_argument("--train-batch", type=int, default=256, help="images per GPU per training step")
     ap.add_argument("--train-steps", type=int, default=20)
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="CPU-baseline budget (seconds of CPU work)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write y and grad_x of the last timed step as DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -450,8 +454,8 @@ def cpu_model_name():
 def cpu_ref_setup(C, H, W, R, dtype_name, B):
     """-> (callable running one fwd+bwd of the CPU arm on B maps, kind, description).
 
-    kind "reference": the UNMODIFIED reference operator (models/pooling/nfp.py, staged by __graft_entry__.build()
-    under the git-ignored baseline/_ref/ or read from /root/reference) -- NFPPooling(C, R, 'cosine', padding=R) forward
+    kind "reference": the UNMODIFIED reference operator (models/pooling/nfp.py, read from NFP_REFERENCE_ROOT or from the
+    copy __graft_entry__.build() staged under the git-ignored oracle/_ref/) -- NFPPooling(C, R, 'cosine', padding=R) forward
     + autograd backward.  kind "port": the same ATen operator sequence restated (oracle/nfp_convform.py), used only
     when the reference files are not there.  (bench.py's CPU legs are the only product-side use of oracle/.)"""
     tdtype = torch.float32 if dtype_name == "fp32" else torch.bfloat16
@@ -469,7 +473,7 @@ def cpu_ref_setup(C, H, W, R, dtype_name, B):
             y = layer(xr)
             y.backward(g)
             return y, xr.grad
-        return run, "reference", ("the unmodified reference NFPPooling (models/pooling/nfp.py via baseline/_ref): "
+        return run, "reference", ("the unmodified reference NFPPooling (models/pooling/nfp.py via oracle/ref_loader): "
                                   "reflect-pad + one-hot depthwise convs + F.cosine_similarity + autograd")
     from oracle.nfp_convform import ConvFormCosineNFP, forward_backward
     layer = ConvFormCosineNFP(C, R=R, padding=R).to(tdtype)
@@ -546,6 +550,28 @@ def run_reference_arm(args, C, H, W, where):
     emit(line)
 
 
+DUMP_BYTES = 64 * 10**6
+
+
+def dump_outputs(out_dir, lb, step):
+    """What a caller of the timed path receives from step `step` of a window (LayerBench.step): y of its forward and
+    grad_x of its backward, as float32 DIR/y.npy and DIR/grad_x.npy.  Above DUMP_BYTES in all, the same seeded sample
+    of batch rows is kept from both, their indices in DIR/batch_rows.npy."""
+    import numpy as np
+    i = step % lb.nbuf
+    arrays = {"y": lb.y[i], "grad_x": lb.gx[lb.cold(i)]}
+    n = min(lb.B, DUMP_BYTES // (sum(a[0].numel() for a in arrays.values()) * 4))
+    if n == 0:
+        raise SystemExit(f"--dump-outputs: one batch row of y and grad_x is larger than {DUMP_BYTES} bytes")
+    os.makedirs(out_dir, exist_ok=True)
+    if n < lb.B:
+        rows = torch.randperm(lb.B, generator=torch.Generator().manual_seed(0))[:n].sort().values
+        arrays = {k: a[rows.to(a.device)] for k, a in arrays.items()}
+        np.save(os.path.join(out_dir, "batch_rows.npy"), rows.double().numpy())
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.float().cpu().numpy())
+
+
 # ----------------------------------------------------------------------------------------------
 _JSON_OUT = None
 
@@ -572,6 +598,8 @@ def main():
     claim_stdout()
     C, H, W, where = SHAPES[args.shape]
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs dumps the b200 arm; the reference arm sizes its batch by timing")
         run_reference_arm(args, C, H, W, where)
         return
 
@@ -624,6 +652,8 @@ def main():
     t_step_total = lb.timed(lb.step, args.steps, args.warmup, sampler, "timed", barrier, windows=args.windows,
                             reduce=max_over_ranks)
     window_ms = [t * 1e3 for t in lb.last_windows]
+    if args.dump_outputs and rank == 0:   # before the passes below reuse the buffers
+        dump_outputs(args.dump_outputs, lb, args.steps - 1)
     value = world * args.steps * B / t_step_total
     # ---- per-kernel launch durations (same rotation, back-to-back launches of one kernel) ---------
     sampler_tag = "kernels"

@@ -123,7 +123,7 @@ def make_model(cfg, device, impl="b200"):
     if impl == "b200":
         import neighbour_feature_pooling_b200 as nfpb
         pool = nfpb.nfp_pooling(Params=Params)
-    else:  # CPU baseline: the reference's own nfp_pooling (staged under baseline/_ref), else its conv-form port
+    else:  # CPU baseline: the reference's own nfp_pooling (staged under oracle/_ref), else its conv-form port
         from oracle import ref_loader
         if ref_loader.reference_available():
             _, ref_pool = ref_loader.load_reference()

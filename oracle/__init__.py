@@ -7,7 +7,7 @@ baseline -- never as a fallback for the CUDA path.
 
 Parity status: **pinned**.  The reference ships no tests or golden vectors
 (SURVEY.md section 4), so the oracle is pinned by executing the reference's own
-Python modules in the build container (``oracle/check_against_reference.py``)
+Python modules where a checkout of it exists (``oracle/check_against_reference.py``)
 and by the committed fixtures under ``tests/golden/`` generated from the
 reference by ``oracle/make_golden.py``.
 """

@@ -1,8 +1,8 @@
 """TEST INFRASTRUCTURE ONLY -- pin the oracle against the reference itself.
 
-Run in the build container (needs ``/root/reference``):
+Needs a checkout of the original project:
 
-    python -m oracle.check_against_reference
+    NFP_REFERENCE_ROOT=/path/to/Neighbour_Feature_Pooling python -m oracle.check_against_reference
 
 For every measure x geometry case it executes the unmodified reference module
 (forward and autograd backward, fp64) and the oracle restatement on the same

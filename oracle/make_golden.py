@@ -1,8 +1,8 @@
 """TEST INFRASTRUCTURE ONLY -- generate golden vectors from the reference.
 
-Run in the build container (needs ``/root/reference``):
+Needs a checkout of the original project:
 
-    python -m oracle.make_golden
+    NFP_REFERENCE_ROOT=/path/to/Neighbour_Feature_Pooling python -m oracle.make_golden
 
 Executes the *unmodified* reference ``NFPPooling`` / ``nfp_pooling`` modules on
 seeded inputs and stores inputs, outputs and input-gradients as small ``.npz``
@@ -120,7 +120,11 @@ def main():
                                       padding=geom[6], dilation=geom[7], padding_mode=geom[8],
                                       similarity=similarity, p=p, relu=relu))
                     cid += 1
-    np.savez_compressed(os.path.join(OUT_DIR, "nfp_measures.npz"), **arrays)
+    half = len(index) // 2   # two files by case, each under 1 MB (tests/_util.py merges them)
+    for part, cases in ((1, index[:half]), (2, index[half:])):
+        keys = {c["key"] for c in cases}
+        np.savez_compressed(os.path.join(OUT_DIR, f"nfp_measures_{part}.npz"),
+                            **{k: v for k, v in arrays.items() if k.split("_")[0] in keys})
     with open(os.path.join(OUT_DIR, "nfp_measures.json"), "w") as f:
         json.dump(dict(generator="oracle/make_golden.py", torch=torch.__version__,
                        reference="models/pooling/nfp.py NFPPooling (unmodified, CPU)",

@@ -10,7 +10,7 @@ oracle run in fp64.  The floating-point semantics that live in ATen
 same ATen ops the reference calls.
 
 Pinned against the reference itself by ``oracle/check_against_reference.py``
-(run in the build container, where ``/root/reference`` exists) and by the
+(run where a reference checkout is named by ``NFP_REFERENCE_ROOT``) and by the
 fixtures in ``tests/golden/`` (``oracle/make_golden.py``).
 
 Citations are ``file:line`` relative to the reference checkout.

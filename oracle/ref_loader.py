@@ -1,10 +1,13 @@
 """TEST INFRASTRUCTURE ONLY -- import the *unmodified* reference modules.
 
-Works only where the reference checkout exists (the build container:
-``/root/reference``; never on the GPU box).  The reference imports
-``matplotlib.pyplot`` without using it (``models/pooling/nfp.py:12``); that
-package is not installed here, so an empty stub is injected before import.
-Nothing is copied out of the reference tree.
+The original Neighbour_Feature_Pooling project is not part of this repository.
+It is read from the checkout named by ``NFP_REFERENCE_ROOT``, else from a copy
+of its files inside the tree (git-ignored): ``oracle/_ref/``, where
+``__graft_entry__.build()`` stages them, or ``baseline/_ref/``, where earlier
+builds did.  Such a copy travels with the working tree to a machine that has no
+checkout.  The reference imports ``matplotlib.pyplot`` without using it
+(``models/pooling/nfp.py:12``); if that package is not installed, an empty stub
+is injected before import.
 """
 from __future__ import annotations
 
@@ -13,38 +16,42 @@ import sys
 import types
 
 _REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-# the reference checkout (build container), else the copy of its two operator files that __graft_entry__.build()
-# leaves under the git-ignored baseline/_ref/ (it travels to the GPU box with the repo snapshot)
-STAGED_ROOT = os.path.join(_REPO, "baseline", "_ref")
-REFERENCE_ROOT = os.environ.get("NFP_REFERENCE_ROOT") or (
-    "/root/reference" if os.path.isfile("/root/reference/models/pooling/nfp.py") else STAGED_ROOT)
-OPERATOR_FILES = ("models/__init__.py", "models/pooling/nfp.py", "models/NFP_Pooling.py")
+STAGED_ROOTS = (os.path.join(_REPO, "oracle", "_ref"), os.path.join(_REPO, "baseline", "_ref"))
+# the operator files, and the heads module that tests/test_modules_contract.py runs on the drop-in
+OPERATOR_FILES = ("models/__init__.py", "models/pooling/nfp.py", "models/NFP_Pooling.py", "models/nfp_heads.py")
+
+
+def _has_reference(root: str) -> bool:
+    return bool(root) and os.path.isfile(os.path.join(root, "models", "pooling", "nfp.py"))
+
+
+REFERENCE_ROOT = os.environ.get("NFP_REFERENCE_ROOT") or next(
+    (r for r in STAGED_ROOTS if _has_reference(r)), STAGED_ROOTS[0])
 
 
 def reference_available() -> bool:
-    return os.path.isfile(os.path.join(REFERENCE_ROOT, "models", "pooling", "nfp.py"))
+    return _has_reference(REFERENCE_ROOT)
 
 
-def stage_reference(src_root: str = "/root/reference") -> bool:
-    """Copy the reference's two operator files (unmodified) to baseline/_ref/ so that bench.py can time the REAL
-    reference on a box that has no /root/reference.  baseline/_ref/ is git-ignored: nothing enters the history."""
+def stage_reference(src_root: str = os.environ.get("NFP_REFERENCE_ROOT", "")) -> bool:
+    """Copy OPERATOR_FILES, unmodified, from the checkout `src_root` to oracle/_ref/ so that bench.py's CPU arm and the
+    reference tests can use them where that checkout is absent.  Returns whether a copy is in the tree."""
     import shutil
-    if not os.path.isfile(os.path.join(src_root, "models", "pooling", "nfp.py")):
-        return os.path.isfile(os.path.join(STAGED_ROOT, "models", "pooling", "nfp.py"))
-    for rel in OPERATOR_FILES:
-        src, dst = os.path.join(src_root, rel), os.path.join(STAGED_ROOT, rel)
-        os.makedirs(os.path.dirname(dst), exist_ok=True)
-        if os.path.isfile(src):
-            shutil.copyfile(src, dst)
-        elif rel.endswith("__init__.py"):
-            open(dst, "w").close()
-    return True
+    if _has_reference(src_root) and os.path.abspath(src_root) != STAGED_ROOTS[0]:
+        for rel in OPERATOR_FILES:
+            src, dst = os.path.join(src_root, rel), os.path.join(STAGED_ROOTS[0], rel)
+            os.makedirs(os.path.dirname(dst), exist_ok=True)
+            if os.path.isfile(src):
+                shutil.copyfile(src, dst)
+            elif rel.endswith("__init__.py"):
+                open(dst, "w").close()
+    return any(_has_reference(r) for r in STAGED_ROOTS)
 
 
 def load_reference():
     """Return ``(NFPPooling, nfp_pooling)`` classes of the reference."""
     if not reference_available():
-        raise RuntimeError(f"reference checkout not found at {REFERENCE_ROOT}")
+        raise RuntimeError(f"reference not found at {REFERENCE_ROOT} (set NFP_REFERENCE_ROOT to a checkout of it)")
     for name in ("matplotlib", "matplotlib.pyplot"):
         if name not in sys.modules:
             try:

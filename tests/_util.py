@@ -11,7 +11,9 @@ GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 def load_measure_cases():
     with open(os.path.join(GOLDEN, "nfp_measures.json")) as f:
         index = json.load(f)["cases"]
-    arrays = np.load(os.path.join(GOLDEN, "nfp_measures.npz"))
+    arrays = {}
+    for part in (1, 2):   # stored in two halves by case (oracle/make_golden.py) to keep each file under 1 MB
+        arrays.update(np.load(os.path.join(GOLDEN, f"nfp_measures_{part}.npz")))
     return index, arrays
 
 

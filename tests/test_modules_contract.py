@@ -129,7 +129,7 @@ def test_install_dropin_import_paths():
     assert "models.pooling.nfp" not in sys.modules
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference checkout only exists in the build container")
+@pytest.mark.skipif(not reference_available(), reason="needs the original project: NFP_REFERENCE_ROOT or a copy staged under oracle/_ref")
 def test_reference_heads_run_unchanged_on_the_dropin():
     """models/nfp_heads.py is un-importable upstream (missing EnhancedNFPPooling); with the drop-in
     installed it imports, and its constructors' CPU dummy probes (nfp_heads.py:24-27,95-97) work."""

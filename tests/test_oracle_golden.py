@@ -93,7 +93,7 @@ def test_algorithmic_bytes_table():
     assert O.algorithmic_bytes_per_map(256, 14, 14, 2, 2) == 319872
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference checkout only exists in the build container")
+@pytest.mark.skipif(not reference_available(), reason="needs the original project: NFP_REFERENCE_ROOT or a copy staged under oracle/_ref")
 def test_oracle_against_live_reference_subset():
     from oracle import check_against_reference as chk
     from oracle.ref_loader import load_reference
