@@ -7,7 +7,9 @@
 * size-independent properties at BASELINE.json's full sizes (B=256, 512x7x7 / 256x14x14).
 
 Tolerances (BASELINE.json north_star): fp32 <= 1e-5 relative (max-norm), bf16 <= 2e-2 against the
-fp32/fp64 reference evaluated on the bf16-rounded input.
+fp32/fp64 reference evaluated on the bf16-rounded input.  Input gradients are scored with grad_err (tests/_util.py):
+each image and each pixel-norm region (||x|| <= 2 eps, small, ordinary) on its own scale, so that the 1e6-sized
+gradients of the planted degenerate pixels do not set the scale for all the others.
 """
 import numpy as np
 import pytest
@@ -17,7 +19,8 @@ import neighbour_feature_pooling_b200 as nfpb
 from neighbour_feature_pooling_b200 import NFPPooling, nfp_pooling, functional as NF
 from oracle import nfp_oracle as O
 
-from _util import case_id, case_kwargs, load_measure_cases, load_multi_radius_cases, load_wrapper_cases, rel_err
+from _util import (case_id, case_kwargs, grad_err, grad_errs, load_measure_cases, load_multi_radius_cases,
+                   load_wrapper_cases, rel_err, worst)
 
 pytestmark = pytest.mark.gpu
 
@@ -49,7 +52,10 @@ def test_golden_fp32(c, cuda_device):
         y, gx = _run(x, g, case_kwargs(c), cuda_device, path=path)
         gtol = FP32_TOL if c["measure"].lower() == "cosine" else max(tol, 2e-5)
         assert rel_err(y, ARR[c["key"] + "_y_f64"]) < tol, path
-        assert rel_err(gx, ARR[c["key"] + "_gx_f64"]) < gtol, path
+        # per region over the (1-3 image) batch: the fixtures pin each measure's semantics; the per-image scale is for
+        # the batched kernels' tests, and Geman's own fp32 evaluation is too ill-conditioned for it (0.66 of the bound)
+        errs = grad_errs(gx, ARR[c["key"] + "_gx_f64"], x, per_image=False)
+        assert max(errs.values()) < gtol, (path, worst(errs))
 
 
 @pytest.mark.parametrize("c", [c for c in INDEX if c["measure"] in ("cosine", "dot", "gfc", "emd")], ids=case_id)
@@ -59,7 +65,7 @@ def test_golden_bf16(c, cuda_device):
     y_ref, gx_ref = O.nfp_forward_backward(x.double(), g.double(), **case_kwargs(c))
     y, gx = _run(x, g, case_kwargs(c), cuda_device, dtype=torch.bfloat16)
     assert rel_err(y, y_ref) < BF16_TOL
-    assert rel_err(gx, gx_ref) < BF16_TOL
+    assert grad_err(gx, gx_ref, x, per_image=False) < BF16_TOL
 
 
 GEOMS = [  # (B, C, H, W, R, stride, padding, dilation, mode)
@@ -146,7 +152,8 @@ def test_planar_cosine_vs_oracle(shape, mode, dtype, similarity, cuda_device):
     y, gx = _run(x, g, kw, cuda_device, dtype=dtype)
     tol = FP32_TOL if dtype == torch.float32 else BF16_TOL
     assert rel_err(y, y_ref) < tol
-    assert rel_err(gx, gx_ref) < tol
+    errs = grad_errs(gx, gx_ref, x)
+    assert max(errs.values()) < tol, worst(errs)
     if R <= 2:  # bit-reproducible (gather form, no atomics)
         y2, gx2 = _run(x, g, kw, cuda_device, dtype=dtype)
         assert torch.equal(y, y2) and torch.equal(gx, gx2)
@@ -172,29 +179,27 @@ def test_fused_cosine_vs_oracle(shape, mode, dtype, cuda_device):
     g = torch.randn(B, K, H, W, generator=gen)
     if dtype == torch.bfloat16:
         g = g.bfloat16().float()
-    if B > 32:   # more images than resident CTAs: exercises the persistent image loop; oracle on a slice
-        sl = slice(B - 4, B)
-        y_ref, gx_ref = O.nfp_forward_backward(x[sl].double(), g[sl].double(), **kw)
-        y, gx = _run(x, g, kw, cuda_device, dtype=dtype)
-        y, gx = y[sl], gx[sl]
-    else:
-        y_ref, gx_ref = O.nfp_forward_backward(x.double(), g.double(), **kw)
-        y, gx = _run(x, g, kw, cuda_device, dtype=dtype)
+    # more images than resident CTAs exercises the persistent image loop: oracle on a slice
+    sl = slice(B - 4, B) if B > 32 else slice(0, B)
+    y_ref, gx_ref = O.nfp_forward_backward(x[sl].double(), g[sl].double(), **kw)
+    y, gx = _run(x, g, kw, cuda_device, dtype=dtype)
+    y, gx = y[sl], gx[sl]
     tol = FP32_TOL if dtype == torch.float32 else BF16_TOL
     assert rel_err(y, y_ref) < tol
-    assert rel_err(gx, gx_ref) < tol
+    errs = grad_errs(gx, gx_ref, x[sl])
+    assert max(errs.values()) < tol, worst(errs)
     if dtype == torch.float32 and B <= 32:
         # and the CUDA paths agree with each other
         y2, gx2 = _run(x, g, kw, cuda_device, path="generic")
-        assert rel_err(y, y2) < FP32_TOL and rel_err(gx, gx2) < FP32_TOL
+        assert rel_err(y, y2) < FP32_TOL and grad_err(gx, gx2, x) < FP32_TOL
     # the cluster-split kernels (NFPB200_PATH_SPLIT: the measured experiment of DESIGN.md 4.2) on the same problem
     cfg_split = NF.replace(cfg, path="split")
     assert NF.describe(shape[:4], dtype, cfg_split).startswith("fused/split")
     y3, gx3 = _run(x, g, kw, cuda_device, dtype=dtype, path="split")
-    if B > 32:
-        y3, gx3 = y3[sl], gx3[sl]
+    y3, gx3 = y3[sl], gx3[sl]
     assert rel_err(y3, y_ref) < tol
-    assert rel_err(gx3, gx_ref) < tol
+    errs = grad_errs(gx3, gx_ref, x[sl])
+    assert max(errs.values()) < tol, worst(errs)
 
 
 @pytest.mark.parametrize("shape", [(40, 8, 7, 7, 1), (40, 16, 7, 7, 2), (24, 2, 14, 14, 1), (24, 4, 14, 14, 2),
@@ -259,7 +264,7 @@ def test_wrapper_golden(cuda_device):
         out = pool(x)
         out.backward(torch.from_numpy(arr[k + "_g"]).to(cuda_device))
         assert rel_err(out.detach().cpu(), arr[k + "_out"]) < FP32_TOL
-        assert rel_err(x.grad.cpu(), arr[k + "_gx"]) < FP32_TOL
+        assert grad_err(x.grad.cpu(), arr[k + "_gx"], arr[k + "_x"]) < FP32_TOL
         assert rel_err(pool.nfp_proj.weight.grad.cpu(), arr[k + "_gw"]) < FP32_TOL
         assert rel_err(pool.nfp_proj.bias.grad.cpu(), arr[k + "_gb"]) < FP32_TOL
 
@@ -552,7 +557,7 @@ def test_pooled_vs_oracle(case, dtype, cuda_device):
     tol = FP32_TOL if dtype == torch.float32 else BF16_TOL
     assert rel_err(a.detach().float().cpu(), gap_x_ref) < tol
     assert rel_err(n.detach().float().cpu(), gap_nfp_ref) < tol
-    assert rel_err(xd.grad.float().cpu(), gx_ref) < tol
+    assert grad_err(xd.grad.float().cpu(), gx_ref, x) < tol, worst(grad_errs(xd.grad.float().cpu(), gx_ref, x))
     if NF.describe((B, C, H, W), dtype, cfg, op=2).startswith("fused/"):   # the cluster-split pooled kernels as well
         cfg_s = NF.replace(cfg, path="split")
         xs_ = x.to(cuda_device, dtype).requires_grad_(True)
@@ -560,7 +565,7 @@ def test_pooled_vs_oracle(case, dtype, cuda_device):
         ((a2.float() * g1.to(cuda_device)).sum() + (n2.float() * g2.to(cuda_device)).sum()).backward()
         assert rel_err(a2.detach().float().cpu(), gap_x_ref) < tol
         assert rel_err(n2.detach().float().cpu(), gap_nfp_ref) < tol
-        assert rel_err(xs_.grad.float().cpu(), gx_ref) < tol
+        assert grad_err(xs_.grad.float().cpu(), gx_ref, x) < tol, worst(grad_errs(xs_.grad.float().cpu(), gx_ref, x))
 
 
 def test_nfp_pooling_respects_customised_layers(cuda_device):
@@ -624,7 +629,7 @@ def test_channels_last_bf16_without_repack(shape, mode, similarity, cuda_device)
     assert y.is_contiguous() and y.shape == (B, K, H, W)
     assert xd.grad.stride() == xd.stride() or H * W == 1, "gradient comes back channels_last"
     assert rel_err(y.detach().float().cpu(), y_ref) < BF16_TOL
-    assert rel_err(xd.grad.float().cpu(), gx_ref) < BF16_TOL
+    assert grad_err(xd.grad.float().cpu(), gx_ref, x) < BF16_TOL, worst(grad_errs(xd.grad.float().cpu(), gx_ref, x))
     # the NCHW kernels on the same values agree to bf16 rounding, and the token path repeats bit for bit
     xn = x.to(cuda_device, torch.bfloat16).requires_grad_(True)
     yn = layer(xn)
@@ -645,7 +650,7 @@ def test_channels_last_bf16_without_repack(shape, mode, similarity, cuda_device)
     ((a.float() * g1.to(cuda_device)).sum() + (n.float() * g2.to(cuda_device)).sum()).backward()
     assert rel_err(a.detach().float().cpu(), x.double().mean((2, 3))) < BF16_TOL
     assert rel_err(n.detach().float().cpu(), y_map.mean((2, 3))) < BF16_TOL
-    assert rel_err(x3.grad.float().cpu(), gx_map + (g1.double() / (H * W))[:, :, None, None]) < BF16_TOL
+    assert grad_err(x3.grad.float().cpu(), gx_map + (g1.double() / (H * W))[:, :, None, None], x) < BF16_TOL
 
 
 def test_vit_token_view_without_transpose_copy(cuda_device):
@@ -849,13 +854,14 @@ def test_multi_radius_one_launch_vs_oracle(shape, mode, similarity, dtype, cuda_
     assert y.shape == (B, 32, H, W)
     tol = FP32_TOL if dtype == torch.float32 else BF16_TOL
     assert rel_err(y.detach().float().cpu()[sl], y_ref) < tol
-    assert rel_err(xd.grad.float().cpu()[sl], gx_ref) < tol
+    errs = grad_errs(xd.grad.float().cpu()[sl], gx_ref, x[sl])
+    assert max(errs.values()) < tol, worst(errs)
     # against the same kernels launched once per radius (+ cat): the forward values are the same table entries
     x2 = x.to(cuda_device, dtype).requires_grad_(True)
     y2 = torch.cat([b(x2) for b in blocks.nfp_blocks], dim=1)
     y2.backward(g.to(cuda_device, dtype))
     assert rel_err(y.detach().float().cpu(), y2.detach().float().cpu()) < (2e-6 if dtype == torch.float32 else 1e-2)
-    assert rel_err(xd.grad.float().cpu(), x2.grad.float().cpu()) < (1e-5 if dtype == torch.float32 else 2e-2)
+    assert grad_err(xd.grad.float().cpu(), x2.grad.float().cpu(), x) < (1e-5 if dtype == torch.float32 else 2e-2)
     # bit-repeatable
     x3 = x.to(cuda_device, dtype).requires_grad_(True)
     y3 = blocks(x3)
@@ -946,7 +952,8 @@ def test_multi_radius_other_map_sizes(shape, mode, similarity, dtype, cuda_devic
     assert any("radii 1+2 in one launch" in t and "planar/band" in t for t in trace), trace
     tol = FP32_TOL if dtype == torch.float32 else BF16_TOL
     assert rel_err(y.detach().float().cpu(), y_ref) < tol
-    assert rel_err(xd.grad.float().cpu(), gx_ref) < tol
+    errs = grad_errs(xd.grad.float().cpu(), gx_ref, x)
+    assert max(errs.values()) < tol, worst(errs)
     x2 = x.to(cuda_device, dtype).requires_grad_(True)   # bit-repeatable
     y2 = mr(x2)
     y2.backward(g.to(cuda_device, dtype))
