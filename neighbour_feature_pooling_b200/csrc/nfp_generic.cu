@@ -365,9 +365,9 @@ __global__ void __launch_bounds__(kThreads) scs_forward_kernel(const float* __re
   y[idx] = from_f32<T>(P.similarity ? v : 1.f - v);
 }
 
-// coefficients of every pair (SoA: coef[u * npairs + idx])
-template <typename T, int M>
-__global__ void __launch_bounds__(kThreads) pair_coef_kernel(const T* __restrict__ x, const T* __restrict__ gy,
+// coefficients of every pair (SoA: coef[u * npairs + idx]); gy is T (map mode) or fp32 (pooled mode, GT = float)
+template <typename T, typename GT, int M>
+__global__ void __launch_bounds__(kThreads) pair_coef_kernel(const T* __restrict__ x, const GT* __restrict__ gy,
                                                              float* __restrict__ coef, KParams P,
                                                              long long npairs) {
   long long idx = (long long)blockIdx.x * kThreads + threadIdx.x;
@@ -607,19 +607,19 @@ int forward_t(const KParams& P, int measure, const T* x, T* y, const LaunchCtx& 
 }
 
 // workspace layout of backward: [coef: 5*npairs f32]
-template <typename T>
-int backward_t(const KParams& P, int measure, const T* x, const T* gy, T* gx, const float* g_gap_x,
+template <typename T, typename GT>
+int backward_t(const KParams& P, int measure, const T* x, const GT* gy, T* gx, const float* g_gap_x,
                char* ws, cudaStream_t stream) {
   const long long npairs = (long long)P.B * P.K * P.Ho * P.Wo;
   const long long nx = (long long)P.B * P.C * P.H * P.W;
   float* coef = (float*)ws;
   NFP_DISPATCH_MEASURE(measure,
-    (pair_coef_kernel<T, M><<<blocks_for(npairs), kThreads, 0, stream>>>(x, gy, coef, P, npairs)));
+    (pair_coef_kernel<T, GT, M><<<blocks_for(npairs), kThreads, 0, stream>>>(x, gy, coef, P, npairs)));
   if (measure == NFPB200_ATTENTION) {
     long long pix = (long long)P.B * P.Ho * P.Wo;
-    attention_coef_kernel<T><<<blocks_for(pix), kThreads, 0, stream>>>(gy, coef, P);
+    attention_coef_kernel<GT><<<blocks_for(pix), kThreads, 0, stream>>>(gy, coef, P);
   } else if (measure == NFPB200_SCS) {
-    scs_coef_kernel_a<T><<<blocks_for(npairs), kThreads, 0, stream>>>(gy, coef, P, npairs);
+    scs_coef_kernel_a<GT><<<blocks_for(npairs), kThreads, 0, stream>>>(gy, coef, P, npairs);
     scs_coef_kernel_b<<<blocks_for(npairs), kThreads, 0, stream>>>(coef, P, npairs);
   }
   NFP_DISPATCH_MEASURE(measure,
@@ -640,7 +640,7 @@ size_t generic_workspace_bytes(const KParams& P, int dtype, int measure, int op)
     case NFPB200_OP_FORWARD: return fwd;
     case NFPB200_OP_BACKWARD: return bwd;
     case NFPB200_OP_POOL_FORWARD: return align256(esz * npairs) + fwd;   // [y map][forward scratch]
-    case NFPB200_OP_POOL_BACKWARD: return align256(esz * npairs) + bwd;  // [gy map][backward scratch]
+    case NFPB200_OP_POOL_BACKWARD: return align256(4 * npairs) + bwd;    // [fp32 gy map][backward scratch]
   }
   return 0;
 }
@@ -670,10 +670,10 @@ int generic_forward(const KParams& P, int dtype, int measure, const void* x, voi
 int generic_backward(const KParams& P, int dtype, int measure, const void* x, const void* gy, void* gx,
                      const LaunchCtx& ctx) {
   if (dtype == NFPB200_BF16)
-    return backward_t<__nv_bfloat16>(P, measure, (const __nv_bfloat16*)x, (const __nv_bfloat16*)gy,
-                                     (__nv_bfloat16*)gx, nullptr, (char*)ctx.ws, ctx.stream);
-  return backward_t<float>(P, measure, (const float*)x, (const float*)gy, (float*)gx, nullptr, (char*)ctx.ws,
-                           ctx.stream);
+    return backward_t<__nv_bfloat16, __nv_bfloat16>(P, measure, (const __nv_bfloat16*)x, (const __nv_bfloat16*)gy,
+                                                     (__nv_bfloat16*)gx, nullptr, (char*)ctx.ws, ctx.stream);
+  return backward_t<float, float>(P, measure, (const float*)x, (const float*)gy, (float*)gx, nullptr, (char*)ctx.ws,
+                                  ctx.stream);
 }
 
 namespace {
@@ -693,11 +693,13 @@ template <typename T>
 int pool_backward_t(const KParams& P, int measure, const T* x, const float* g_gap_x, const float* g_gap_nfp,
                     T* gx, const LaunchCtx& ctx) {
   const size_t npairs = (size_t)P.B * P.K * P.Ho * P.Wo;
-  T* gymap = (T*)ctx.ws;
-  expand_gap_grad_kernel<T><<<blocks_for((long long)npairs), kThreads, 0, ctx.stream>>>(
+  // the map gradient g_gap_nfp / (Ho*Wo) stays fp32 also for bf16 x: rounded to bf16, its 2^-9 error is multiplied by
+  // the per-tap derivatives, which cancel to far smaller sums at pixels near a clamp (norm ~ eps, |c| + |n| ~ eps)
+  float* gymap = (float*)ctx.ws;
+  expand_gap_grad_kernel<float><<<blocks_for((long long)npairs), kThreads, 0, ctx.stream>>>(
       g_gap_nfp, gymap, P.Ho * P.Wo, (long long)npairs);
-  return backward_t<T>(P, measure, x, gymap, gx, g_gap_x, (char*)ctx.ws + align256(sizeof(T) * npairs),
-                       ctx.stream);
+  return backward_t<T, float>(P, measure, x, gymap, gx, g_gap_x, (char*)ctx.ws + align256(sizeof(float) * npairs),
+                              ctx.stream);
 }
 }  // namespace
 

@@ -11,6 +11,8 @@ fp32/fp64 reference evaluated on the bf16-rounded input.  Input gradients are sc
 each image and each pixel-norm region (||x|| <= 2 eps, small, ordinary) on its own scale, so that the 1e6-sized
 gradients of the planted degenerate pixels do not set the scale for all the others.
 """
+import zlib
+
 import numpy as np
 import pytest
 import torch
@@ -19,8 +21,8 @@ import neighbour_feature_pooling_b200 as nfpb
 from neighbour_feature_pooling_b200 import NFPPooling, nfp_pooling, functional as NF
 from oracle import nfp_oracle as O
 
-from _util import (case_id, case_kwargs, grad_err, grad_errs, load_measure_cases, load_multi_radius_cases,
-                   load_wrapper_cases, rel_err, worst)
+from _util import (case_id, case_kwargs, elem_grad_errs, grad_err, grad_errs, load_measure_cases,
+                   load_multi_radius_cases, load_wrapper_cases, rel_err, worst)
 
 pytestmark = pytest.mark.gpu
 
@@ -86,7 +88,7 @@ def test_random_vs_oracle_generic(measure, geom, cuda_device):
     B, C, H, W, R, s, pad, d, mode = geom
     if H * W > 4096 and measure not in ("cosine", "norm", "dot"):
         pytest.skip("large map checked for the hot measures only")
-    gen = torch.Generator().manual_seed(hash((measure, geom)) % (2 ** 31))
+    gen = torch.Generator().manual_seed(zlib.crc32(repr((measure, geom)).encode()))   # stable across processes
     x = torch.randn(B, C, H, W, generator=gen)
     kw = dict(R=R, measure=measure, p=2 if measure in ("norm", "scs") else 1, stride=s, padding=pad,
               dilation=d, padding_mode=mode)
@@ -96,7 +98,11 @@ def test_random_vs_oracle_generic(measure, geom, cuda_device):
     y, gx = _run(x, g, kw, cuda_device, path="generic")
     tol = LOOSE.get(measure, FP32_TOL)
     assert rel_err(y, y_ref) < tol
-    assert rel_err(gx, gx_ref) < max(tol, 2e-5)
+    # each image and each magnitude bucket on its own scale (elem_grad_errs): near-zero denominators set no one's scale
+    from test_generic_parity_gpu import aten_fp32, allowed
+    _, t_gx = allowed(measure, torch.float32, aten_fp32("map", x, [g], kw))
+    errs = elem_grad_errs(gx, gx_ref, O.geometry(H, W, R, s, pad, d, mode))
+    assert all(e < t_gx[k] for k, e in errs.items()), [(k, e, t_gx[k]) for k, e in errs.items() if not e < t_gx[k]]
     # the generic backward gathers through the inverse index map in a fixed order (no atomics): same bits every time
     y2, gx2 = _run(x, g, kw, cuda_device, path="generic")
     assert torch.equal(y.view(torch.int32), y2.view(torch.int32))
