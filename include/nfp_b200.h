@@ -12,6 +12,9 @@
  *   nfpb200_pool_forward   <- nfp_pooling.forward up to the projection: GAP(x) and
  *                             GAP(NFP(x))                   (models/NFP_Pooling.py:27-31)
  *   nfpb200_pool_backward  <- autograd through those two lines
+ *   nfpb200_pooled_map_forward  <- adaptive_avg_pool2d(NFPPooling(x), (1, 1)).view(B, -1): every stage of
+ *                             MobileNetV3_MultiStageNFP   (models/texture_pooling.py:249-256)
+ *   nfpb200_pooled_map_backward <- autograd through those lines
  *   nfpb200_output_shape   <- Conv2d output-size rule behind NFPPooling.output_size
  *                                                           (nfp.py:125-130, 42-47)
  *   nfpb200_desc_t         <- the constructor arguments     (nfp.py:16-18); inner_R: the two NFP layers of
@@ -42,7 +45,7 @@
 extern "C" {
 #endif
 
-#define NFPB200_ABI_VERSION 3
+#define NFPB200_ABI_VERSION 4
 
 /* element type of x / y / gy / gx.  Accumulation is always fp32. */
 enum { NFPB200_F32 = 0, NFPB200_BF16 = 1 };
@@ -107,8 +110,15 @@ enum {
  * neighbours, nfp.py:152-156).  Honoured by the fused kernels; other paths return NFPB200_EUNSUPPORTED. */
 #define NFPB200_FLAG_Y_F32 0x200
 
-/* operations, for nfpb200_workspace_bytes / nfpb200_describe_path */
-enum { NFPB200_OP_FORWARD = 0, NFPB200_OP_BACKWARD = 1, NFPB200_OP_POOL_FORWARD = 2, NFPB200_OP_POOL_BACKWARD = 3 };
+/* operations, for nfpb200_workspace_bytes / nfpb200_describe_path / nfpb200_launch_count */
+enum {
+  NFPB200_OP_FORWARD = 0,
+  NFPB200_OP_BACKWARD = 1,
+  NFPB200_OP_POOL_FORWARD = 2,
+  NFPB200_OP_POOL_BACKWARD = 3,
+  NFPB200_OP_POOLED_MAP_FORWARD = 4,  /* ABI v4 */
+  NFPB200_OP_POOLED_MAP_BACKWARD = 5  /* ABI v4 */
+};
 
 /* error codes (negative); positive return values are cudaError_t */
 enum {
@@ -169,14 +179,15 @@ int nfpb200_debug_phase_timing(unsigned long long* device_stamps);
 /* (H', W') = Conv2d output size for the descriptor's geometry; validates the descriptor. */
 int nfpb200_output_shape(const nfpb200_desc_t* desc, int32_t* Ho, int32_t* Wo);
 
-/* Device scratch the given op needs (0 for the fused kernels; per-pixel tables for the planar kernels, pair
- * coefficients for the generic ones).  The caller allocates it and passes it in. */
+/* Device scratch the given op needs (0 for the fused kernels' map and pool ops; per-pixel tables for the planar kernels,
+ * pair coefficients for the generic ones; for the pooled-map ops see nfpb200_pooled_map_forward).  The caller allocates
+ * it and passes it in. */
 int nfpb200_workspace_bytes(const nfpb200_desc_t* desc, int32_t op, size_t* bytes);
 
 /* Writes the name of the kernel path the op would take ("fused/...", "planar/..." or "generic/...") into buf. */
 int nfpb200_describe_path(const nfpb200_desc_t* desc, int32_t op, char* buf, size_t buf_bytes);
 
-/* Number of kernel launches the op issues on `stream` (bench.py's gpu_launches). */
+/* Number of kernel launches the op issues on `stream` (bench.py's gpu_launches), counting a cudaMemsetAsync as one. */
 int nfpb200_launch_count(const nfpb200_desc_t* desc, int32_t op, int32_t* launches);
 
 /* y (B, K, H', W') = NFP(x)   (desc->inner_R = r > 0: (B, K_r + K, H, W), see nfpb200_desc_t).  */
@@ -197,6 +208,29 @@ int nfpb200_pool_forward(const nfpb200_desc_t* desc, const void* x, float* gap_x
 int nfpb200_pool_backward(const nfpb200_desc_t* desc, const void* x, const float* g_gap_x,
                           const float* g_gap_nfp, void* gx,
                           void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---- pooled similarity map (ABI v4) ----------------------------------------------------------------------------
+ * The reference's multi-stage head pools every NFP map right away (models/texture_pooling.py:249-256:
+ * adaptive_avg_pool2d(nfp(x), (1, 1)).view(B, -1)); these entry points compute only that, without writing the map:
+ *   gap_nfp (B, K) fp32 = mean over the H' x W' output pixels of NFP(x), whatever desc->dtype.
+ * desc->inner_R != 0 returns NFPB200_EUNSUPPORTED.  What each problem takes (nfpb200_describe_path names it):
+ *   - NHWC bf16 covered by the token kernels: their pooled mode ("fused/token_*"); GAP(x) goes to the workspace;
+ *   - NCHW covered by the ring kernels: their pooled mode ("fused/stream_*"); GAP(x) goes to the workspace;
+ *   - NCHW cosine, stride 1, dilation 1, padding = R <= 2, not circular, whose map mode takes "planar/band": the row-band
+ *     kernels' pooled mode ("planar/band").  Forward: 2 launches (per-band partial sums (B, n_bands, K) fp32 in the
+ *     workspace, then a kernel that sums them in band order and divides by H' W'); backward: 1 launch, no workspace;
+ *   - anything else, and NFPB200_PATH_GENERIC: the generic kernels' pooled mode ("generic/pairs") without its GAP(x) part.
+ * NFPB200_PATH_FUSED: the ring / token kernels or NFPB200_EUNSUPPORTED.  No float atomics on any path: results are
+ * bit-identical from run to run. */
+int nfpb200_pooled_map_forward(const nfpb200_desc_t* desc, const void* x, float* gap_nfp,
+                               void* workspace, size_t workspace_bytes, void* stream);
+
+/* gx = d<g_gap_nfp, GAP(NFP(x))>/dx ; g_gap_nfp is fp32 (B, K).  Same paths as the forward.  The ring and token kernels
+ * read a zero (B, C) g_gap_x from the workspace, which this call clears first with one cudaMemsetAsync (2 launches in
+ * all); the row-band kernels (1 launch) keep g_gap_nfp / (H' W') in fp32 registers and shared memory and read no per-pixel
+ * gradient; the generic kernels expand it to an fp32 map in the workspace. */
+int nfpb200_pooled_map_backward(const nfpb200_desc_t* desc, const void* x, const float* g_gap_nfp, void* gx,
+                                void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- fused nfp_pooling head (NFP_Pooling.py:25-36), one launch each way ---------------------------------------
  *   out (B, C) = GAP(x) * (proj_w . GAP(NFP(x)) + proj_b)        proj_w (C, K) fp32 row-major = nfp_proj.weight,

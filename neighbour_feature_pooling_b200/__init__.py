@@ -20,9 +20,9 @@ import sys
 import types
 
 from . import _capi, functional
-from .functional import NFPConfig, nfp_gap_pair, nfp_multi_radius, nfp_similarity
-from .modules import (EnhancedNFPPooling, MultiRadiusNFP, NFPPooling, fuse_multi_radius, nfp_pooling,
-                      unfuse_multi_radius)
+from .functional import NFPConfig, nfp_gap_pair, nfp_multi_radius, nfp_pooled_similarity, nfp_similarity
+from .modules import (EnhancedNFPPooling, MultiRadiusNFP, NFPPooling, fuse_multi_radius, fuse_pooled_nfp, nfp_pooling,
+                      unfuse_multi_radius, unfuse_pooled_nfp)
 
 __version__ = "0.1.0"
 
@@ -67,5 +67,6 @@ def library_path() -> str:
 
 
 __all__ = ["NFPPooling", "EnhancedNFPPooling", "nfp_pooling", "NFPConfig", "nfp_similarity", "nfp_gap_pair",
-           "nfp_multi_radius", "MultiRadiusNFP", "fuse_multi_radius", "unfuse_multi_radius",
+           "nfp_multi_radius", "nfp_pooled_similarity", "MultiRadiusNFP", "fuse_multi_radius", "unfuse_multi_radius",
+           "fuse_pooled_nfp", "unfuse_pooled_nfp",
            "install_dropin", "uninstall_dropin", "library_path", "functional"]

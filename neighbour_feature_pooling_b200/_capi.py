@@ -15,7 +15,7 @@ import threading
 _LIB_PATH = os.environ.get("NFPB200_LIB") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "lib",
                                                           "libnfp_b200.so")
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 F32, BF16 = 0, 1
 PAD_MODES = {"zeros": 0, "reflect": 1, "replicate": 2, "circular": 3}
@@ -29,6 +29,7 @@ PATHS = {"auto": 0, "generic": 1, "fused": 2, "split": 3}
 HINT_X_STABLE = 0x100   # NFPB200_HINT_X_STABLE, OR-ed into Desc.path for the backward entry points
 FLAG_Y_F32 = 0x200      # NFPB200_FLAG_Y_F32, OR-ed into Desc.path for nfpb200_forward with bf16 x: y is fp32
 OP_FORWARD, OP_BACKWARD, OP_POOL_FORWARD, OP_POOL_BACKWARD = 0, 1, 2, 3
+OP_POOLED_MAP_FORWARD, OP_POOLED_MAP_BACKWARD = 4, 5   # GAP(NFP(x)) alone (ABI v4)
 LAYOUT_NCHW, LAYOUT_NHWC = 0, 1
 
 EXPORTS = (
@@ -36,6 +37,7 @@ EXPORTS = (
     "nfpb200_workspace_bytes", "nfpb200_describe_path", "nfpb200_launch_count",
     "nfpb200_forward", "nfpb200_backward", "nfpb200_pool_forward", "nfpb200_pool_backward",
     "nfpb200_debug_phase_timing", "nfpb200_head_supported", "nfpb200_head_forward", "nfpb200_head_backward",
+    "nfpb200_pooled_map_forward", "nfpb200_pooled_map_backward",
 )
 
 
@@ -105,6 +107,10 @@ def load():
         lib.nfpb200_head_forward.argtypes = [dp, vp, vp, vp, vp, vp, vp, vp]
         lib.nfpb200_head_backward.restype = ctypes.c_int
         lib.nfpb200_head_backward.argtypes = [dp, vp, vp, vp, vp, vp, vp, vp, vp]
+        lib.nfpb200_pooled_map_forward.restype = ctypes.c_int
+        lib.nfpb200_pooled_map_forward.argtypes = [dp, vp, vp, vp, ctypes.c_size_t, vp]
+        lib.nfpb200_pooled_map_backward.restype = ctypes.c_int
+        lib.nfpb200_pooled_map_backward.argtypes = [dp, vp, vp, vp, vp, ctypes.c_size_t, vp]
         got = lib.nfpb200_abi_version()
         if got != ABI_VERSION:
             raise RuntimeError(f"libnfp_b200.so ABI version {got}, host code expects {ABI_VERSION}; rebuild")

@@ -64,8 +64,23 @@ int make_params(const nfpb200_desc_t* d, KParams* out) {
   return NFPB200_OK;
 }
 
+inline bool pooled_map_op(int op) { return op == NFPB200_OP_POOLED_MAP_FORWARD || op == NFPB200_OP_POOLED_MAP_BACKWARD; }
+// the pool op whose kernels a pooled-map op reuses on the ring, token and generic paths
+inline int pool_op_of(int op) {
+  return op == NFPB200_OP_POOLED_MAP_FORWARD ? NFPB200_OP_POOL_FORWARD
+                                              : (op == NFPB200_OP_POOLED_MAP_BACKWARD ? NFPB200_OP_POOL_BACKWARD : op);
+}
+inline size_t align256(size_t b) { return (b + 255) & ~(size_t)255; }
+
 // 4 = token (channels-last), 3 = planar, 2 = fused (cluster-split or streaming-ring kernels), 0 = generic, <0 = error
 int choose_path(const nfpb200_desc_t* d, const KParams& P, int op) {
+  if (pooled_map_op(op)) {
+    // the pool ops' choice (token, ring, generic; inner_R refused), with the row-band kernels' pooled mode taking the
+    // shapes whose map mode takes "planar/band" instead of the generic kernels
+    const int path = choose_path(d, P, pool_op_of(op));
+    const bool generic_forced = (d->path & ~kPathFlags) == NFPB200_PATH_GENERIC;
+    return (path == 0 && !generic_forced && planar_pooled_supported(P, d->dtype, d->measure)) ? 3 : path;
+  }
   if (P.rin) {  // multi-radius launch: the fused kernels' map modes or nothing
     if (op != NFPB200_OP_FORWARD && op != NFPB200_OP_BACKWARD) return NFPB200_EUNSUPPORTED;
     const int want = d->path & ~kPathFlags;
@@ -89,6 +104,8 @@ int choose_path(const nfpb200_desc_t* d, const KParams& P, int op) {
 }
 
 size_t path_workspace_bytes(int path, const nfpb200_desc_t* d, const KParams& P, int op) {
+  // pooled-map ops on the ring / token kernels: their GAP(x) output (forward) or zero g_gap_x input (backward), (B, C) fp32
+  if (pooled_map_op(op) && (path == 2 || path == 4)) return align256((size_t)P.B * P.C * sizeof(float));
   if (path == 3) return planar_workspace_bytes(P, d->dtype, op);
   if (path == 4) return 0;
   return path ? 0 : generic_workspace_bytes(P, d->dtype, d->measure, op);
@@ -147,7 +164,7 @@ int nfpb200_workspace_bytes(const nfpb200_desc_t* desc, int32_t op, size_t* byte
   KParams P;
   int rc = make_params(desc, &P);
   if (rc) return rc;
-  if (!bytes || op < NFPB200_OP_FORWARD || op > NFPB200_OP_POOL_BACKWARD) return NFPB200_EINVAL;
+  if (!bytes || op < NFPB200_OP_FORWARD || op > NFPB200_OP_POOLED_MAP_BACKWARD) return NFPB200_EINVAL;
   int path = choose_path(desc, P, op);
   if (path < 0) return path;
   *bytes = path_workspace_bytes(path, desc, P, op);
@@ -158,12 +175,12 @@ int nfpb200_describe_path(const nfpb200_desc_t* desc, int32_t op, char* buf, siz
   KParams P;
   int rc = make_params(desc, &P);
   if (rc) return rc;
-  if (!buf || buf_bytes == 0 || op < NFPB200_OP_FORWARD || op > NFPB200_OP_POOL_BACKWARD) return NFPB200_EINVAL;
+  if (!buf || buf_bytes == 0 || op < NFPB200_OP_FORWARD || op > NFPB200_OP_POOLED_MAP_BACKWARD) return NFPB200_EINVAL;
   int path = choose_path(desc, P, op);
   if (path < 0) return path;
   snprintf(buf, buf_bytes, "%s",
            path == 4 ? token_name(P) : path == 3 ? planar_name(P, desc->dtype, op)
-                     : (path == 2 ? stream_name(P, desc->dtype, desc->measure, op) : "generic/pairs"));
+                     : (path == 2 ? stream_name(P, desc->dtype, desc->measure, pool_op_of(op)) : "generic/pairs"));
   return NFPB200_OK;
 }
 
@@ -171,10 +188,12 @@ int nfpb200_launch_count(const nfpb200_desc_t* desc, int32_t op, int32_t* launch
   KParams P;
   int rc = make_params(desc, &P);
   if (rc) return rc;
-  if (!launches || op < NFPB200_OP_FORWARD || op > NFPB200_OP_POOL_BACKWARD) return NFPB200_EINVAL;
+  if (!launches || op < NFPB200_OP_FORWARD || op > NFPB200_OP_POOLED_MAP_BACKWARD) return NFPB200_EINVAL;
   int path = choose_path(desc, P, op);
   if (path < 0) return path;
-  *launches = path == 4 ? 1 : path == 3 ? planar_launch_count(P, desc->dtype, op) : (path ? 1 : generic_launch_count(P, desc->dtype, desc->measure, op));
+  if (path == 3) *launches = planar_launch_count(P, desc->dtype, op);
+  else if (path == 2 || path == 4) *launches = op == NFPB200_OP_POOLED_MAP_BACKWARD ? 2 : 1;   // + the g_gap_x memset
+  else *launches = generic_launch_count(P, desc->dtype, desc->measure, op);
   return NFPB200_OK;
 }
 
@@ -233,6 +252,33 @@ int nfpb200_pool_backward(const nfpb200_desc_t* desc, const void* x, const float
   if (path == 4) return token_run(P, NFPB200_OP_POOL_BACKWARD, x, nullptr, nullptr, gx, g_gap_x, g_gap_nfp, nullptr, nullptr, ctx);
   if (path == 2) return stream_pool_backward(P, desc->dtype, x, g_gap_x, g_gap_nfp, gx, ctx);
   return generic_pool_backward(P, desc->dtype, desc->measure, x, g_gap_x, g_gap_nfp, gx, ctx);
+}
+
+// ---- pooled similarity map: GAP(NFP(x)) alone ---------------------------------------------------------------------
+int nfpb200_pooled_map_forward(const nfpb200_desc_t* desc, const void* x, float* gap_nfp, void* workspace,
+                               size_t workspace_bytes, void* stream) {
+  if (!x || !gap_nfp) return NFPB200_EINVAL;
+  if (misaligned(x)) return NFPB200_EALIGN;
+  NFP_PROLOGUE(NFPB200_OP_POOLED_MAP_FORWARD)
+  if (path == 3) return planar_pooled_forward(P, desc->dtype, x, gap_nfp, ctx);
+  float* gap_x = static_cast<float*>(workspace);   // ring / token kernels: GAP(x) is written to the workspace
+  if (path == 4) return token_run(P, NFPB200_OP_POOL_FORWARD, x, nullptr, nullptr, nullptr, nullptr, nullptr, gap_x, gap_nfp, ctx);
+  if (path == 2) return stream_pool_forward(P, desc->dtype, x, gap_x, gap_nfp, ctx);
+  return generic_pool_forward(P, desc->dtype, desc->measure, x, nullptr, gap_nfp, ctx);
+}
+
+int nfpb200_pooled_map_backward(const nfpb200_desc_t* desc, const void* x, const float* g_gap_nfp, void* gx,
+                                void* workspace, size_t workspace_bytes, void* stream) {
+  if (!x || !g_gap_nfp || !gx) return NFPB200_EINVAL;
+  if (misaligned(x) || misaligned(gx)) return NFPB200_EALIGN;
+  NFP_PROLOGUE(NFPB200_OP_POOLED_MAP_BACKWARD)
+  if (path == 3) return planar_pooled_backward(P, desc->dtype, x, g_gap_nfp, gx, ctx);
+  if (path == 0) return generic_pool_backward(P, desc->dtype, desc->measure, x, nullptr, g_gap_nfp, gx, ctx);
+  // ring / token kernels: a zero g_gap_x (B, C) in the workspace
+  float* zero = static_cast<float*>(workspace);
+  if (cudaError_t e = cudaMemsetAsync(zero, 0, (size_t)P.B * P.C * sizeof(float), ctx.stream)) return (int)e;
+  if (path == 4) return token_run(P, NFPB200_OP_POOL_BACKWARD, x, nullptr, nullptr, gx, zero, g_gap_nfp, nullptr, nullptr, ctx);
+  return stream_pool_backward(P, desc->dtype, x, zero, g_gap_nfp, gx, ctx);
 }
 
 // ---- fused nfp_pooling head -------------------------------------------------------------------------------------

@@ -114,12 +114,18 @@ int token_run(const KParams& P, int op, const void* x, const void* gy, void* y, 
 int token_head_run(const KParams& P, int op, const void* x, const float* proj_w, const float* proj_b, float* out,
                    float* gap_x, float* gap_nfp, const float* g_out, void* gx, const LaunchCtx& ctx);
 
-// planar kernels (cosine, stride 1, dilation 1, pad = R, any map size; map mode only): nfp_planar.cu
+// planar kernels (cosine, stride 1, dilation 1, pad = R, any map size): nfp_planar.cu.  Map mode (NFPB200_OP_FORWARD /
+// _BACKWARD) in the band and table forms; pooled-map mode (GAP(NFP(x)), NFPB200_OP_POOLED_MAP_*) in the band form only
+// (planar_pooled_supported).  Not used by nfpb200_pool_* / nfpb200_head_*.
 bool planar_supported(const KParams& P, int dtype, int measure, int op);
+bool planar_pooled_supported(const KParams& P, int dtype, int measure);
 size_t planar_workspace_bytes(const KParams& P, int dtype, int op);
 int planar_launch_count(const KParams& P, int dtype, int op);
 const char* planar_name(const KParams& P, int dtype, int op);
 int planar_forward(const KParams& P, int dtype, const void* x, void* y, const LaunchCtx& ctx);
 int planar_backward(const KParams& P, int dtype, const void* x, const void* gy, void* gx, const LaunchCtx& ctx);
+int planar_pooled_forward(const KParams& P, int dtype, const void* x, float* gap_nfp, const LaunchCtx& ctx);
+int planar_pooled_backward(const KParams& P, int dtype, const void* x, const float* g_gap_nfp, void* gx,
+                           const LaunchCtx& ctx);
 
 }  // namespace nfp

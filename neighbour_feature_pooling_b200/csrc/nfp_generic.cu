@@ -641,6 +641,8 @@ size_t generic_workspace_bytes(const KParams& P, int dtype, int measure, int op)
     case NFPB200_OP_BACKWARD: return bwd;
     case NFPB200_OP_POOL_FORWARD: return align256(esz * npairs) + fwd;   // [y map][forward scratch]
     case NFPB200_OP_POOL_BACKWARD: return align256(4 * npairs) + bwd;    // [fp32 gy map][backward scratch]
+    case NFPB200_OP_POOLED_MAP_FORWARD: return align256(esz * npairs) + fwd;
+    case NFPB200_OP_POOLED_MAP_BACKWARD: return align256(4 * npairs) + bwd;
   }
   return 0;
 }
@@ -657,6 +659,8 @@ int generic_launch_count(const KParams& P, int dtype, int measure, int op) {
     case NFPB200_OP_BACKWARD: return bwd;
     case NFPB200_OP_POOL_FORWARD: return fwd + 2;
     case NFPB200_OP_POOL_BACKWARD: return bwd + 1;
+    case NFPB200_OP_POOLED_MAP_FORWARD: return fwd + 1;    // no GAP(x) pass
+    case NFPB200_OP_POOLED_MAP_BACKWARD: return bwd + 1;
   }
   return 0;
 }
@@ -685,11 +689,13 @@ int pool_forward_t(const KParams& P, int measure, const T* x, float* gap_x, floa
   int rc = forward_t<T>(P, measure, x, ymap, inner);
   if (rc) return rc;
   const long long px = (long long)P.B * P.C, py = (long long)P.B * P.K;
-  gap_kernel<T><<<blocks_for(px * 32), kThreads, 0, ctx.stream>>>(x, gap_x, P.H * P.W, px);
+  if (gap_x)   // null: GAP(NFP(x)) only (nfpb200_pooled_map_forward)
+    gap_kernel<T><<<blocks_for(px * 32), kThreads, 0, ctx.stream>>>(x, gap_x, P.H * P.W, px);
   gap_kernel<T><<<blocks_for(py * 32), kThreads, 0, ctx.stream>>>(ymap, gap_nfp, P.Ho * P.Wo, py);
   return (int)cudaGetLastError();
 }
 template <typename T>
+// g_gap_x null: the gradient of GAP(NFP(x)) alone (nfpb200_pooled_map_backward; gather_kernel then starts from 0)
 int pool_backward_t(const KParams& P, int measure, const T* x, const float* g_gap_x, const float* g_gap_nfp,
                     T* gx, const LaunchCtx& ctx) {
   const size_t npairs = (size_t)P.B * P.K * P.Ho * P.Wo;

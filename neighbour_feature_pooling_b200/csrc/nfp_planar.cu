@@ -11,6 +11,9 @@
 //           the dots of every band pixel with its whole window, the forward values or the k x k stencil coefficients
 //           (closed form of ATen's cosine_similarity backward, SURVEY.md 8 a3) and the stencil application all run out of
 //           that slab -- x is read from HBM once per launch, the per-pixel tables / coefficient planes never exist.
+//           Pooled mode (GAP(NFP(x)) alone, nfpb200_pooled_map_*): the same band kernels sum the K values per CTA in a
+//           fixed order into per-band partials (+ one tiny kernel that adds them in band order), and the backward reads the
+//           upstream gradient as K fp32 constants per image instead of a map.
 //   scalar  ("planar/table", any shape) separate launches exchanging per-pixel tables through the caller's workspace:
 //             table    T[b][v][p]   v = 0: |x_p|^2,  v = 1..K/2: dot(x_p, x_q) for the "forward" window neighbours q,
 //                                   v = K/2+1: 1 / max(|x_p|, eps)
@@ -21,6 +24,8 @@
 // The window radius is a template parameter: all tap / offset loops are unrolled and the per-thread arrays live in
 // registers.
 #include <stdlib.h>
+
+#include <utility>
 
 #include "nfp_common.cuh"
 #include "nfp_ptx.cuh"
@@ -338,8 +343,16 @@ struct GyView {
     return v;
   }
 };
-template <typename T, int R>
-__device__ __forceinline__ float folded_taps_view(const GyView<T, R>& gv, int pix, const int (&fy)[2 * R + 1],
+// Upstream gradient of the pooled mode (GAP(NFP(x))): d GAP / d y[n][pix] = g_gap_nfp[b][n] / (H W) for every pixel, kept
+// in fp32 whatever the dtype of x (rounded to bf16, its error would be multiplied by per-tap derivatives that cancel to
+// far smaller sums near the norm clamp).  `g` points at the image's K values in shared memory.
+struct GapGradView {
+  const float* g;
+  __device__ __forceinline__ float at(int n, int) const { return g[n]; }
+};
+// View: GyView (map gradient) or GapGradView (pooled mode), anything with at(tap, pixel)
+template <int R, typename View>
+__device__ __forceinline__ float folded_taps_view(const View& gv, int pix, const int (&fy)[2 * R + 1],
                                                   const int (&fx)[2 * R + 1], int oy, int ox) {
   constexpr int k = 2 * R + 1, CTR = R * k + R;
   float s = 0.f;
@@ -386,9 +399,9 @@ __device__ __forceinline__ void band_forward_pixel(const float (&acc)[(2 * R + 1
 
 // the k x k stencil coefficients of one band pixel (closed form of ATen's cosine_similarity backward, gather form):
 // w[o] multiplies x[p + off(o)]; outside the map: 0
-template <typename T, int R, bool INTERIOR>
+template <int R, bool INTERIOR, typename View>
 __device__ __forceinline__ void band_coefficients(const float (&acc)[(2 * R + 1) * (2 * R + 1)], const float* inv, int ps, int p,
-                                                  int pr, int pc, const PlanarParams& q, const GyView<T, R>& gv, float sgn,
+                                                  int pr, int pc, const PlanarParams& q, const View& gv, float sgn,
                                                   float (&w)[(2 * R + 1) * (2 * R + 1)]) {
   constexpr int k = 2 * R + 1, KK = k * k, K = KK - 1, CTR = R * k + R;
   const float t0 = acc[CTR], ip = inv[ps];
@@ -419,14 +432,14 @@ __device__ __forceinline__ void band_coefficients(const float (&acc)[(2 * R + 1)
       const int v = window_pixel(pr, pc, oy - R, ox - R, q);
       w[o] = 0.f;
       if (v >= 0) {
-        const float s = folded_taps_view<T, R>(gv, p, FY[R], FX[R], oy, ox) +
-                        folded_taps_view<T, R>(gv, v, FY[oy], FX[ox], k - 1 - oy, k - 1 - ox);
+        const float s = folded_taps_view<R>(gv, p, FY[R], FX[R], oy, ox) +
+                        folded_taps_view<R>(gv, v, FY[oy], FX[ox], k - 1 - oy, k - 1 - ox);
         w[o] = sgn * s * ip * inv[ps + (v - p)];
         s_dot = fmaf(w[o], acc[o], s_dot);
       }
     }
     // taps of p that land on p itself (replicate padding): y = <p,p>/(N N), gradient 2 G (1/N^2 - y/(N |p|)) x_p
-    sw = 2.f * sgn * folded_taps_view<T, R>(gv, p, FY[R], FX[R], R, R) * ip * ip;
+    sw = 2.f * sgn * folded_taps_view<R>(gv, p, FY[R], FX[R], R, R) * ip * ip;
   }
   w[CTR] = sw - rnp * (s_dot + sw * t0);
 }
@@ -467,9 +480,10 @@ struct BandSplit {
   }
 };
 
-template <typename T, int R>
-__global__ void __launch_bounds__(kThreads) planar_fused_fwd_kernel(const T* __restrict__ x, T* __restrict__ y, PlanarParams q,
-                                                                    int TH, int A) {
+// Forward of one band: emit(yv, p) receives the K values of every band pixel p exactly once (map mode stores them, the
+// pooled mode sums them).
+template <typename T, int R, typename Emit>
+__device__ __forceinline__ void band_forward(const T* __restrict__ x, const PlanarParams& q, int TH, int A, Emit&& emit) {
   using Wn = Win<R>;
   constexpr int k = Wn::k, KK = Wn::KK, K = Wn::K, ESZ = (int)sizeof(T);
   extern __shared__ __align__(128) unsigned char sm[];
@@ -481,18 +495,6 @@ __global__ void __launch_bounds__(kThreads) planar_fused_fwd_kernel(const T* __r
   float* inv = reinterpret_cast<float*>(xs + (size_t)q.C * pitch);
   band_norms<T>(xs, inv, q, r0, A, top, bot, pitch);
   const BandSplit bs(r0, TH, q.H, q.W, R);
-  T* yb0 = y + (size_t)b * (K + q.kin) * q.P;   // multi-radius launch: kin planes of the inner radius in front
-  auto store_y = [&](const float (&yv)[K], int p) {
-#pragma unroll
-    for (int n = 0; n < K; ++n) {
-      const T v = from_f32<T>(yv[n]);
-      yb0[(size_t)(n + q.kin) * q.P + p] = v;
-      if constexpr (R >= 2) {
-        const int n1 = inner_tap(n, R, 1);   // a constant per unrolled n
-        if (n1 >= 0 && q.kin) yb0[(size_t)n1 * q.P + p] = v;
-      }
-    }
-  };
   {
     int off[KK];  // the same for every interior pixel
 #pragma unroll
@@ -504,7 +506,7 @@ __global__ void __launch_bounds__(kThreads) planar_fused_fwd_kernel(const T* __r
       float acc[KK], yv[K];
       band_dots<T, R>(xs + (size_t)ps * ESZ, pitch, q.C, off, acc);
       band_forward_pixel<R, true>(acc, inv, ps, p, pr, pc, q, yv);
-      store_y(yv, p);
+      emit(yv, p);
     }
   }
   for (int u = threadIdx.x; u < bs.n_brd; u += blockDim.x) {
@@ -520,15 +522,80 @@ __global__ void __launch_bounds__(kThreads) planar_fused_fwd_kernel(const T* __r
     }
     band_dots<T, R>(xs + (size_t)ps * ESZ, pitch, q.C, off, acc);
     band_forward_pixel<R, false>(acc, inv, ps, p, pr, pc, q, yv);
-    store_y(yv, p);
+    emit(yv, p);
   }
 }
 
 template <typename T, int R>
-__global__ void __launch_bounds__(kThreads) planar_fused_bwd_kernel(const T* __restrict__ x, const T* __restrict__ gy,
-                                                                    T* __restrict__ gx, PlanarParams q, int TH, int A) {
+__global__ void __launch_bounds__(kThreads) planar_fused_fwd_kernel(const T* __restrict__ x, T* __restrict__ y, PlanarParams q,
+                                                                    int TH, int A) {
+  constexpr int K = Win<R>::K;
+  T* yb0 = y + (size_t)blockIdx.y * (K + q.kin) * q.P;   // multi-radius launch: kin planes of the inner radius in front
+  band_forward<T, R>(x, q, TH, A, [&](const float (&yv)[K], int p) {
+#pragma unroll
+    for (int n = 0; n < K; ++n) {
+      const T v = from_f32<T>(yv[n]);
+      yb0[(size_t)(n + q.kin) * q.P + p] = v;
+      if constexpr (R >= 2) {
+        const int n1 = inner_tap(n, R, 1);   // a constant per unrolled n
+        if (n1 >= 0 && q.kin) yb0[(size_t)n1 * q.P + p] = v;
+      }
+    }
+  });
+}
+
+// Pooled mode: every thread sums the K values of its pixels in registers; the CTA reduces them in a fixed order (shuffle
+// tree per warp, then the warps' sums in warp order) and writes its band's partial sums part[b][band][n].  No atomics.
+template <typename T, int R>
+__global__ void __launch_bounds__(kThreads) planar_pooled_fwd_kernel(const T* __restrict__ x, float* __restrict__ part,
+                                                                     PlanarParams q, int TH, int A) {
+  constexpr int K = Win<R>::K;
+  __shared__ float red[kThreads / 32][K];
+  float s[K];
+#pragma unroll
+  for (int n = 0; n < K; ++n) s[n] = 0.f;
+  band_forward<T, R>(x, q, TH, A, [&](const float (&yv)[K], int) {
+#pragma unroll
+    for (int n = 0; n < K; ++n) s[n] += yv[n];
+  });
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int n = 0; n < K; ++n) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) s[n] += __shfl_xor_sync(0xffffffffu, s[n], o);
+  }
+  if (lane == 0) {
+#pragma unroll
+    for (int n = 0; n < K; ++n) red[warp][n] = s[n];
+  }
+  __syncthreads();
+  if (threadIdx.x < K) {
+    float t = 0.f;
+    for (int w = 0; w < (int)(blockDim.x >> 5); ++w) t += red[w][threadIdx.x];
+    part[((size_t)blockIdx.y * gridDim.x + blockIdx.x) * K + threadIdx.x] = t;
+  }
+}
+
+// gap_nfp[b][n] = (sum of the band partials, in band order) / (H W)
+__global__ void __launch_bounds__(kThreads) planar_pooled_finish_kernel(const float* __restrict__ part,
+                                                                        float* __restrict__ gap_nfp, int n_bands, int K,
+                                                                        int BK, int P) {
+  const int i = blockIdx.x * kThreads + threadIdx.x;
+  if (i >= BK) return;
+  const int b = i / K, n = i - b * K;
+  const float* pb = part + (size_t)b * n_bands * K + n;
+  float t = 0.f;
+  for (int j = 0; j < n_bands; ++j) t += pb[(size_t)j * K];
+  gap_nfp[i] = t / (float)P;
+}
+
+// Backward of one band: gx = stencil(x) with the k x k coefficients of every band pixel, the upstream gradient read
+// through gv (GyView or GapGradView).
+template <typename T, int R, typename View>
+__device__ __forceinline__ void band_backward(const T* __restrict__ x, T* __restrict__ gx, const PlanarParams& q, int TH,
+                                              int A, const View& gv) {
   using Wn = Win<R>;
-  constexpr int k = Wn::k, KK = Wn::KK, K = Wn::K, ESZ = (int)sizeof(T);
+  constexpr int k = Wn::k, KK = Wn::KK, ESZ = (int)sizeof(T);
   extern __shared__ __align__(128) unsigned char sm[];
   uint64_t* bar = reinterpret_cast<uint64_t*>(sm);
   unsigned char* xs = sm + 16;
@@ -538,8 +605,6 @@ __global__ void __launch_bounds__(kThreads) planar_fused_bwd_kernel(const T* __r
   float* inv = reinterpret_cast<float*>(xs + (size_t)q.C * pitch);
   band_norms<T>(xs, inv, q, r0, A, top, bot, pitch);
   const float sgn = q.similarity ? 1.f : -1.f;
-  const T* gyimg = gy + (size_t)b * (K + q.kin) * q.P;   // multi-radius launch: [kin inner planes | K planes] per image
-  const GyView<T, R> gv{gyimg + (size_t)q.kin * q.P, q.kin ? gyimg : nullptr, q.P};
   T* gxb = gx + (size_t)b * q.C * q.P;
   const BandSplit bs(r0, TH, q.H, q.W, 2 * R);
   {
@@ -553,7 +618,7 @@ __global__ void __launch_bounds__(kThreads) planar_fused_bwd_kernel(const T* __r
       float acc[KK], w[KK];
       const unsigned char* pl = xs + (size_t)ps * ESZ;
       band_dots<T, R>(pl, pitch, q.C, off, acc);
-      band_coefficients<T, R, true>(acc, inv, ps, p, pr, pc, q, gv, sgn, w);
+      band_coefficients<R, true>(acc, inv, ps, p, pr, pc, q, gv, sgn, w);
       T* gp = gxb + p;
 #pragma unroll(R == 1 ? 4 : 1)
       for (int c = 0; c < q.C; ++c, pl += pitch, gp += q.P) {
@@ -577,7 +642,7 @@ __global__ void __launch_bounds__(kThreads) planar_fused_bwd_kernel(const T* __r
     }
     const unsigned char* pl = xs + (size_t)ps * ESZ;
     band_dots<T, R>(pl, pitch, q.C, off, acc);
-    band_coefficients<T, R, false>(acc, inv, ps, p, pr, pc, q, gv, sgn, w);
+    band_coefficients<R, false>(acc, inv, ps, p, pr, pc, q, gv, sgn, w);
     T* gp = gxb + p;
 #pragma unroll(R == 1 ? 4 : 1)
     for (int c = 0; c < q.C; ++c, pl += pitch, gp += q.P) {
@@ -587,6 +652,26 @@ __global__ void __launch_bounds__(kThreads) planar_fused_bwd_kernel(const T* __r
       gp[0] = from_f32<T>(a);
     }
   }
+}
+
+template <typename T, int R>
+__global__ void __launch_bounds__(kThreads) planar_fused_bwd_kernel(const T* __restrict__ x, const T* __restrict__ gy,
+                                                                    T* __restrict__ gx, PlanarParams q, int TH, int A) {
+  constexpr int K = Win<R>::K;
+  const T* gyimg = gy + (size_t)blockIdx.y * (K + q.kin) * q.P;   // multi-radius launch: [kin inner planes | K planes] per image
+  const GyView<T, R> gv{gyimg + (size_t)q.kin * q.P, q.kin ? gyimg : nullptr, q.P};
+  band_backward<T, R>(x, gx, q, TH, A, gv);
+}
+
+// Pooled mode: the upstream gradient is K constants per image (GapGradView), so no pixel reads a gradient from memory.
+template <typename T, int R>
+__global__ void __launch_bounds__(kThreads) planar_pooled_bwd_kernel(const T* __restrict__ x,
+                                                                     const float* __restrict__ g_gap_nfp,
+                                                                     T* __restrict__ gx, PlanarParams q, int TH, int A) {
+  constexpr int K = Win<R>::K;
+  __shared__ float gs[K];
+  if (threadIdx.x < K) gs[threadIdx.x] = g_gap_nfp[(size_t)blockIdx.y * K + threadIdx.x] / (float)q.P;   // visible after
+  band_backward<T, R>(x, gx, q, TH, A, GapGradView{gs});                                             // band_fetch's barrier
 }
 
 // Band geometry: TH rows per CTA (a multiple of the row granule g that keeps every bulk copy 16-byte aligned and
@@ -630,10 +715,20 @@ BandPlan fused_plan(const KParams& P, int esz) {
   return bp;
 }
 
+// Without the opt-in a block gets at most 48 KB of dynamic + static shared memory.  static_smem: the kernel's static
+// shared memory (0 for the map kernels; the pooled kernels' reduction table / gradient constants, static_smem_of).
 template <typename K>
-cudaError_t allow_smem(K kern, size_t smem) {
-  return smem > 48 * 1024 ? cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBandSmemMax)
-                          : cudaSuccess;
+cudaError_t allow_smem(K kern, size_t smem, size_t static_smem = 0) {
+  return smem + static_smem > 48 * 1024
+             ? cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBandSmemMax)
+             : cudaSuccess;
+}
+// static shared memory of a kernel as the compiler laid it out (callers keep the answer: it never changes)
+template <typename K>
+std::pair<cudaError_t, size_t> static_smem_of(K kern) {
+  cudaFuncAttributes fa{};
+  const cudaError_t e = cudaFuncGetAttributes(&fa, kern);
+  return {e, fa.sharedSizeBytes};
 }
 
 PlanarParams make(const KParams& P) {
@@ -691,6 +786,55 @@ int backward_r(const KParams& P, const T* x, const T* gy, T* gx, const LaunchCtx
   planar_apply_kernel<T, R><<<grid, kThreads, 0, ctx.stream>>>(x, wd, gx, q);
   return (int)cudaGetLastError();
 }
+// pooled mode (band form only): forward = band partials + finish (2 launches, partials in the workspace), backward = one
+// launch without workspace
+template <typename T, int R>
+int pooled_forward_r(const KParams& P, const T* x, float* gap_nfp, const LaunchCtx& ctx) {
+  const PlanarParams q = make(P);
+  const BandPlan fp = fused_plan(P, (int)sizeof(T));
+  if (!fp.ok) return NFPB200_EUNSUPPORTED;
+  const int n_bands = (q.H + fp.TH - 1) / fp.TH;
+  float* part = reinterpret_cast<float*>(ctx.ws);
+  auto kern = planar_pooled_fwd_kernel<T, R>;
+  static const auto st = static_smem_of(kern);   // one per instantiation
+  if (st.first) return (int)st.first;
+  if (cudaError_t e = allow_smem(kern, fp.smem, st.second)) return (int)e;
+  kern<<<dim3((unsigned)n_bands, (unsigned)q.B), fp.threads, fp.smem, ctx.stream>>>(x, part, q, fp.TH, fp.A);
+  const int BK = q.B * P.K;
+  planar_pooled_finish_kernel<<<(BK + kThreads - 1) / kThreads, kThreads, 0, ctx.stream>>>(part, gap_nfp, n_bands, P.K,
+                                                                                           BK, q.P);
+  return (int)cudaGetLastError();
+}
+template <typename T, int R>
+int pooled_backward_r(const KParams& P, const T* x, const float* g_gap_nfp, T* gx, const LaunchCtx& ctx) {
+  const PlanarParams q = make(P);
+  const BandPlan fp = fused_plan(P, (int)sizeof(T));
+  if (!fp.ok) return NFPB200_EUNSUPPORTED;
+  auto kern = planar_pooled_bwd_kernel<T, R>;
+  static const auto st = static_smem_of(kern);   // one per instantiation
+  if (st.first) return (int)st.first;
+  if (cudaError_t e = allow_smem(kern, fp.smem, st.second)) return (int)e;
+  kern<<<dim3((unsigned)((q.H + fp.TH - 1) / fp.TH), (unsigned)q.B), fp.threads, fp.smem, ctx.stream>>>(
+      x, g_gap_nfp, gx, q, fp.TH, fp.A);
+  return (int)cudaGetLastError();
+}
+template <typename T>
+int pooled_forward_t(const KParams& P, const T* x, float* gap_nfp, const LaunchCtx& ctx) {
+  switch (P.R) {
+    case 1: return pooled_forward_r<T, 1>(P, x, gap_nfp, ctx);
+    case 2: return pooled_forward_r<T, 2>(P, x, gap_nfp, ctx);
+    default: return NFPB200_EUNSUPPORTED;
+  }
+}
+template <typename T>
+int pooled_backward_t(const KParams& P, const T* x, const float* g_gap_nfp, T* gx, const LaunchCtx& ctx) {
+  switch (P.R) {
+    case 1: return pooled_backward_r<T, 1>(P, x, g_gap_nfp, gx, ctx);
+    case 2: return pooled_backward_r<T, 2>(P, x, g_gap_nfp, gx, ctx);
+    default: return NFPB200_EUNSUPPORTED;
+  }
+}
+
 template <typename T>
 int forward_t(const KParams& P, const T* x, T* y, const LaunchCtx& ctx) {
   switch (P.R) {
@@ -719,11 +863,21 @@ bool planar_supported(const KParams& P, int dtype, int measure, int op) {
   if (P.rin) return P.R == 2 && P.rin == 1 && fused_plan(P, dtype == NFPB200_BF16 ? 2 : 4).ok;
   return true;
 }
+// pooled map (GAP(NFP(x)), NFPB200_OP_POOLED_MAP_*): the band form only -- other shapes take the generic kernels
+bool planar_pooled_supported(const KParams& P, int dtype, int measure) {
+  return !P.rin && planar_supported(P, dtype, measure, NFPB200_OP_FORWARD) && fused_plan(P, dtype == NFPB200_BF16 ? 2 : 4).ok;
+}
 size_t planar_workspace_bytes(const KParams& P, int dtype, int op) {
-  if (fused_plan(P, dtype == NFPB200_BF16 ? 2 : 4).ok) return 0;
+  const BandPlan fp = fused_plan(P, dtype == NFPB200_BF16 ? 2 : 4);
+  if (op == NFPB200_OP_POOLED_MAP_FORWARD)   // the band partials (B, n_bands, K)
+    return fp.ok ? align256((size_t)P.B * ((P.H + fp.TH - 1) / fp.TH) * P.K * sizeof(float)) : 0;
+  if (op == NFPB200_OP_POOLED_MAP_BACKWARD) return 0;
+  if (fp.ok) return 0;
   return op == NFPB200_OP_FORWARD ? table_bytes(P) : table_bytes(P) + coef_bytes(P);
 }
 int planar_launch_count(const KParams& P, int dtype, int op) {
+  if (op == NFPB200_OP_POOLED_MAP_FORWARD) return 2;
+  if (op == NFPB200_OP_POOLED_MAP_BACKWARD) return 1;
   if (fused_plan(P, dtype == NFPB200_BF16 ? 2 : 4).ok) return 1;
   return op == NFPB200_OP_FORWARD ? 2 : 3;
 }
@@ -741,6 +895,16 @@ int planar_backward(const KParams& P, int dtype, const void* x, const void* gy, 
   if (dtype == NFPB200_BF16)
     return backward_t<__nv_bfloat16>(P, (const __nv_bfloat16*)x, (const __nv_bfloat16*)gy, (__nv_bfloat16*)gx, ctx);
   return backward_t<float>(P, (const float*)x, (const float*)gy, (float*)gx, ctx);
+}
+int planar_pooled_forward(const KParams& P, int dtype, const void* x, float* gap_nfp, const LaunchCtx& ctx) {
+  if (dtype == NFPB200_BF16) return pooled_forward_t<__nv_bfloat16>(P, (const __nv_bfloat16*)x, gap_nfp, ctx);
+  return pooled_forward_t<float>(P, (const float*)x, gap_nfp, ctx);
+}
+int planar_pooled_backward(const KParams& P, int dtype, const void* x, const float* g_gap_nfp, void* gx,
+                           const LaunchCtx& ctx) {
+  if (dtype == NFPB200_BF16)
+    return pooled_backward_t<__nv_bfloat16>(P, (const __nv_bfloat16*)x, g_gap_nfp, (__nv_bfloat16*)gx, ctx);
+  return pooled_backward_t<float>(P, (const float*)x, g_gap_nfp, (float*)gx, ctx);
 }
 
 }  // namespace nfp

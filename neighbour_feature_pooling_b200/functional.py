@@ -4,6 +4,8 @@
                        (reference models/pooling/nfp.py:132-134): (B,C,H,W) -> (B,K,H',W')
 ``nfp_gap_pair``    -- the fused head of ``nfp_pooling.forward``
                        (reference models/NFP_Pooling.py:27-31): (GAP(x), GAP(NFP(x)))
+``nfp_pooled_similarity`` -- what every stage of the multi-stage head keeps of its map
+                       (reference models/texture_pooling.py:249-256): GAP(NFP(x)) -> (B, K)
 
 Both launch the hand-written sm_100a kernels of libnfp_b200.so on the current
 CUDA stream.  Backward recomputes the similarities from ``x``; nothing but ``x``
@@ -282,6 +284,41 @@ class _NFPGapPair(torch.autograd.Function):
         return gx, None, None
 
 
+class _NFPPooledMap(torch.autograd.Function):
+    """GAP(NFP(x)) (B, K) fp32 without writing the map (nfpb200_pooled_map_forward / _backward)."""
+
+    @staticmethod
+    def forward(ctx, x, cfg, layout=0):
+        desc = _desc_for(x, cfg, layout)
+        gap_nfp = torch.empty((x.shape[0], cfg.out_channels), dtype=torch.float32, device=x.device)
+        _trace(desc, _capi.OP_POOLED_MAP_FORWARD, "pooled map")
+        with torch.cuda.device(x.device):
+            ws, ws_ptr, ws_n = _workspace(desc, _capi.OP_POOLED_MAP_FORWARD, x.device)
+            rc = _capi.load().nfpb200_pooled_map_forward(ctypes.byref(desc), x.data_ptr(), gap_nfp.data_ptr(),
+                                                         ws_ptr, ws_n, _stream(x.device))
+        _capi.check(rc, "nfpb200_pooled_map_forward")
+        ctx.save_for_backward(x)
+        ctx.cfg = cfg
+        ctx.layout = layout
+        return gap_nfp
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, g_gap_nfp):
+        (x,) = ctx.saved_tensors
+        desc = _desc_for(x, ctx.cfg, ctx.layout)
+        if _X_STABLE_HINT:
+            desc.path |= _capi.HINT_X_STABLE
+        g_gap_nfp = g_gap_nfp.float().contiguous()   # fp32 whatever the dtype of x
+        gx = _empty_like_layout(x, ctx.layout)
+        with torch.cuda.device(x.device):
+            ws, ws_ptr, ws_n = _workspace(desc, _capi.OP_POOLED_MAP_BACKWARD, x.device)
+            rc = _capi.load().nfpb200_pooled_map_backward(ctypes.byref(desc), x.data_ptr(), g_gap_nfp.data_ptr(),
+                                                          gx.data_ptr(), ws_ptr, ws_n, _stream(x.device))
+        _capi.check(rc, "nfpb200_pooled_map_backward")
+        return gx, None, None
+
+
 class _NFPHead(torch.autograd.Function):
     """out = GAP(x) * (W GAP(NFP(x)) + b) in ONE launch each way (nfpb200_head_forward / _backward); the projection's
     parameter gradients are three tiny PyTorch ops on the (B, C) / (B, K) tensors the forward leaves behind."""
@@ -453,6 +490,20 @@ def nfp_gap_pair(x: torch.Tensor, cfg: NFPConfig):
     return gx.to(x.dtype), gn.to(out_dtype)
 
 
+def nfp_pooled_similarity(x: torch.Tensor, cfg: NFPConfig) -> torch.Tensor:
+    """``adaptive_avg_pool2d(nfp_similarity(x, cfg), 1).flatten(1)`` -> (B, k*k-1), differentiable w.r.t. ``x``,
+    without writing the similarity map: what each stage of the reference's multi-stage head keeps of its map
+    (models/texture_pooling.py:249-256).  The result has the map's dtype: float32 under CUDA autocast, else the dtype of
+    ``x``; the kernels accumulate in fp32 either way.  Only ``x`` is saved for the backward."""
+    if x.device.type != "cuda":
+        _reject_cpu(x)
+    if x.dim() == 4:
+        _check_geometry(x.shape[2], x.shape[3], cfg)
+    xk, out_dtype, layout = _prepare(x, cfg)
+    gn = _NFPPooledMap.apply(xk, cfg, layout)   # fp32
+    return gn if gn.dtype == out_dtype else gn.to(out_dtype)
+
+
 def describe(x_shape, dtype: torch.dtype, cfg: NFPConfig, op: int = _capi.OP_FORWARD, layout: int = 0) -> str:
     """Name of the kernel path a problem would take (for tests / bench reporting)."""
     B, C, H, W = x_shape
@@ -462,5 +513,5 @@ def describe(x_shape, dtype: torch.dtype, cfg: NFPConfig, op: int = _capi.OP_FOR
     return _capi.describe_path(desc, op)
 
 
-__all__ = ["NFPConfig", "nfp_similarity", "nfp_gap_pair", "nfp_head", "nfp_multi_radius", "multi_radius_fusable", "shape_probe", "conv_output_size", "describe",
+__all__ = ["NFPConfig", "nfp_similarity", "nfp_gap_pair", "nfp_pooled_similarity", "nfp_head", "nfp_multi_radius", "multi_radius_fusable", "shape_probe", "conv_output_size", "describe",
            "replace", "math"]

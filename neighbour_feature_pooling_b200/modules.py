@@ -271,5 +271,45 @@ def unfuse_multi_radius(blocks):
         b.__dict__.pop("forward", None)
 
 
+class _PooledForward:
+    """``forward`` of a layer fused by ``fuse_pooled_nfp``: ``GAP(NFP(x))`` as a ``(B, K, 1, 1)`` tensor on CUDA, the
+    stock forward for every other input.  A module-level class holding the layer (not a closure), so that ``pickle`` /
+    ``torch.save`` and ``copy.deepcopy`` round-trip a fused layer, and a copy's forward runs on the copy."""
+
+    def __init__(self, layer):
+        self.layer = layer
+
+    def __call__(self, x):
+        layer = self.layer
+        if x.device.type != "cuda":   # CPU shape probes and CPU errors: exactly as the stock layer answers them
+            return type(layer).forward(layer, x)
+        return NF.nfp_pooled_similarity(x, layer.config)[:, :, None, None]
+
+
+def fuse_pooled_nfp(layer) -> bool:
+    """Make a stock ``NFPPooling`` / ``EnhancedNFPPooling`` layer return ``adaptive_avg_pool2d(NFP(x), 1)``, shape
+    ``(B, K, 1, 1)``, computed without writing the similarity map (``functional.nfp_pooled_similarity``).
+
+    For callers that global-pool the layer's output right away, as every stage of the reference's
+    ``MobileNetV3_MultiStageNFP`` does (models/texture_pooling.py:249-256: ``adaptive_avg_pool2d(nfp(x), (1, 1))`` then
+    ``.view(B, -1)``): their own pool and view are then exact identities, so the unmodified head gets the same values.
+    It is valid ONLY for such callers: anything else that reads the layer's output sees a 1 x 1 map.  Forward hooks
+    registered on the layer after this call see the ``(B, K, 1, 1)`` tensor.  CPU inputs (constructor shape probes
+    included) take the stock forward.
+
+    Only the instance's ``forward`` attribute is set; parameters, ``state_dict`` keys and the module tree are unchanged,
+    and ``unfuse_pooled_nfp`` restores the stock forward.  Returns False and changes nothing when the layer is not a
+    stock cosine layer (a subclass, a re-bound ``forward`` / ``similarity_measure``, hooks, another measure)."""
+    if not _stock(layer) or layer.config.measure != "cosine":
+        return False
+    layer.forward = _PooledForward(layer)
+    return True
+
+
+def unfuse_pooled_nfp(layer):
+    if isinstance(layer.__dict__.get("forward"), _PooledForward):
+        del layer.__dict__["forward"]
+
+
 __all__ = ["NFPPooling", "EnhancedNFPPooling", "nfp_pooling", "MultiRadiusNFP", "fuse_multi_radius",
-           "unfuse_multi_radius"]
+           "unfuse_multi_radius", "fuse_pooled_nfp", "unfuse_pooled_nfp"]
