@@ -21,9 +21,19 @@
  *                             MultiRadiusNFPHead evaluated together (models/nfp_heads.py:86-93,111-112)
  *
  * Conventions
- *   - plain C types only; every buffer is caller-owned DEVICE memory (NCHW,
- *     contiguous, 16-byte aligned), the library keeps no pointer after a call
- *     returns and never allocates on the hot path;
+ *   - plain C types only; every buffer is caller-owned DEVICE memory (NCHW
+ *     contiguous unless desc->layout says otherwise), the library keeps no
+ *     pointer after a call returns and never allocates on the hot path;
+ *   - alignment, checked before any CUDA call (NFPB200_EALIGN below it):
+ *       16 bytes: x, y, gy, gx, proj_w and a non-null workspace (bulk copies
+ *                 and 16-byte vector accesses);
+ *        4 bytes: the fp32 vectors gap_x, gap_nfp, g_gap_x, g_gap_nfp, out,
+ *                 g_out and proj_b (read and written one float at a time);
+ *     nothing else is assumed: no buffer needs more than its own size;
+ *   - the library reads only the bytes its inputs span and writes only the
+ *     bytes its outputs span, never an input, and never an element of the
+ *     workspace beyond nfpb200_workspace_bytes; the workspace's contents on
+ *     entry do not affect any result;
  *   - every call is asynchronous on `stream` (a cudaStream_t passed as void*);
  *   - return value: 0 on success, a negative NFPB200_E* code for argument
  *     errors, a positive cudaError_t for CUDA failures.  No C++ exception
@@ -129,7 +139,7 @@ enum {
   NFPB200_EWORKSPACE = -4,   /* workspace too small / null */
   NFPB200_EUNSUPPORTED = -5, /* e.g. NFPB200_PATH_FUSED on a problem the fused kernels do not cover */
   NFPB200_EDEVICE = -6,      /* the current device is not sm_100 */
-  NFPB200_EALIGN = -7        /* a tensor pointer is not 16-byte aligned (the fused kernels move data with TMA) */
+  NFPB200_EALIGN = -7        /* a pointer below its alignment (Conventions above), or a batch stride not a multiple of 8 */
 };
 
 /* Constructor arguments of NFPPooling (nfp.py:16-18) plus the tensor shape. */
@@ -161,7 +171,8 @@ typedef struct nfpb200_desc {
                                planes, the planar row-band kernels; anything else: NFPB200_EUNSUPPORTED, and the caller
                                issues one launch per radius */
   int64_t x_batch_stride;   /* NHWC only: elements between consecutive images of x; 0 = dense (H*W*C); multiple of 8 */
-  int64_t gx_batch_stride;  /* NHWC only: the same for gx */
+  int64_t gx_batch_stride;  /* NHWC only: the same for gx.  Above the dense stride, nothing is written between images:
+                               the elements from H*W*C to gx_batch_stride of each image keep their contents */
 } nfpb200_desc_t;
 
 int nfpb200_abi_version(void);
@@ -190,21 +201,24 @@ int nfpb200_describe_path(const nfpb200_desc_t* desc, int32_t op, char* buf, siz
 /* Number of kernel launches the op issues on `stream` (bench.py's gpu_launches), counting a cudaMemsetAsync as one. */
 int nfpb200_launch_count(const nfpb200_desc_t* desc, int32_t op, int32_t* launches);
 
-/* y (B, K, H', W') = NFP(x)   (desc->inner_R = r > 0: (B, K_r + K, H, W), see nfpb200_desc_t).  */
+/* y (B, K, H', W') = NFP(x)   (desc->inner_R = r > 0: (B, K_r + K, H, W), see nfpb200_desc_t).
+ * Alignment: x, y, workspace 16 bytes. */
 int nfpb200_forward(const nfpb200_desc_t* desc, const void* x, void* y,
                     void* workspace, size_t workspace_bytes, void* stream);
 
 /* gx (B, C, H, W) = d<gy, NFP(x)>/dx ; similarities are recomputed from x, nothing is saved by forward.
- * (desc->inner_R = r > 0: gy is (B, K_r + K, H, W) and gx the sum of both layers' input gradients.) */
+ * (desc->inner_R = r > 0: gy is (B, K_r + K, H, W) and gx the sum of both layers' input gradients.)
+ * Alignment: x, gy, gx, workspace 16 bytes. */
 int nfpb200_backward(const nfpb200_desc_t* desc, const void* x, const void* gy, void* gx,
                      void* workspace, size_t workspace_bytes, void* stream);
 
 /* Fused head of nfp_pooling (NFP_Pooling.py:27-31): gap_x (B, C) = mean_hw x, gap_nfp (B, K) = mean_hw NFP(x).
- * Both outputs are fp32 regardless of desc->dtype. */
+ * Both outputs are fp32 regardless of desc->dtype.  Alignment: x, workspace 16 bytes; gap_x, gap_nfp 4 bytes. */
 int nfpb200_pool_forward(const nfpb200_desc_t* desc, const void* x, float* gap_x, float* gap_nfp,
                          void* workspace, size_t workspace_bytes, void* stream);
 
-/* gx = d(<g_gap_x, GAP(x)> + <g_gap_nfp, GAP(NFP(x))>)/dx ; g_* are fp32 (B, C) and (B, K). */
+/* gx = d(<g_gap_x, GAP(x)> + <g_gap_nfp, GAP(NFP(x))>)/dx ; g_* are fp32 (B, C) and (B, K).
+ * Alignment: x, gx, workspace 16 bytes; g_gap_x, g_gap_nfp 4 bytes. */
 int nfpb200_pool_backward(const nfpb200_desc_t* desc, const void* x, const float* g_gap_x,
                           const float* g_gap_nfp, void* gx,
                           void* workspace, size_t workspace_bytes, void* stream);
@@ -221,14 +235,15 @@ int nfpb200_pool_backward(const nfpb200_desc_t* desc, const void* x, const float
  *     workspace, then a kernel that sums them in band order and divides by H' W'); backward: 1 launch, no workspace;
  *   - anything else, and NFPB200_PATH_GENERIC: the generic kernels' pooled mode ("generic/pairs") without its GAP(x) part.
  * NFPB200_PATH_FUSED: the ring / token kernels or NFPB200_EUNSUPPORTED.  No float atomics on any path: results are
- * bit-identical from run to run. */
+ * bit-identical from run to run.  Alignment: x, workspace 16 bytes; gap_nfp 4 bytes. */
 int nfpb200_pooled_map_forward(const nfpb200_desc_t* desc, const void* x, float* gap_nfp,
                                void* workspace, size_t workspace_bytes, void* stream);
 
 /* gx = d<g_gap_nfp, GAP(NFP(x))>/dx ; g_gap_nfp is fp32 (B, K).  Same paths as the forward.  The ring and token kernels
  * read a zero (B, C) g_gap_x from the workspace, which this call clears first with one cudaMemsetAsync (2 launches in
  * all); the row-band kernels (1 launch) keep g_gap_nfp / (H' W') in fp32 registers and shared memory and read no per-pixel
- * gradient; the generic kernels expand it to an fp32 map in the workspace. */
+ * gradient; the generic kernels expand it to an fp32 map in the workspace.
+ * Alignment: x, gx, workspace 16 bytes; g_gap_nfp 4 bytes. */
 int nfpb200_pooled_map_backward(const nfpb200_desc_t* desc, const void* x, const float* g_gap_nfp, void* gx,
                                 void* workspace, size_t workspace_bytes, void* stream);
 
@@ -239,7 +254,8 @@ int nfpb200_pooled_map_backward(const nfpb200_desc_t* desc, const void* x, const
  * them for the parameter gradients (d proj_w = (g_out * gap_x)^T gap_nfp, d proj_b = sum_b g_out * gap_x), which stay
  * on the caller's side.  Served by the fused NCHW ring kernels and the channels-last token kernels (cosine, pad = R, stride 1);
  * nfpb200_head_supported() returns NFPB200_OK when both directions are, NFPB200_EUNSUPPORTED otherwise -- then compose
- * nfpb200_pool_forward / _backward with the projection on the caller's side. */
+ * nfpb200_pool_forward / _backward with the projection on the caller's side.
+ * Alignment: x, gx, proj_w 16 bytes; proj_b, out, gap_x, gap_nfp, g_out 4 bytes. */
 int nfpb200_head_supported(const nfpb200_desc_t* desc);
 int nfpb200_head_forward(const nfpb200_desc_t* desc, const void* x, const float* proj_w, const float* proj_b, float* out,
                          float* gap_x, float* gap_nfp, void* stream);

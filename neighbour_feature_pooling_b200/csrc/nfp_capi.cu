@@ -138,7 +138,9 @@ const char* nfpb200_status_string(int status) {
     case NFPB200_EWORKSPACE: return "workspace missing or too small (see nfpb200_workspace_bytes)";
     case NFPB200_EUNSUPPORTED: return "the fused kernels do not cover this problem (use NFPB200_PATH_AUTO)";
     case NFPB200_EDEVICE: return "current CUDA device is not compute capability 10.x (B200, sm_100a)";
-    case NFPB200_EALIGN: return "tensor pointers must be 16-byte aligned";
+    case NFPB200_EALIGN:
+      return "misaligned pointer: x, y, gy, gx, proj_w and the workspace must be 16-byte aligned, the fp32 vectors "
+             "4-byte aligned";
     default: break;
   }
   if (status > 0) return cudaGetErrorString((cudaError_t)status);
@@ -197,24 +199,30 @@ int nfpb200_launch_count(const nfpb200_desc_t* desc, int32_t op, int32_t* launch
   return NFPB200_OK;
 }
 
+// The alignment each pointer needs (include/nfp_b200.h), checked before any CUDA call.  16 bytes: x, y, gy, gx and
+// proj_w, which the kernels move with bulk copies and 16-byte vector accesses, and the workspace.  4 bytes: the fp32
+// vectors gap_x, gap_nfp, g_gap_x, g_gap_nfp, out, g_out and proj_b, which every kernel reads and writes one float at a
+// time (the ring kernels' bulk copy of a g_gap_x row is only taken when the row is 16-byte aligned and sized).
 static inline bool misaligned(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) != 0; }
+static inline bool misaligned_f32(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 3u) != 0; }
 
+// argument errors (descriptor, path, workspace size) are host-only and come before the first CUDA call
 #define NFP_PROLOGUE(OP)                                                                      \
   KParams P;                                                                                  \
   int rc = make_params(desc, &P);                                                             \
-  if (rc) return rc;                                                                          \
-  rc = check_device();                                                                        \
   if (rc) return rc;                                                                          \
   const int path = choose_path(desc, P, OP);                                                  \
   if (path < 0) return path;                                                                  \
   const size_t need = path_workspace_bytes(path, desc, P, OP);                                \
   if (need > 0 && (!workspace || workspace_bytes < need)) return NFPB200_EWORKSPACE;          \
+  rc = check_device();                                                                        \
+  if (rc) return rc;                                                                          \
   LaunchCtx ctx{(cudaStream_t)stream, workspace, workspace_bytes};
 
 int nfpb200_forward(const nfpb200_desc_t* desc, const void* x, void* y, void* workspace, size_t workspace_bytes,
                     void* stream) {
   if (!x || !y) return NFPB200_EINVAL;
-  if (misaligned(x) || misaligned(y)) return NFPB200_EALIGN;
+  if (misaligned(x) || misaligned(y) || misaligned(workspace)) return NFPB200_EALIGN;
   NFP_PROLOGUE(NFPB200_OP_FORWARD)
   if (P.y_f32 && path != 2 && path != 4) return NFPB200_EUNSUPPORTED;
   if (path == 4) return token_run(P, NFPB200_OP_FORWARD, x, nullptr, y, nullptr, nullptr, nullptr, nullptr, nullptr, ctx);
@@ -226,7 +234,7 @@ int nfpb200_forward(const nfpb200_desc_t* desc, const void* x, void* y, void* wo
 int nfpb200_backward(const nfpb200_desc_t* desc, const void* x, const void* gy, void* gx, void* workspace,
                      size_t workspace_bytes, void* stream) {
   if (!x || !gy || !gx) return NFPB200_EINVAL;
-  if (misaligned(x) || misaligned(gy) || misaligned(gx)) return NFPB200_EALIGN;
+  if (misaligned(x) || misaligned(gy) || misaligned(gx) || misaligned(workspace)) return NFPB200_EALIGN;
   NFP_PROLOGUE(NFPB200_OP_BACKWARD)
   if (path == 4) return token_run(P, NFPB200_OP_BACKWARD, x, gy, nullptr, gx, nullptr, nullptr, nullptr, nullptr, ctx);
   if (path == 3) return planar_backward(P, desc->dtype, x, gy, gx, ctx);
@@ -237,7 +245,7 @@ int nfpb200_backward(const nfpb200_desc_t* desc, const void* x, const void* gy, 
 int nfpb200_pool_forward(const nfpb200_desc_t* desc, const void* x, float* gap_x, float* gap_nfp, void* workspace,
                          size_t workspace_bytes, void* stream) {
   if (!x || !gap_x || !gap_nfp) return NFPB200_EINVAL;
-  if (misaligned(x)) return NFPB200_EALIGN;
+  if (misaligned(x) || misaligned_f32(gap_x) || misaligned_f32(gap_nfp) || misaligned(workspace)) return NFPB200_EALIGN;
   NFP_PROLOGUE(NFPB200_OP_POOL_FORWARD)
   if (path == 4) return token_run(P, NFPB200_OP_POOL_FORWARD, x, nullptr, nullptr, nullptr, nullptr, nullptr, gap_x, gap_nfp, ctx);
   if (path == 2) return stream_pool_forward(P, desc->dtype, x, gap_x, gap_nfp, ctx);
@@ -247,7 +255,8 @@ int nfpb200_pool_forward(const nfpb200_desc_t* desc, const void* x, float* gap_x
 int nfpb200_pool_backward(const nfpb200_desc_t* desc, const void* x, const float* g_gap_x, const float* g_gap_nfp,
                           void* gx, void* workspace, size_t workspace_bytes, void* stream) {
   if (!x || !g_gap_x || !g_gap_nfp || !gx) return NFPB200_EINVAL;
-  if (misaligned(x) || misaligned(gx)) return NFPB200_EALIGN;
+  if (misaligned(x) || misaligned(gx) || misaligned_f32(g_gap_x) || misaligned_f32(g_gap_nfp) || misaligned(workspace))
+    return NFPB200_EALIGN;
   NFP_PROLOGUE(NFPB200_OP_POOL_BACKWARD)
   if (path == 4) return token_run(P, NFPB200_OP_POOL_BACKWARD, x, nullptr, nullptr, gx, g_gap_x, g_gap_nfp, nullptr, nullptr, ctx);
   if (path == 2) return stream_pool_backward(P, desc->dtype, x, g_gap_x, g_gap_nfp, gx, ctx);
@@ -258,7 +267,7 @@ int nfpb200_pool_backward(const nfpb200_desc_t* desc, const void* x, const float
 int nfpb200_pooled_map_forward(const nfpb200_desc_t* desc, const void* x, float* gap_nfp, void* workspace,
                                size_t workspace_bytes, void* stream) {
   if (!x || !gap_nfp) return NFPB200_EINVAL;
-  if (misaligned(x)) return NFPB200_EALIGN;
+  if (misaligned(x) || misaligned_f32(gap_nfp) || misaligned(workspace)) return NFPB200_EALIGN;
   NFP_PROLOGUE(NFPB200_OP_POOLED_MAP_FORWARD)
   if (path == 3) return planar_pooled_forward(P, desc->dtype, x, gap_nfp, ctx);
   float* gap_x = static_cast<float*>(workspace);   // ring / token kernels: GAP(x) is written to the workspace
@@ -270,7 +279,7 @@ int nfpb200_pooled_map_forward(const nfpb200_desc_t* desc, const void* x, float*
 int nfpb200_pooled_map_backward(const nfpb200_desc_t* desc, const void* x, const float* g_gap_nfp, void* gx,
                                 void* workspace, size_t workspace_bytes, void* stream) {
   if (!x || !g_gap_nfp || !gx) return NFPB200_EINVAL;
-  if (misaligned(x) || misaligned(gx)) return NFPB200_EALIGN;
+  if (misaligned(x) || misaligned(gx) || misaligned_f32(g_gap_nfp) || misaligned(workspace)) return NFPB200_EALIGN;
   NFP_PROLOGUE(NFPB200_OP_POOLED_MAP_BACKWARD)
   if (path == 3) return planar_pooled_backward(P, desc->dtype, x, g_gap_nfp, gx, ctx);
   if (path == 0) return generic_pool_backward(P, desc->dtype, desc->measure, x, nullptr, g_gap_nfp, gx, ctx);
@@ -305,7 +314,9 @@ int nfpb200_head_supported(const nfpb200_desc_t* desc) {
 int nfpb200_head_forward(const nfpb200_desc_t* desc, const void* x, const float* proj_w, const float* proj_b, float* out,
                          float* gap_x, float* gap_nfp, void* stream) {
   if (!x || !proj_w || !out || !gap_x || !gap_nfp) return NFPB200_EINVAL;
-  if (misaligned(x) || misaligned(proj_w)) return NFPB200_EALIGN;
+  if (misaligned(x) || misaligned(proj_w) || misaligned_f32(proj_b) || misaligned_f32(out) || misaligned_f32(gap_x) ||
+      misaligned_f32(gap_nfp))
+    return NFPB200_EALIGN;
   KParams P;
   int rc = make_params(desc, &P);
   if (rc) return rc;
@@ -322,7 +333,9 @@ int nfpb200_head_forward(const nfpb200_desc_t* desc, const void* x, const float*
 int nfpb200_head_backward(const nfpb200_desc_t* desc, const void* x, const float* proj_w, const float* proj_b,
                           const float* gap_x, const float* gap_nfp, const float* g_out, void* gx, void* stream) {
   if (!x || !proj_w || !gap_x || !gap_nfp || !g_out || !gx) return NFPB200_EINVAL;
-  if (misaligned(x) || misaligned(gx) || misaligned(proj_w)) return NFPB200_EALIGN;
+  if (misaligned(x) || misaligned(gx) || misaligned(proj_w) || misaligned_f32(proj_b) || misaligned_f32(gap_x) ||
+      misaligned_f32(gap_nfp) || misaligned_f32(g_out))
+    return NFPB200_EALIGN;
   KParams P;
   int rc = make_params(desc, &P);
   if (rc) return rc;

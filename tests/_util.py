@@ -166,3 +166,90 @@ def elem_grad_err(got, want, geo, dtype=torch.float32):
 def worst(errs, k=4):
     """The k largest entries of a grad_errs() table, for assertion messages."""
     return sorted(errs.items(), key=lambda kv: -kv[1])[:k]
+
+
+# ---- guarded buffers (tests/test_abi_contract_*.py) ------------------------------------------------------------------
+# A typed body inside one larger uint8 allocation, with a lead and a tail guard.  Inputs: body = data, guards = quiet
+# NaN, so a read past either end that feeds a result turns it into NaN.  Outputs and the workspace: body and guards
+# hold a NaN with a recognisable payload (SENTINEL), so a write outside the body, and an element never written, show.
+GUARD_BYTES = 256 * 1024   # larger than any single transfer of any path (a ring chunk, a band slab)
+QNAN = {torch.float32: 0x7FC00000, torch.bfloat16: 0x7FC0, torch.uint8: 0x7F}
+SENTINEL = {torch.float32: 0x7FA5A5A5, torch.bfloat16: 0x7FA5, torch.uint8: 0xA5}
+_BITS = {torch.float32: torch.int32, torch.bfloat16: torch.int16, torch.uint8: torch.uint8}
+
+
+def bits(t):
+    """The raw bit patterns of a float tensor (for exact, NaN-aware comparison)."""
+    return t.contiguous().view(_BITS[t.dtype])
+
+
+def fill_bits(t, pattern):
+    """Fill a float tensor with one bit pattern (e.g. a NaN with a payload, which a float fill cannot express)."""
+    esz = t.element_size()
+    if _BITS[t.dtype] is not torch.uint8 and pattern >= 2 ** (8 * esz - 1):
+        pattern -= 2 ** (8 * esz)   # the same bits as a signed integer
+    t.view(_BITS[t.dtype]).fill_(pattern)
+
+
+class Guarded:
+    """`numel` elements of `dtype` at byte address % 512 == `place`, GUARD_BYTES of guard on each side.
+
+    kind "input": body = `data` (flat, NaN where `data` is NaN), guards quiet NaN; the whole allocation must stay
+    bit-unchanged.  kind "output" / "workspace": body and guards SENTINEL; the guards must stay unchanged, and so must
+    every body element outside `written` (a flat bool mask, default all), while no element inside it may still hold
+    SENTINEL after the call."""
+
+    def __init__(self, numel, dtype, device, kind, data=None, place=16, written=None, guard=GUARD_BYTES):
+        esz = torch.empty(0, dtype=dtype).element_size()
+        assert place % esz == 0 and kind in ("input", "output", "workspace")
+        self.dtype, self.kind, self.numel = dtype, kind, numel
+        self.raw = torch.empty(2 * guard + numel * esz + 512 + 16, dtype=torch.uint8, device=device)
+        lead = guard + (place - (self.raw.data_ptr() + guard)) % 512
+        self.lo, self.hi = lead, lead + numel * esz
+        fill = QNAN[dtype] if kind == "input" else SENTINEL[dtype]
+        n_el = self.raw.numel() // esz
+        fill_bits(self.raw[:n_el * esz].view(dtype), fill)
+        self.raw[n_el * esz:].fill_(0xFF)
+        if data is not None:
+            self.body.copy_(data.reshape(-1).to(device, dtype))
+        self.written = written
+        self.snapshot = self.raw.clone()
+
+    @property
+    def body(self):
+        return self.raw[self.lo:self.hi].view(self.dtype)
+
+    def ptr(self):
+        return self.raw.data_ptr() + self.lo
+
+    def problems(self, name):
+        """What the last call did wrong to this buffer (empty list: nothing)."""
+        out = []
+        raw, ref = self.raw, self.snapshot
+        for side, a, b in (("lead guard", 0, self.lo), ("tail guard", self.hi, raw.numel())):
+            bad = (raw[a:b] != ref[a:b]).nonzero()
+            if bad.numel():
+                out.append(f"{name}: {side} changed at {bad.numel()} bytes, first at {int(bad[0]) - (self.lo if a else a)}"
+                           f" bytes from the body")
+        if self.kind == "input":
+            bad = (raw[self.lo:self.hi] != ref[self.lo:self.hi]).nonzero()
+            if bad.numel():
+                out.append(f"{name}: input body written at {bad.numel()} bytes, first at byte {int(bad[0])}")
+            return out
+        got = bits(self.body)
+        want = bits(ref[self.lo:self.hi].view(self.dtype))
+        wr = self.written if self.written is not None else torch.ones(self.numel, dtype=torch.bool)
+        wr = wr.to(got.device)
+        if self.kind == "output":
+            left = ((got == want) & wr).nonzero()
+            if left.numel():
+                out.append(f"{name}: {left.numel()} elements never written, first at {int(left[0])}")
+        gap = ((got != want) & ~wr).nonzero()
+        if gap.numel():
+            out.append(f"{name}: {gap.numel()} elements written outside the output, first at {int(gap[0])}")
+        return out
+
+
+def guard_problems(bufs):
+    """Every problem of every buffer of a call: {name: Guarded} -> list of messages."""
+    return [m for name, g in bufs.items() if g is not None for m in g.problems(name)]
