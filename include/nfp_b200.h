@@ -55,10 +55,15 @@
 extern "C" {
 #endif
 
-#define NFPB200_ABI_VERSION 4
+#define NFPB200_ABI_VERSION 5
 
-/* element type of x / y / gy / gx.  Accumulation is always fp32. */
-enum { NFPB200_F32 = 0, NFPB200_BF16 = 1 };
+/* element type of x / y / gy / gx.  Accumulation is always fp32; every GAP and head vector is fp32 whatever the dtype.
+ * NFPB200_F16 (IEEE half, ABI v5) is served by two kernel families only: the NCHW streaming-ring kernels ("fused/stream_*")
+ * and the channels-last token kernels ("fused/token_*"), for every op they carry (map, pooled, fused head, inner_R,
+ * pooled map), on exactly the problems a bf16 descriptor sends to them.  Any other fp16 problem -- what bf16 sends to the
+ * planar, generic or cluster-split kernels, and NFPB200_PATH_GENERIC -- returns NFPB200_EUNSUPPORTED: the caller widens
+ * to fp32.  fp16 results are rounded to nearest: a gradient beyond 65504 is +-inf, as a narrowing copy makes it. */
+enum { NFPB200_F32 = 0, NFPB200_BF16 = 1, NFPB200_F16 = 2 };
 
 /* torch.nn.Conv2d padding_mode (nfp.py:17, default 'reflect') */
 enum { NFPB200_PAD_ZEROS = 0, NFPB200_PAD_REFLECT = 1, NFPB200_PAD_REPLICATE = 2, NFPB200_PAD_CIRCULAR = 3 };
@@ -91,7 +96,7 @@ enum {
   NFPB200_LAYOUT_NHWC = 1   /* x[b][h][w][c]: channels of a pixel contiguous, pixels dense, batch stride free.  This is a
                                torch channels_last map and the ViT head's token view (models/texture_pooling.py:181-188:
                                feats[:, 1:].transpose(1, 2).reshape(B, C, H, W), strides (197*C, 1, W*C, C)); served by
-                               the tensor-core "fused/token" kernels (bf16, cosine, pad = R, stride 1) -- anything else
+                               the tensor-core "fused/token" kernels (bf16 / fp16, cosine, pad = R, stride 1) -- anything else
                                returns NFPB200_EUNSUPPORTED and the caller repacks to NCHW */
 };
 
@@ -115,9 +120,9 @@ enum {
  * preceding launch itself. */
 #define NFPB200_HINT_X_STABLE 0x100
 
-/* Optional flag, OR-ed into nfpb200_desc_t.path, for nfpb200_forward with dtype = NFPB200_BF16: y is written as fp32
- * (what the reference produces under torch.autocast on CUDA, where F.cosine_similarity runs in fp32 on the bf16
- * neighbours, nfp.py:152-156).  Honoured by the fused kernels; other paths return NFPB200_EUNSUPPORTED. */
+/* Optional flag, OR-ed into nfpb200_desc_t.path, for nfpb200_forward with dtype = NFPB200_BF16 or NFPB200_F16: y is
+ * written as fp32 (what the reference produces under torch.autocast on CUDA, where F.cosine_similarity runs in fp32 on
+ * the bf16 / fp16 neighbours, nfp.py:152-156).  Honoured by the fused kernels; other paths return NFPB200_EUNSUPPORTED. */
 #define NFPB200_FLAG_Y_F32 0x200
 
 /* operations, for nfpb200_workspace_bytes / nfpb200_describe_path / nfpb200_launch_count */
@@ -145,7 +150,7 @@ enum {
 /* Constructor arguments of NFPPooling (nfp.py:16-18) plus the tensor shape. */
 typedef struct nfpb200_desc {
   int32_t struct_bytes;     /* = sizeof(nfpb200_desc_t); ABI guard */
-  int32_t dtype;            /* NFPB200_F32 | NFPB200_BF16 */
+  int32_t dtype;            /* NFPB200_F32 | NFPB200_BF16 | NFPB200_F16 */
   int32_t B, C, H, W;       /* x is (B, C, H, W) contiguous */
   int32_t R;                /* radius; kernel_size = 2R+1, out_channels K = (2R+1)^2 - 1 (nfp.py:38-39) */
   int32_t stride;
@@ -228,7 +233,7 @@ int nfpb200_pool_backward(const nfpb200_desc_t* desc, const void* x, const float
  * adaptive_avg_pool2d(nfp(x), (1, 1)).view(B, -1)); these entry points compute only that, without writing the map:
  *   gap_nfp (B, K) fp32 = mean over the H' x W' output pixels of NFP(x), whatever desc->dtype.
  * desc->inner_R != 0 returns NFPB200_EUNSUPPORTED.  What each problem takes (nfpb200_describe_path names it):
- *   - NHWC bf16 covered by the token kernels: their pooled mode ("fused/token_*"); GAP(x) goes to the workspace;
+ *   - NHWC bf16 / fp16 covered by the token kernels: their pooled mode ("fused/token_*"); GAP(x) goes to the workspace;
  *   - NCHW covered by the ring kernels: their pooled mode ("fused/stream_*"); GAP(x) goes to the workspace;
  *   - NCHW cosine, stride 1, dilation 1, padding = R <= 2, not circular, whose map mode takes "planar/band": the row-band
  *     kernels' pooled mode ("planar/band").  Forward: 2 launches (per-band partial sums (B, n_bands, K) fp32 in the

@@ -15,9 +15,9 @@ import threading
 _LIB_PATH = os.environ.get("NFPB200_LIB") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "lib",
                                                           "libnfp_b200.so")
 
-ABI_VERSION = 4
+ABI_VERSION = 5
 
-F32, BF16 = 0, 1
+F32, BF16, F16 = 0, 1, 2   # F16 (ABI v5): ring and token kernels only, anything else is NFPB200_EUNSUPPORTED
 PAD_MODES = {"zeros": 0, "reflect": 1, "replicate": 2, "circular": 3}
 MEASURES = {
     "norm": 0, "cosine": 1, "dot": 2, "rmse": 3, "geman": 4, "attention": 5, "emd": 6,
@@ -27,7 +27,7 @@ MEASURES = {
 }
 PATHS = {"auto": 0, "generic": 1, "fused": 2, "split": 3}
 HINT_X_STABLE = 0x100   # NFPB200_HINT_X_STABLE, OR-ed into Desc.path for the backward entry points
-FLAG_Y_F32 = 0x200      # NFPB200_FLAG_Y_F32, OR-ed into Desc.path for nfpb200_forward with bf16 x: y is fp32
+FLAG_Y_F32 = 0x200      # NFPB200_FLAG_Y_F32, OR-ed into Desc.path for nfpb200_forward with bf16 / fp16 x: y is fp32
 OP_FORWARD, OP_BACKWARD, OP_POOL_FORWARD, OP_POOL_BACKWARD = 0, 1, 2, 3
 OP_POOLED_MAP_FORWARD, OP_POOLED_MAP_BACKWARD = 4, 5   # GAP(NFP(x)) alone (ABI v4)
 LAYOUT_NCHW, LAYOUT_NHWC = 0, 1

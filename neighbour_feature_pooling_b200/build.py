@@ -21,7 +21,7 @@ INCLUDE = os.path.join(REPO_ROOT, "include")
 LIB_DIR = os.path.join(PKG_DIR, "lib")
 LIB_PATH = os.path.join(LIB_DIR, "libnfp_b200.so")
 OBJ_DIR = os.path.join(PKG_DIR, "build")
-SOURCES = ["nfp_capi.cu", "nfp_generic.cu", "nfp_stream.cu", "nfp_stream_f32.cu", "nfp_stream_bf16.cu",
+SOURCES = ["nfp_capi.cu", "nfp_generic.cu", "nfp_stream.cu", "nfp_stream_f32.cu", "nfp_stream_bf16.cu", "nfp_stream_f16.cu",
            "nfp_split_f32.cu", "nfp_split_bf16.cu", "nfp_planar.cu", "nfp_token.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

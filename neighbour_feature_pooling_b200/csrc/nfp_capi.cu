@@ -16,7 +16,7 @@ constexpr int kPathFlags = NFPB200_HINT_X_STABLE | NFPB200_FLAG_Y_F32;
 
 int make_params(const nfpb200_desc_t* d, KParams* out) {
   if (!d || d->struct_bytes != (int32_t)sizeof(nfpb200_desc_t)) return NFPB200_EINVAL;
-  if (d->dtype != NFPB200_F32 && d->dtype != NFPB200_BF16) return NFPB200_EINVAL;
+  if (d->dtype != NFPB200_F32 && d->dtype != NFPB200_BF16 && d->dtype != NFPB200_F16) return NFPB200_EINVAL;
   if (d->B <= 0 || d->C <= 0 || d->H <= 0 || d->W <= 0) return NFPB200_EINVAL;
   if (d->R < 1 || d->stride < 1 || d->dilation < 1 || d->padding < 0) return NFPB200_EINVAL;
   if (d->padding_mode < NFPB200_PAD_ZEROS || d->padding_mode > NFPB200_PAD_CIRCULAR) return NFPB200_EINVAL;
@@ -49,7 +49,7 @@ int make_params(const nfpb200_desc_t* d, KParams* out) {
   P.similarity = d->similarity != 0;
   P.x_stable = (d->path & NFPB200_HINT_X_STABLE) != 0;
   P.force_split = (d->path & ~kPathFlags) == NFPB200_PATH_SPLIT;
-  P.y_f32 = (d->path & NFPB200_FLAG_Y_F32) != 0 && d->dtype == NFPB200_BF16;
+  P.y_f32 = (d->path & NFPB200_FLAG_Y_F32) != 0 && (d->dtype == NFPB200_BF16 || d->dtype == NFPB200_F16);
   P.diff_taps = d->difference_taps != 0;
   P.eps = d->eps; P.p = d->p; P.q = d->q_scs;
   P.pkind = P_GENERAL;
@@ -72,8 +72,24 @@ inline int pool_op_of(int op) {
 }
 inline size_t align256(size_t b) { return (b + 255) & ~(size_t)255; }
 
+// fp16 is served by two kernel families only, the ones the live heads use: the NCHW streaming-ring kernels (2) and the
+// channels-last token kernels (4), for every op they carry, on exactly the problems a bf16 descriptor sends to them.
+// Everything else -- what bf16 sends to the planar, generic or cluster-split kernels, NFPB200_PATH_GENERIC -- is
+// NFPB200_EUNSUPPORTED, and the caller widens to fp32.  Decided here, before any dispatcher that picks kernels by dtype.
+int choose_path_f16(const nfpb200_desc_t* d, const KParams& P, int op) {
+  const int want = d->path & ~kPathFlags;
+  if (want == NFPB200_PATH_GENERIC) return NFPB200_EUNSUPPORTED;
+  // multi-radius launches: map mode, ring / token kernels, not under NFPB200_PATH_SPLIT (as for bf16)
+  if (P.rin && ((op != NFPB200_OP_FORWARD && op != NFPB200_OP_BACKWARD) || want == NFPB200_PATH_SPLIT))
+    return NFPB200_EUNSUPPORTED;
+  const int pop = pool_op_of(op);
+  if (P.layout == NFPB200_LAYOUT_NHWC) return token_supported(P, NFPB200_F16, d->measure, pop) ? 4 : NFPB200_EUNSUPPORTED;
+  return stream_supported(P, NFPB200_F16, d->measure, pop) ? 2 : NFPB200_EUNSUPPORTED;
+}
+
 // 4 = token (channels-last), 3 = planar, 2 = fused (cluster-split or streaming-ring kernels), 0 = generic, <0 = error
 int choose_path(const nfpb200_desc_t* d, const KParams& P, int op) {
+  if (d->dtype == NFPB200_F16) return choose_path_f16(d, P, op);
   if (pooled_map_op(op)) {
     // the pool ops' choice (token, ring, generic; inner_R refused), with the row-band kernels' pooled mode taking the
     // shapes whose map mode takes "planar/band" instead of the generic kernels
@@ -225,7 +241,7 @@ int nfpb200_forward(const nfpb200_desc_t* desc, const void* x, void* y, void* wo
   if (misaligned(x) || misaligned(y) || misaligned(workspace)) return NFPB200_EALIGN;
   NFP_PROLOGUE(NFPB200_OP_FORWARD)
   if (P.y_f32 && path != 2 && path != 4) return NFPB200_EUNSUPPORTED;
-  if (path == 4) return token_run(P, NFPB200_OP_FORWARD, x, nullptr, y, nullptr, nullptr, nullptr, nullptr, nullptr, ctx);
+  if (path == 4) return token_run(P, desc->dtype, NFPB200_OP_FORWARD, x, nullptr, y, nullptr, nullptr, nullptr, nullptr, nullptr, ctx);
   if (path == 3) return planar_forward(P, desc->dtype, x, y, ctx);
   if (path == 2) return stream_forward(P, desc->dtype, x, y, ctx);
   return generic_forward(P, desc->dtype, desc->measure, x, y, ctx);
@@ -236,7 +252,7 @@ int nfpb200_backward(const nfpb200_desc_t* desc, const void* x, const void* gy, 
   if (!x || !gy || !gx) return NFPB200_EINVAL;
   if (misaligned(x) || misaligned(gy) || misaligned(gx) || misaligned(workspace)) return NFPB200_EALIGN;
   NFP_PROLOGUE(NFPB200_OP_BACKWARD)
-  if (path == 4) return token_run(P, NFPB200_OP_BACKWARD, x, gy, nullptr, gx, nullptr, nullptr, nullptr, nullptr, ctx);
+  if (path == 4) return token_run(P, desc->dtype, NFPB200_OP_BACKWARD, x, gy, nullptr, gx, nullptr, nullptr, nullptr, nullptr, ctx);
   if (path == 3) return planar_backward(P, desc->dtype, x, gy, gx, ctx);
   if (path == 2) return stream_backward(P, desc->dtype, x, gy, gx, ctx);
   return generic_backward(P, desc->dtype, desc->measure, x, gy, gx, ctx);
@@ -247,7 +263,7 @@ int nfpb200_pool_forward(const nfpb200_desc_t* desc, const void* x, float* gap_x
   if (!x || !gap_x || !gap_nfp) return NFPB200_EINVAL;
   if (misaligned(x) || misaligned_f32(gap_x) || misaligned_f32(gap_nfp) || misaligned(workspace)) return NFPB200_EALIGN;
   NFP_PROLOGUE(NFPB200_OP_POOL_FORWARD)
-  if (path == 4) return token_run(P, NFPB200_OP_POOL_FORWARD, x, nullptr, nullptr, nullptr, nullptr, nullptr, gap_x, gap_nfp, ctx);
+  if (path == 4) return token_run(P, desc->dtype, NFPB200_OP_POOL_FORWARD, x, nullptr, nullptr, nullptr, nullptr, nullptr, gap_x, gap_nfp, ctx);
   if (path == 2) return stream_pool_forward(P, desc->dtype, x, gap_x, gap_nfp, ctx);
   return generic_pool_forward(P, desc->dtype, desc->measure, x, gap_x, gap_nfp, ctx);
 }
@@ -258,7 +274,7 @@ int nfpb200_pool_backward(const nfpb200_desc_t* desc, const void* x, const float
   if (misaligned(x) || misaligned(gx) || misaligned_f32(g_gap_x) || misaligned_f32(g_gap_nfp) || misaligned(workspace))
     return NFPB200_EALIGN;
   NFP_PROLOGUE(NFPB200_OP_POOL_BACKWARD)
-  if (path == 4) return token_run(P, NFPB200_OP_POOL_BACKWARD, x, nullptr, nullptr, gx, g_gap_x, g_gap_nfp, nullptr, nullptr, ctx);
+  if (path == 4) return token_run(P, desc->dtype, NFPB200_OP_POOL_BACKWARD, x, nullptr, nullptr, gx, g_gap_x, g_gap_nfp, nullptr, nullptr, ctx);
   if (path == 2) return stream_pool_backward(P, desc->dtype, x, g_gap_x, g_gap_nfp, gx, ctx);
   return generic_pool_backward(P, desc->dtype, desc->measure, x, g_gap_x, g_gap_nfp, gx, ctx);
 }
@@ -271,7 +287,7 @@ int nfpb200_pooled_map_forward(const nfpb200_desc_t* desc, const void* x, float*
   NFP_PROLOGUE(NFPB200_OP_POOLED_MAP_FORWARD)
   if (path == 3) return planar_pooled_forward(P, desc->dtype, x, gap_nfp, ctx);
   float* gap_x = static_cast<float*>(workspace);   // ring / token kernels: GAP(x) is written to the workspace
-  if (path == 4) return token_run(P, NFPB200_OP_POOL_FORWARD, x, nullptr, nullptr, nullptr, nullptr, nullptr, gap_x, gap_nfp, ctx);
+  if (path == 4) return token_run(P, desc->dtype, NFPB200_OP_POOL_FORWARD, x, nullptr, nullptr, nullptr, nullptr, nullptr, gap_x, gap_nfp, ctx);
   if (path == 2) return stream_pool_forward(P, desc->dtype, x, gap_x, gap_nfp, ctx);
   return generic_pool_forward(P, desc->dtype, desc->measure, x, nullptr, gap_nfp, ctx);
 }
@@ -286,7 +302,7 @@ int nfpb200_pooled_map_backward(const nfpb200_desc_t* desc, const void* x, const
   // ring / token kernels: a zero g_gap_x (B, C) in the workspace
   float* zero = static_cast<float*>(workspace);
   if (cudaError_t e = cudaMemsetAsync(zero, 0, (size_t)P.B * P.C * sizeof(float), ctx.stream)) return (int)e;
-  if (path == 4) return token_run(P, NFPB200_OP_POOL_BACKWARD, x, nullptr, nullptr, gx, zero, g_gap_nfp, nullptr, nullptr, ctx);
+  if (path == 4) return token_run(P, desc->dtype, NFPB200_OP_POOL_BACKWARD, x, nullptr, nullptr, gx, zero, g_gap_nfp, nullptr, nullptr, ctx);
   return stream_pool_backward(P, desc->dtype, x, zero, g_gap_nfp, gx, ctx);
 }
 
@@ -326,7 +342,7 @@ int nfpb200_head_forward(const nfpb200_desc_t* desc, const void* x, const float*
   if (rc < 0) return rc;
   LaunchCtx ctx{(cudaStream_t)stream, nullptr, 0};
   if (rc == 4)
-    return token_head_run(P, NFPB200_OP_POOL_FORWARD, x, proj_w, proj_b, out, gap_x, gap_nfp, nullptr, nullptr, ctx);
+    return token_head_run(P, desc->dtype, NFPB200_OP_POOL_FORWARD, x, proj_w, proj_b, out, gap_x, gap_nfp, nullptr, nullptr, ctx);
   return stream_head_forward(P, desc->dtype, x, proj_w, proj_b, out, gap_x, gap_nfp, ctx);
 }
 
@@ -345,7 +361,7 @@ int nfpb200_head_backward(const nfpb200_desc_t* desc, const void* x, const float
   if (rc < 0) return rc;
   LaunchCtx ctx{(cudaStream_t)stream, nullptr, 0};
   if (rc == 4)
-    return token_head_run(P, NFPB200_OP_POOL_BACKWARD, x, proj_w, proj_b, nullptr, const_cast<float*>(gap_x),
+    return token_head_run(P, desc->dtype, NFPB200_OP_POOL_BACKWARD, x, proj_w, proj_b, nullptr, const_cast<float*>(gap_x),
                           const_cast<float*>(gap_nfp), g_out, gx, ctx);
   return stream_head_backward(P, desc->dtype, x, proj_w, proj_b, gap_x, gap_nfp, g_out, gx, ctx);
 }

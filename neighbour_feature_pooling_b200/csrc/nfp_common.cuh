@@ -3,6 +3,7 @@
 
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <math.h>
 #include <stdint.h>
 
@@ -23,7 +24,7 @@ struct KParams {
   int layout;           // NFPB200_LAYOUT_*
   long long x_batch_stride, gx_batch_stride;  // NHWC: elements between images (0 = dense)
   int force_split;      // NFPB200_PATH_SPLIT: the cluster-split kernels or nothing
-  int y_f32;            // NFPB200_FLAG_Y_F32: forward writes y as fp32 although x is bf16
+  int y_f32;            // NFPB200_FLAG_Y_F32: forward writes y as fp32 although x is bf16 / fp16
   int x_stable;         // NFPB200_HINT_X_STABLE: x is not an output of the launch that precedes this one
   int rin, Kin;         // multi-radius launch (desc.inner_R): inner radius r (0 = off) and its tap count (2r+1)^2 - 1
   float eps, p, q;
@@ -62,10 +63,13 @@ __host__ __device__ __forceinline__ void tap_rc(int t, int k, int K, int& a, int
 template <typename T> __device__ __forceinline__ float to_f32(T v);
 template <> __device__ __forceinline__ float to_f32<float>(float v) { return v; }
 template <> __device__ __forceinline__ float to_f32<__nv_bfloat16>(__nv_bfloat16 v) { return __bfloat162float(v); }
+template <> __device__ __forceinline__ float to_f32<__half>(__half v) { return __half2float(v); }
 
 template <typename T> __device__ __forceinline__ T from_f32(float v);
 template <> __device__ __forceinline__ float from_f32<float>(float v) { return v; }
 template <> __device__ __forceinline__ __nv_bfloat16 from_f32<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
+// round to nearest: a value beyond 65504 becomes +-inf (as a narrowing copy does); nothing is clamped
+template <> __device__ __forceinline__ __half from_f32<__half>(float v) { return __float2half_rn(v); }
 
 __device__ __forceinline__ float sgnf(float v) { return (v > 0.f) ? 1.f : ((v < 0.f) ? -1.f : 0.f); }
 
@@ -105,14 +109,14 @@ int stream_head_forward(const KParams& P, int dtype, const void* x, const float*
 int stream_head_backward(const KParams& P, int dtype, const void* x, const float* proj_w, const float* proj_b,
                          const float* gap_x, const float* gap_nfp, const float* g_out, void* gx, const LaunchCtx& ctx);
 
-// channels-last ("token") tensor-core kernels (bf16, cosine, stride 1, dilation 1, pad = R): nfp_token.cu
+// channels-last ("token") tensor-core kernels (bf16 / fp16, cosine, stride 1, dilation 1, pad = R): nfp_token.cu
 bool token_supported(const KParams& P, int dtype, int measure, int op);
 const char* token_name(const KParams& P);
-int token_run(const KParams& P, int op, const void* x, const void* gy, void* y, void* gx, const float* g_gap_x,
+int token_run(const KParams& P, int dtype, int op, const void* x, const void* gy, void* y, void* gx, const float* g_gap_x,
               const float* g_gap_nfp, float* gap_x, float* gap_nfp, const LaunchCtx& ctx);
 
-int token_head_run(const KParams& P, int op, const void* x, const float* proj_w, const float* proj_b, float* out,
-                   float* gap_x, float* gap_nfp, const float* g_out, void* gx, const LaunchCtx& ctx);
+int token_head_run(const KParams& P, int dtype, int op, const void* x, const float* proj_w, const float* proj_b,
+                   float* out, float* gap_x, float* gap_nfp, const float* g_out, void* gx, const LaunchCtx& ctx);
 
 // planar kernels (cosine, stride 1, dilation 1, pad = R, any map size): nfp_planar.cu.  Map mode (NFPB200_OP_FORWARD /
 // _BACKWARD) in the band and table forms; pooled-map mode (GAP(NFP(x)), NFPB200_OP_POOLED_MAP_*) in the band form only

@@ -4,6 +4,7 @@
 
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <stdint.h>
 
 namespace nfp {
@@ -125,10 +126,16 @@ template <> __device__ __forceinline__ float ldx<float>(const unsigned char* p) 
 template <> __device__ __forceinline__ float ldx<__nv_bfloat16>(const unsigned char* p) {
   return __uint_as_float(((uint32_t) * reinterpret_cast<const unsigned short*>(p)) << 16);
 }
+template <> __device__ __forceinline__ float ldx<__half>(const unsigned char* p) {
+  return __half2float(*reinterpret_cast<const __half*>(p));
+}
 template <typename T> __device__ __forceinline__ void stx(unsigned char* p, float v);
 template <> __device__ __forceinline__ void stx<float>(unsigned char* p, float v) { *reinterpret_cast<float*>(p) = v; }
 template <> __device__ __forceinline__ void stx<__nv_bfloat16>(unsigned char* p, float v) {
   *reinterpret_cast<__nv_bfloat16*>(p) = __float2bfloat16_rn(v);
+}
+template <> __device__ __forceinline__ void stx<__half>(unsigned char* p, float v) {
+  *reinterpret_cast<__half*>(p) = __float2half_rn(v);
 }
 
 }  // namespace ptx

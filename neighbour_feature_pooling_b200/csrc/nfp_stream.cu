@@ -35,7 +35,11 @@ bool split_ok(const KParams& P, int dtype, int mode) {
   }();
   if (!want_split && !P.force_split) return false;
   if (P.rin) return false;  // multi-radius launches: ring kernels only
-  return (dtype == NFPB200_BF16 ? split::plan_bf16(P, mode) : split::plan_f32(P, mode)).ok;
+  switch (dtype) {
+    case NFPB200_F32: return split::plan_f32(P, mode).ok;
+    case NFPB200_BF16: return split::plan_bf16(P, mode).ok;
+    default: return false;   // NFPB200_F16: the cluster-split kernels carry no fp16 instantiation
+  }
 }
 
 int run(const KParams& P, int dtype, int mode, stream::StreamArgs a, cudaStream_t s) {
@@ -48,23 +52,34 @@ int run(const KParams& P, int dtype, int mode, stream::StreamArgs a, cudaStream_
     sa.x_early = a.x_early;
     sa.y_f32 = P.y_f32;
     sa.dbg = stream::g_debug_stamps.load(std::memory_order_relaxed);
-    return dtype == NFPB200_BF16 ? split::launch_bf16(P, mode, sa, s) : split::launch_f32(P, mode, sa, s);
+    return dtype == NFPB200_BF16 ? split::launch_bf16(P, mode, sa, s) : split::launch_f32(P, mode, sa, s);  // never F16
   }
   a.B = P.B; a.C = P.C;
   a.pad_mode = P.mode; a.similarity = P.similarity; a.eps = P.eps;
   a.y_f32 = P.y_f32;
   a.kin = P.Kin; a.rin = P.rin;
   a.dbg = stream::g_debug_stamps.load(std::memory_order_relaxed);
-  return dtype == NFPB200_BF16 ? stream::launch_bf16(P, mode, a, s) : stream::launch_f32(P, mode, a, s);
+  switch (dtype) {
+    case NFPB200_F32: return stream::launch_f32(P, mode, a, s);
+    case NFPB200_BF16: return stream::launch_bf16(P, mode, a, s);
+    case NFPB200_F16: return stream::launch_f16(P, mode, a, s);
+    default: return NFPB200_EINVAL;
+  }
 }
 
 }  // namespace
 
 bool stream_supported(const KParams& P, int dtype, int measure, int op) {
   if (!geometry_ok(P, measure)) return false;
-  if (split_ok(P, dtype, op_mode(op))) return true;
+  const int mode = op_mode(op);
+  if (dtype == NFPB200_F16) {
+    // the ring kernels serve fp16 exactly where they serve bf16 (same element size, same plans); a problem the
+    // cluster-split kernels would take for bf16 (NFPB200_PATH_SPLIT, NFPB200_FUSED_IMPL=split) is not served
+    return !P.force_split && !split_ok(P, NFPB200_BF16, mode) && stream::plan_ok_f16(P, mode);
+  }
+  if (split_ok(P, dtype, mode)) return true;
   if (P.force_split) return false;
-  return dtype == NFPB200_BF16 ? stream::plan_ok_bf16(P, op_mode(op)) : stream::plan_ok_f32(P, op_mode(op));
+  return dtype == NFPB200_BF16 ? stream::plan_ok_bf16(P, mode) : stream::plan_ok_f32(P, mode);
 }
 
 const char* stream_name(const KParams& P, int dtype, int measure, int op) {

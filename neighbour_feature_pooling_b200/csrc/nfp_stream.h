@@ -1,5 +1,5 @@
 // Internal interface between the dtype-specific translation units of the streaming fused kernels
-// (nfp_stream_f32.cu, nfp_stream_bf16.cu) and the dispatcher (nfp_stream.cu).
+// (nfp_stream_f32.cu, nfp_stream_bf16.cu, nfp_stream_f16.cu) and the dispatcher (nfp_stream.cu).
 #pragma once
 
 #include <atomic>
@@ -55,8 +55,10 @@ struct StreamArgs {
 
 bool plan_ok_f32(const KParams& P, int mode);
 bool plan_ok_bf16(const KParams& P, int mode);
+bool plan_ok_f16(const KParams& P, int mode);
 int launch_f32(const KParams& P, int mode, const StreamArgs& a, cudaStream_t stream);
 int launch_bf16(const KParams& P, int mode, const StreamArgs& a, cudaStream_t stream);
+int launch_f16(const KParams& P, int mode, const StreamArgs& a, cudaStream_t stream);
 // device buffer set through nfpb200_debug_phase_timing (null = off); atomic, so setting it while another host thread
 // launches is a benign race: that launch stamps either into the old buffer, the new one, or not at all
 extern std::atomic<unsigned long long*> g_debug_stamps;

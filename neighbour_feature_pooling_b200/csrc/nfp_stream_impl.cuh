@@ -1,6 +1,6 @@
 // Streaming fused NFP kernels for sm_100a: cosine measure, stride 1, dilation 1, padding = R
 // (the configuration every live model path of the reference uses: models/NFP_Pooling.py:10-16,
-// models/texture_pooling.py:232,302).  Included by nfp_stream_f32.cu / nfp_stream_bf16.cu.
+// models/texture_pooling.py:232,302).  Included by nfp_stream_f32.cu / nfp_stream_bf16.cu / nfp_stream_f16.cu.
 //
 // One CTA owns one image at a time (persistent loop over b = blockIdx.x, += gridDim.x).  Inside
 // the CTA one PRODUCER warp streams the image's x as chunks of CC channels (CC x H x W contiguous

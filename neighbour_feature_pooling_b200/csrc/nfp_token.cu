@@ -1,4 +1,4 @@
-// Channels-last ("token") fused NFP kernels for sm_100a, bf16: cosine measure, stride 1, dilation 1, padding = R.
+// Channels-last ("token") fused NFP kernels for sm_100a, bf16 or fp16: cosine measure, stride 1, dilation 1, padding = R.
 //
 // Input layout: x[b][p][c] with the C channels of a pixel contiguous and an arbitrary batch stride -- what a
 // channels_last (NHWC) feature map is in memory, and what the reference's ViT head builds as a VIEW of the backbone's
@@ -6,25 +6,31 @@
 // (197*C, 1, W*C, C); models/vittiny.py:129-135).  The NCHW kernels would need a repack copy each way; here the
 // channel contraction runs on tensor cores straight from that layout:
 //
-//   load     the image's P x C bf16 matrix X -> shared memory with 16-byte cp.async copies, 16-byte chunks XOR-swizzled
+//   load     the image's P x C bf16 / fp16 matrix X -> shared memory with 16-byte cp.async copies, 16-byte chunks XOR-swizzled
 //            by (row & 7) so that every ldmatrix below is bank-conflict-free; two image buffers when they fit (the next
 //            image streams in while the current one is processed).
 //   Gram     G = X X^T restricted to the band the k x k window needs: mma.sync.m16n8k16 (bf16 x bf16 -> fp32: the
 //            products are exact, accumulation is fp32 as in the NCHW kernels).  A = 16 pixel rows, B = the pixel rows
 //            of the n-tiles at and after the diagonal (X is both operands; dot(p,q) = dot(q,p)), K = channels, split
-//            over warps.  The accumulator entries whose (row, column) pair is a forward window direction go to the
+//            over warps (fp16: mma.sync.m16n8k16 f16 x f16 -> fp32, equally exact).  The accumulator entries whose (row, column) pair is a forward window direction go to the
 //            per-pixel table the NCHW kernels build with FMAs (|x_p|^2 and (k*k-1)/2 dots per pixel).
 //   forward  y = dot / (max(|p|,eps) max(|q|,eps)) via the compile-time stencil tables -> (B, K, H, W) (NCHW, as the
-//            reference returns it; bf16 or, under autocast, fp32); pooled mode reduces instead.
+//            reference returns it; the dtype of x or, under autocast, fp32); pooled mode reduces instead.
 //   backward the closed-form stencil coefficients Wd[p][o] (same code as the NCHW kernels: gather form, no atomics)
 //            are scattered into the banded P x P matrix M (bf16 hi + lo parts: 16 mantissa bits), and
 //            gx = M X runs on the tensor cores again: A = M (16 rows x the 3..5 k-tiles of the band), B = X through
-//            ldmatrix.trans, fp32 accumulators -> bf16 -> per-warp staging -> 128-byte row segments of gx (channels-last).
+//            ldmatrix.trans, fp32 accumulators -> bf16 / fp16 -> per-warp staging -> 128-byte row segments of gx
+//            (channels-last).  fp16 x: M stays bf16 hi + lo -- its entries reach ~1/eps^2 at degenerate pixels and span
+//            ~1e6 within a row, beyond fp16's range, so an fp16 M would flush the ordinary entries to subnormals.  Each
+//            X fragment is split in registers into bf16 hi + lo instead (exact: an fp16 value has 11 significant bits;
+//            the f16 and bf16 m16n8k16 fragment layouts are the same), and gx = M_hi X_hi + M_hi X_lo + M_lo X_hi.
 //
 // Bit-reproducible: every sum has a fixed order.  fp32 channels-last inputs are not covered (TF32 would break the 1e-5
 // parity bound): the host side repacks those to NCHW.
 #include <stdio.h>
 #include <stdlib.h>
+
+#include <type_traits>
 
 #include "nfp_common.cuh"
 #include "nfp_ptx.cuh"
@@ -45,6 +51,7 @@ using stream::MODE_POOL_BWD;
 using stream::MODE_POOL_FWD;
 
 typedef __nv_bfloat16 bf16;
+typedef __half f16;
 
 struct TokenArgs {
   const void* x;
@@ -102,6 +109,52 @@ __device__ __forceinline__ void mma_bf16(float (&d)[4], const uint32_t (&a)[4], 
       "mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, {%0, %1, %2, %3};"
       : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
       : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
+}
+
+__device__ __forceinline__ void mma_f16(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
+  asm volatile(
+      "mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, {%0, %1, %2, %3};"
+      : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
+      : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
+}
+// X X^T step in the element type of x (both operands are X)
+template <typename T>
+__device__ __forceinline__ void mma_x(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
+  if constexpr (std::is_same<T, f16>::value) mma_f16(d, a, b0, b1);
+  else mma_bf16(d, a, b0, b1);
+}
+// two packed elements of x -> fp32
+template <typename T>
+__device__ __forceinline__ void unpack_x2(uint32_t v, float& lo, float& hi) {
+  if constexpr (std::is_same<T, f16>::value) {
+    const float2 f = __half22float2(*reinterpret_cast<const __half2*>(&v));
+    lo = f.x; hi = f.y;
+  } else {
+    lo = __uint_as_float(v << 16);
+    hi = __uint_as_float(v & 0xffff0000u);
+  }
+}
+// two fp32 values -> packed elements of x (round to nearest: fp16 overflows to +-inf, nothing is clamped)
+template <typename T>
+__device__ __forceinline__ uint32_t pack_x2(float lo, float hi) {
+  uint32_t r;
+  if constexpr (std::is_same<T, f16>::value) {
+    const __half2 h = __floats2half2_rn(lo, hi);
+    r = *reinterpret_cast<const uint32_t*>(&h);
+  } else {
+    const __nv_bfloat162 h = __floats2bfloat162_rn(lo, hi);
+    r = *reinterpret_cast<const uint32_t*>(&h);
+  }
+  return r;
+}
+// a B fragment register of fp16 X (two halves) -> the same two values as bf16 hi + lo registers, exactly
+__device__ __forceinline__ void split_f16x2(uint32_t v, uint32_t& hi, uint32_t& lo) {
+  const float2 f = __half22float2(*reinterpret_cast<const __half2*>(&v));
+  const __nv_bfloat162 h = __floats2bfloat162_rn(f.x, f.y);
+  const float2 hf = __bfloat1622float2(h);
+  const __nv_bfloat162 l = __floats2bfloat162_rn(f.x - hf.x, f.y - hf.y);
+  hi = *reinterpret_cast<const uint32_t*>(&h);
+  lo = *reinterpret_cast<const uint32_t*>(&l);
 }
 
 template <class C>
@@ -164,7 +217,7 @@ struct Lay {
   }
 };
 
-template <class C, int MODE, int NW>
+template <typename T, class C, int MODE, int NW>
 __global__ void __launch_bounds__(NW * 32, NW == kNWSmall ? 2 : 1) token_kernel(const TokenArgs a, const Tables<C>* __restrict__ gt) {
   using G = Geo<C>;
   constexpr int W = C::W, R = C::R, k = C::k, KK = C::KK, K = C::K, P = C::P, NV = C::NV, PNV = C::PNV;
@@ -234,7 +287,7 @@ __global__ void __launch_bounds__(NW * 32, NW == kNWSmall ? 2 : 1) token_kernel(
       for (int i = tid; i < GY_BYTES / 16; i += NT) cp_async16(gd + i * 16, gsrc + i * 16);
     }
     cp_async_commit();
-    const bf16* src = reinterpret_cast<const bf16*>(a.x) + (size_t)b * a.xbs;
+    const T* src = reinterpret_cast<const T*>(a.x) + (size_t)b * a.xbs;
     const uint32_t xb = xs0 + bf * L.x_stride;
     int row = ld_row0, ch = ld_ch0;
     while (row < P) {   // (row, chunk) walk in steps of NT chunks, no divisions
@@ -318,11 +371,11 @@ __global__ void __launch_bounds__(NW * 32, NW == kNWSmall ? 2 : 1) token_kernel(
       auto Gv = [&](int flat) -> float {
         if constexpr (POOLED) return reinterpret_cast<const float*>(smem_raw + L.gyraw)[flat / P];
         else {
-          float v = ldx<bf16>(g + flat * 2);
+          float v = ldx<T>(g + flat * 2);
           if constexpr (R >= 2) {
             if (a.kin) {  // multi-radius launch: the same tap of the inner radius' map adds its gradient
               const int n = flat / P, n1 = inner_tap(n, R, a.rin);
-              if (n1 >= 0) v += ldx<bf16>(gin + (n1 * P + flat - n * P) * 2);
+              if (n1 >= 0) v += ldx<T>(gin + (n1 * P + flat - n * P) * 2);
             }
           }
           return v;
@@ -394,8 +447,8 @@ __global__ void __launch_bounds__(NW * 32, NW == kNWSmall ? 2 : 1) token_kernel(
         auto compute = [&](const uint32_t (&af)[4], const uint32_t (&bq)[NBP][4]) {
 #pragma unroll
           for (int jp = 0; jp < NBP; ++jp) {
-            mma_bf16(acc[2 * jp], af, bq[jp][0], bq[jp][1]);
-            if (2 * jp + 1 < NTN) mma_bf16(acc[2 * jp + 1], af, bq[jp][2], bq[jp][3]);
+            mma_x<T>(acc[2 * jp], af, bq[jp][0], bq[jp][1]);
+            if (2 * jp + 1 < NTN) mma_x<T>(acc[2 * jp + 1], af, bq[jp][2], bq[jp][3]);
           }
         };
         uint32_t af0[4], bq0[NBP][4], af1[4], bq1[NBP][4];
@@ -443,8 +496,10 @@ __global__ void __launch_bounds__(NW * 32, NW == kNWSmall ? 2 : 1) token_kernel(
         float s0 = 0.f, s1 = 0.f;
         for (int p = 0; p < P; ++p) {
           const uint32_t v = *reinterpret_cast<const uint32_t*>(xbp + p * row_bytes + ((((w2 >> 2) ^ (p & 7)) << 4) | ((w2 & 3) << 2)));
-          s0 += __uint_as_float(v << 16);
-          s1 += __uint_as_float(v & 0xffff0000u);
+          float v0, v1;
+          unpack_x2<T>(v, v0, v1);
+          s0 += v0;
+          s1 += v1;
         }
         a.gap_x[(size_t)b * Cch + 2 * w2] = s0 / (float)P;
         a.gap_x[(size_t)b * Cch + 2 * w2 + 1] = s1 / (float)P;
@@ -467,13 +522,13 @@ __global__ void __launch_bounds__(NW * 32, NW == kNWSmall ? 2 : 1) token_kernel(
         } else {
           const size_t yb = (size_t)b * (K + a.kin) * P;
           if (a.y_f32) reinterpret_cast<float*>(a.y)[yb + a.kin * P + idx] = yv;
-          else reinterpret_cast<bf16*>(a.y)[yb + a.kin * P + idx] = __float2bfloat16_rn(yv);
+          else reinterpret_cast<T*>(a.y)[yb + a.kin * P + idx] = from_f32<T>(yv);
           if constexpr (R >= 2) {
             if (a.kin) {  // multi-radius launch: the inner radius' taps are the inner taps of this window
               const int n1 = inner_tap(idx / P, R, a.rin);
               if (n1 >= 0) {
                 if (a.y_f32) reinterpret_cast<float*>(a.y)[yb + n1 * P + p] = yv;
-                else reinterpret_cast<bf16*>(a.y)[yb + n1 * P + p] = __float2bfloat16_rn(yv);
+                else reinterpret_cast<T*>(a.y)[yb + n1 * P + p] = from_f32<T>(yv);
               }
             }
           }
@@ -564,7 +619,7 @@ __global__ void __launch_bounds__(NW * 32, NW == kNWSmall ? 2 : 1) token_kernel(
       const uint32_t mhi_a = smem_u32(mhi), mlo_a = smem_u32(mlo);
       unsigned char* stg = smem_raw + L.stg + warp * 16 * kStgStride;
       const float* ggx = reinterpret_cast<const float*>(smem_raw + L.ggx);
-      bf16* gxb = reinterpret_cast<bf16*>(a.gx) + (size_t)b * a.gxbs;
+      T* gxb = reinterpret_cast<T*>(a.gx) + (size_t)b * a.gxbs;
       const int nchunk = Cch >> 6;
       for (int item = warp; item < MT * nchunk; item += NW) {
         const int mt = item / nchunk, cc = item - mt * nchunk;
@@ -593,22 +648,39 @@ __global__ void __launch_bounds__(NW * 32, NW == kNWSmall ? 2 : 1) token_kernel(
           ldmatrix_x4(alo, mlo_a + moff);
 #pragma unroll
           for (int np = 0; np < 4; ++np) ldmatrix_x4_trans(bx[np], bb + (((bch + 2 * np) ^ bxr) << 4));
+          if constexpr (std::is_same<T, f16>::value) {
+            // fp16 X: bf16 hi + lo fragments in registers, M_hi X_hi + M_hi X_lo + M_lo X_hi (M_lo X_lo, ~2^-18 of a
+            // term, is below the 16-bit precision M is held at)
 #pragma unroll
-          for (int np = 0; np < 4; ++np) {
-            mma_bf16(acc[2 * np], ahi, bx[np][0], bx[np][1]);
-            mma_bf16(acc[2 * np + 1], ahi, bx[np][2], bx[np][3]);
-          }
+            for (int np = 0; np < 4; ++np) {
+              uint32_t xh[4], xl[4];
 #pragma unroll
-          for (int np = 0; np < 4; ++np) {
-            mma_bf16(acc[2 * np], alo, bx[np][0], bx[np][1]);
-            mma_bf16(acc[2 * np + 1], alo, bx[np][2], bx[np][3]);
+              for (int i = 0; i < 4; ++i) split_f16x2(bx[np][i], xh[i], xl[i]);
+              mma_bf16(acc[2 * np], ahi, xh[0], xh[1]);
+              mma_bf16(acc[2 * np + 1], ahi, xh[2], xh[3]);
+              mma_bf16(acc[2 * np], ahi, xl[0], xl[1]);
+              mma_bf16(acc[2 * np + 1], ahi, xl[2], xl[3]);
+              mma_bf16(acc[2 * np], alo, xh[0], xh[1]);
+              mma_bf16(acc[2 * np + 1], alo, xh[2], xh[3]);
+            }
+          } else {
+#pragma unroll
+            for (int np = 0; np < 4; ++np) {
+              mma_bf16(acc[2 * np], ahi, bx[np][0], bx[np][1]);
+              mma_bf16(acc[2 * np + 1], ahi, bx[np][2], bx[np][3]);
+            }
+#pragma unroll
+            for (int np = 0; np < 4; ++np) {
+              mma_bf16(acc[2 * np], alo, bx[np][0], bx[np][1]);
+              mma_bf16(acc[2 * np + 1], alo, bx[np][2], bx[np][3]);
+            }
           }
         }
-        // fragments -> bf16 -> staging (row stride 144 B: conflict-free) -> 128-byte row segments of gx
+        // fragments -> dtype of x -> staging (row stride 144 B: conflict-free) -> 128-byte row segments of gx
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
-          *reinterpret_cast<__nv_bfloat162*>(stg + g8 * kStgStride + (8 * j + 2 * t4) * 2) = __floats2bfloat162_rn(acc[j][0], acc[j][1]);
-          *reinterpret_cast<__nv_bfloat162*>(stg + (g8 + 8) * kStgStride + (8 * j + 2 * t4) * 2) = __floats2bfloat162_rn(acc[j][2], acc[j][3]);
+          *reinterpret_cast<uint32_t*>(stg + g8 * kStgStride + (8 * j + 2 * t4) * 2) = pack_x2<T>(acc[j][0], acc[j][1]);
+          *reinterpret_cast<uint32_t*>(stg + (g8 + 8) * kStgStride + (8 * j + 2 * t4) * 2) = pack_x2<T>(acc[j][2], acc[j][3]);
         }
         __syncwarp();
 #pragma unroll
@@ -666,13 +738,13 @@ Plan plan_for(const KParams& P) {
   return pl;
 }
 
-template <class C, int MODE, int NW>
+template <typename T, class C, int MODE, int NW>
 int launch_nw(const KParams& P, const Plan& pl, TokenArgs a, cudaStream_t stream) {
   a.nbuf = pl.nbuf;
   a.KS = pl.KS;
   a.KSlog = 0;
   while ((1 << a.KSlog) < pl.KS) ++a.KSlog;
-  auto kern = token_kernel<C, MODE, NW>;
+  auto kern = token_kernel<T, C, MODE, NW>;
   constexpr int kMaxDev = 64;
   static int sm_count[kMaxDev] = {0};
   int dev = 0;
@@ -704,20 +776,22 @@ int launch_nw(const KParams& P, const Plan& pl, TokenArgs a, cudaStream_t stream
   return (int)cudaLaunchKernelEx(&cfg, kern, a, gt);
 }
 
-template <class C, int MODE>
+// the plan depends on the element size only (2 bytes for both dtypes): fp16 coverage is bf16 coverage
+template <typename T, class C, int MODE>
 int launch_mode(const KParams& P, TokenArgs a, cudaStream_t stream) {
   const Plan pl = plan_for<C, MODE>(P);
   if (!pl.ok) return NFPB200_EUNSUPPORTED;
-  return pl.nw == kNWSmall ? launch_nw<C, MODE, kNWSmall>(P, pl, a, stream) : launch_nw<C, MODE, kNWBig>(P, pl, a, stream);
+  return pl.nw == kNWSmall ? launch_nw<T, C, MODE, kNWSmall>(P, pl, a, stream)
+                           : launch_nw<T, C, MODE, kNWBig>(P, pl, a, stream);
 }
 
-template <class C>
+template <typename T, class C>
 int launch_cfg(const KParams& P, int mode, const TokenArgs& a, cudaStream_t stream) {
   switch (mode) {
-    case MODE_FWD: return launch_mode<C, MODE_FWD>(P, a, stream);
-    case MODE_BWD: return launch_mode<C, MODE_BWD>(P, a, stream);
-    case MODE_POOL_FWD: return launch_mode<C, MODE_POOL_FWD>(P, a, stream);
-    default: return launch_mode<C, MODE_POOL_BWD>(P, a, stream);
+    case MODE_FWD: return launch_mode<T, C, MODE_FWD>(P, a, stream);
+    case MODE_BWD: return launch_mode<T, C, MODE_BWD>(P, a, stream);
+    case MODE_POOL_FWD: return launch_mode<T, C, MODE_POOL_FWD>(P, a, stream);
+    default: return launch_mode<T, C, MODE_POOL_BWD>(P, a, stream);
   }
 }
 template <class C>
@@ -730,12 +804,20 @@ bool plan_ok_cfg(const KParams& P, int mode) {
   }
 }
 
-int launch(const KParams& P, int mode, const TokenArgs& a, cudaStream_t stream) {
+template <typename T>
+int launch_dtype(const KParams& P, int mode, const TokenArgs& a, cudaStream_t stream) {
 #define X(H_, W_, R_, TW_) \
-  if (P.H == H_ && P.W == W_ && P.R == R_) return launch_cfg<Cfg<H_, W_, R_, TW_>>(P, mode, a, stream);
+  if (P.H == H_ && P.W == W_ && P.R == R_) return launch_cfg<T, Cfg<H_, W_, R_, TW_>>(P, mode, a, stream);
   NFP_STREAM_SHAPES(X)
 #undef X
   return NFPB200_EUNSUPPORTED;
+}
+int launch(const KParams& P, int dtype, int mode, const TokenArgs& a, cudaStream_t stream) {
+  switch (dtype) {
+    case NFPB200_BF16: return launch_dtype<bf16>(P, mode, a, stream);
+    case NFPB200_F16: return launch_dtype<f16>(P, mode, a, stream);
+    default: return NFPB200_EUNSUPPORTED;
+  }
 }
 bool plan_ok(const KParams& P, int mode) {
 #define X(H_, W_, R_, TW_) \
@@ -759,7 +841,7 @@ int token_mode(int op) {
 }  // namespace
 
 bool token_supported(const KParams& P, int dtype, int measure, int op) {
-  if (dtype != NFPB200_BF16 || measure != NFPB200_COSINE) return false;
+  if ((dtype != NFPB200_BF16 && dtype != NFPB200_F16) || measure != NFPB200_COSINE) return false;
   if (P.stride != 1 || P.dil != 1 || P.pad != P.R || P.mode == NFPB200_PAD_CIRCULAR) return false;
   return token::plan_ok(P, token_mode(op));
 }
@@ -773,8 +855,8 @@ const char* token_name(const KParams& P) {
   return nm;
 }
 
-int token_head_run(const KParams& P, int op, const void* x, const float* proj_w, const float* proj_b, float* out,
-                   float* gap_x, float* gap_nfp, const float* g_out, void* gx, const LaunchCtx& ctx) {
+int token_head_run(const KParams& P, int dtype, int op, const void* x, const float* proj_w, const float* proj_b,
+                   float* out, float* gap_x, float* gap_nfp, const float* g_out, void* gx, const LaunchCtx& ctx) {
   token::TokenArgs a{};
   a.x = x; a.gx = gx; a.gap_x = gap_x; a.gap_nfp = gap_nfp;
   a.proj_w = proj_w; a.proj_b = proj_b; a.head_out = out; a.head_gout = g_out;
@@ -784,10 +866,10 @@ int token_head_run(const KParams& P, int op, const void* x, const float* proj_w,
   a.gxbs = P.gx_batch_stride > 0 ? P.gx_batch_stride : dense;
   a.pad_mode = P.mode; a.similarity = P.similarity; a.eps = P.eps; a.y_f32 = 0;
   a.dbg = stream::g_debug_stamps.load(std::memory_order_relaxed);
-  return token::launch(P, token_mode(op), a, ctx.stream);
+  return token::launch(P, dtype, token_mode(op), a, ctx.stream);
 }
 
-int token_run(const KParams& P, int op, const void* x, const void* gy, void* y, void* gx, const float* g_gap_x,
+int token_run(const KParams& P, int dtype, int op, const void* x, const void* gy, void* y, void* gx, const float* g_gap_x,
               const float* g_gap_nfp, float* gap_x, float* gap_nfp, const LaunchCtx& ctx) {
   token::TokenArgs a{};
   a.x = x; a.gy = gy; a.y = y; a.gx = gx;
@@ -799,7 +881,7 @@ int token_run(const KParams& P, int op, const void* x, const void* gy, void* y, 
   a.pad_mode = P.mode; a.similarity = P.similarity; a.eps = P.eps; a.y_f32 = P.y_f32;
   a.kin = P.Kin; a.rin = P.rin;
   a.dbg = stream::g_debug_stamps.load(std::memory_order_relaxed);
-  return token::launch(P, token_mode(op), a, ctx.stream);
+  return token::launch(P, dtype, token_mode(op), a, ctx.stream);
 }
 
 }  // namespace nfp

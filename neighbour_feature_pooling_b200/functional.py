@@ -98,7 +98,12 @@ def _reject_cpu(x: torch.Tensor):
         "as shape probes under torch.no_grad().)")
 
 
-_KERNEL_DTYPES = {torch.float32: _capi.F32, torch.bfloat16: _capi.BF16}
+_KERNEL_DTYPES = {torch.float32: _capi.F32, torch.bfloat16: _capi.BF16, torch.float16: _capi.F16}
+_DTYPE_NAMES = {_capi.F32: "f32", _capi.BF16: "bf16", _capi.F16: "f16"}
+# the ops each entry point issues: an fp16 input is kept only when all of them take it (_prepare)
+MAP_OPS = (_capi.OP_FORWARD, _capi.OP_BACKWARD)
+POOL_OPS = (_capi.OP_POOL_FORWARD, _capi.OP_POOL_BACKWARD)
+POOLED_MAP_OPS = (_capi.OP_POOLED_MAP_FORWARD, _capi.OP_POOLED_MAP_BACKWARD)
 # diagnostics: when a set is installed here (bench_train.py does during its eager warm-up), every forward records the
 # kernel path it takes ("fused/token_7x7_r1 bf16 pool", ...)
 PATH_TRACE = None
@@ -106,7 +111,7 @@ PATH_TRACE = None
 
 def _trace(desc, op, what):
     if PATH_TRACE is not None:
-        PATH_TRACE.add(f"{_capi.describe_path(desc, op)} {'bf16' if desc.dtype == _capi.BF16 else 'f32'} "
+        PATH_TRACE.add(f"{_capi.describe_path(desc, op)} {_DTYPE_NAMES[desc.dtype]} "
                        f"{'channels-last' if desc.layout else 'nchw'} {what}")
 
 # NFPB200_HINT_X_STABLE (include/nfp_b200.h) is opt-in: it pays only when the backward directly follows another fused NFP
@@ -115,15 +120,18 @@ def _trace(desc, op, what):
 _X_STABLE_HINT = os.environ.get("NFPB200_X_STABLE_HINT", "0") == "1"
 
 
-def _prepare(x: torch.Tensor, cfg: NFPConfig = None):
+def _prepare(x: torch.Tensor, cfg: NFPConfig = None, ops=MAP_OPS):
     """-> (tensor in a kernel dtype, dtype to return results in, memory layout the kernels will read)
 
     Under ``torch.autocast('cuda')`` the reference extracts the neighbours with convs in the autocast dtype and then
     runs ``F.cosine_similarity`` (``norm``, ``sum``, ``softmax`` ... for the other measures), which is on autocast's
-    fp32 list: its similarity map is float32.  A bf16 input therefore gives an fp32 map (the fused forward writes
-    fp32 directly, NFPB200_FLAG_Y_F32).  An fp32 input is NOT rounded to the autocast dtype first: the kernels
-    accumulate in fp32 anyway, so the result only differs from the reference's by the reference's own input rounding
-    (well inside the 2e-2 bf16 tolerance), and the cast kernel is saved."""
+    fp32 list: its similarity map is float32.  A bf16 / fp16 input therefore gives an fp32 map (the fused forward
+    writes fp32 directly, NFPB200_FLAG_Y_F32).  An NCHW fp32 input is NOT rounded to the autocast dtype first: the
+    kernels accumulate in fp32 anyway, so the result only differs from the reference's by the reference's own input
+    rounding, and the cast kernel is saved.
+
+    fp16 is served by the ring (NCHW) and token (channels-last) kernels only: an fp16 input is kept as it is when every
+    op in `ops` (the ops the caller will issue) takes it in the layout chosen below, and widened to fp32 otherwise."""
     if x.dim() != 4:
         raise RuntimeError(f"NFP expects a 4-D (B, C, H, W) input, got {tuple(x.shape)}")
     if not x.is_floating_point():
@@ -133,22 +141,48 @@ def _prepare(x: torch.Tensor, cfg: NFPConfig = None):
         out_dtype = torch.float32
     if x.dtype == torch.float64:
         raise RuntimeError("NFP kernels compute in fp32; float64 inputs are not supported")
-    if x.dtype not in _KERNEL_DTYPES:  # fp16: widen, the kernels accumulate in fp32 anyway
-        x = x.float()
+    widened = False
+    if x.dtype == torch.float16:
+        kept = _prepare_f16(x, cfg, ops)
+        if kept is not None:
+            return kept[0], out_dtype, kept[1]
+        x, widened = x.float(), True   # not covered by the fp16 kernels: widen, the kernels accumulate in fp32 anyway
     if cfg is not None and _channels_last_ok(x, cfg):
         return x, out_dtype, _capi.LAYOUT_NHWC     # consumed in place: no repack copy
     if (cfg is not None and x.dtype == torch.float32 and x.dim() == 4 and torch.is_autocast_enabled("cuda")
-            and torch.get_autocast_dtype("cuda") == torch.bfloat16 and _is_channels_last_view(x)):
-        # fp32 channels-last map under bf16 autocast (a ViT's final LayerNorm emits fp32 tokens): the reference's
-        # extraction convs would round it to bf16 (nfp.py:152-153); doing the same costs one cast kernel (4 B in,
-        # 2 B out per element) instead of an NCHW repack (4 B in, 4 B out) and keeps the tensor-core path
-        xb = x.to(torch.bfloat16)
-        if _channels_last_ok(xb, cfg):
+            and torch.get_autocast_dtype("cuda") in (torch.bfloat16, torch.float16) and _is_channels_last_view(x)
+            and not widened):
+        # fp32 channels-last map under bf16 / fp16 autocast (a ViT's final LayerNorm emits fp32 tokens): the reference's
+        # extraction convs would round it to the autocast dtype (nfp.py:152-153); doing the same costs one cast kernel
+        # (4 B in, 2 B out per element) instead of an NCHW repack (4 B in, 4 B out) and keeps the tensor-core path
+        ac = torch.get_autocast_dtype("cuda")
+        xb = x.to(ac)
+        if _channels_last_ok(xb, cfg, ops if ac == torch.float16 else None):
             return xb, out_dtype, _capi.LAYOUT_NHWC
     x = x.contiguous()
     if x.data_ptr() % 16:   # a view at an odd storage offset: the kernels move data with 16-byte TMA copies
         x = x.clone()
     return x, out_dtype, _capi.LAYOUT_NCHW
+
+
+def _served(x: torch.Tensor, cfg: NFPConfig, layout: int, ops) -> bool:
+    """True when every op in `ops` has a kernel path for x in `layout`."""
+    desc = _desc_for(x, cfg, layout)
+    buf = ctypes.create_string_buffer(64)
+    lib = _capi.load()
+    return all(lib.nfpb200_describe_path(ctypes.byref(desc), op, buf, 64) == 0 for op in ops)
+
+
+def _prepare_f16(x: torch.Tensor, cfg: NFPConfig, ops):
+    """fp16 x as the ring / token kernels read it -> (tensor, layout), or None when they do not cover the problem."""
+    if cfg is None:
+        return None
+    if _channels_last_ok(x, cfg, ops):
+        return x, _capi.LAYOUT_NHWC
+    xc = x.contiguous()
+    if xc.data_ptr() % 16:
+        xc = xc.clone()
+    return (xc, _capi.LAYOUT_NCHW) if _served(xc, cfg, _capi.LAYOUT_NCHW, ops) else None
 
 
 def _is_channels_last_view(x: torch.Tensor) -> bool:
@@ -159,17 +193,16 @@ def _is_channels_last_view(x: torch.Tensor) -> bool:
     return C > 1 and sc == 1 and sw == C and sh == W * C and (B == 1 or sb >= H * W * C) and not x.is_contiguous()
 
 
-def _channels_last_ok(x: torch.Tensor, cfg: NFPConfig) -> bool:
-    """True when the tensor-core channels-last kernels (fused/token_*) take x as it lies in memory."""
-    if x.dtype != torch.bfloat16 or x.dim() != 4 or not _is_channels_last_view(x):
+def _channels_last_ok(x: torch.Tensor, cfg: NFPConfig, ops=None) -> bool:
+    """True when the tensor-core channels-last kernels (fused/token_*) take x as it lies in memory: for every op in
+    `ops` (fp16), or for the map backward (bf16, ops None)."""
+    if x.dtype not in (torch.bfloat16, torch.float16) or x.dim() != 4 or not _is_channels_last_view(x):
         return False
     if x.data_ptr() % 16 or (x.shape[0] > 1 and x.stride(0) % 8):
         return False
     if cfg.path == "generic":
         return False
-    desc = _desc_for(x, cfg, _capi.LAYOUT_NHWC)
-    buf = ctypes.create_string_buffer(64)
-    return _capi.load().nfpb200_describe_path(ctypes.byref(desc), _capi.OP_BACKWARD, buf, 64) == 0
+    return _served(x, cfg, _capi.LAYOUT_NHWC, ops if ops is not None else (_capi.OP_BACKWARD,))
 
 
 def _desc_for(x: torch.Tensor, cfg: NFPConfig, layout: int = 0) -> _capi.Desc:
@@ -205,9 +238,9 @@ class _NFPSimilarity(torch.autograd.Function):
     def forward(ctx, x, cfg, y_f32=False, layout=0):
         desc = _desc_for(x, cfg, layout)
         Ho, Wo = _capi.output_shape(desc)
-        # bf16 x, fp32 map (autocast): the fused kernels write fp32 directly; other paths write bf16 (widened by
+        # bf16 / fp16 x, fp32 map (autocast): the fused kernels write fp32 directly; other paths write bf16 (widened by
         # the caller)
-        y_f32 = bool(y_f32) and x.dtype == torch.bfloat16 and \
+        y_f32 = bool(y_f32) and x.dtype in (torch.bfloat16, torch.float16) and \
             _capi.describe_path(desc, _capi.OP_FORWARD).startswith("fused/")
         if y_f32:
             desc.path |= _capi.FLAG_Y_F32
@@ -334,7 +367,7 @@ class _NFPHead(torch.autograd.Function):
         gap_nfp = torch.empty((B, cfg.out_channels), dtype=torch.float32, device=x.device)
         if PATH_TRACE is not None:
             PATH_TRACE.add(f"{_capi.describe_path(desc, _capi.OP_POOL_FORWARD)} "
-                           f"{'bf16' if desc.dtype == _capi.BF16 else 'f32'} {'channels-last' if layout else 'nchw'} "
+                           f"{_DTYPE_NAMES[desc.dtype]} {'channels-last' if layout else 'nchw'} "
                            "fused head (GAP, GAP(NFP), proj, product)")
         with torch.cuda.device(x.device):
             rc = _capi.load().nfpb200_head_forward(ctypes.byref(desc), x.data_ptr(), w.data_ptr(),
@@ -375,7 +408,7 @@ def nfp_head(x: torch.Tensor, weight: torch.Tensor, bias, cfg: NFPConfig):
     if x.device.type != "cuda" or x.dim() != 4 or weight.device != x.device:
         return None
     _check_geometry(x.shape[2], x.shape[3], cfg)
-    xk, out_dtype, layout = _prepare(x, cfg)
+    xk, out_dtype, layout = _prepare(x, cfg, POOL_OPS)
     desc = _desc_for(xk, cfg, layout)
     if _capi.load().nfpb200_head_supported(ctypes.byref(desc)) != 0:
         return None
@@ -393,9 +426,9 @@ class _NFPMultiRadius(torch.autograd.Function):
         desc = _desc_for(x, cfg, layout)
         desc.inner_R = inner_R
         Ho, Wo = _capi.output_shape(desc)
-        # bf16 x, fp32 map (autocast): the fused kernels write fp32 directly; the planar band kernels write bf16 (widened
-        # by the caller)
-        y_f32 = bool(y_f32) and x.dtype == torch.bfloat16 and \
+        # bf16 / fp16 x, fp32 map (autocast): the fused kernels write fp32 directly; the planar band kernels write bf16
+        # (widened by the caller)
+        y_f32 = bool(y_f32) and x.dtype in (torch.bfloat16, torch.float16) and \
             _capi.describe_path(desc, _capi.OP_FORWARD).startswith("fused/")
         if y_f32:
             desc.path |= _capi.FLAG_Y_F32
@@ -484,7 +517,7 @@ def nfp_gap_pair(x: torch.Tensor, cfg: NFPConfig):
         _reject_cpu(x)
     if x.dim() == 4:
         _check_geometry(x.shape[2], x.shape[3], cfg)
-    xk, out_dtype, layout = _prepare(x, cfg)
+    xk, out_dtype, layout = _prepare(x, cfg, POOL_OPS)
     gx, gn = _NFPGapPair.apply(xk, cfg, layout)   # both fp32 (the kernels accumulate in fp32)
     # NFP_Pooling.py:27: avgpool(x) keeps the dtype of x (also under autocast); :31: the similarity map's dtype
     return gx.to(x.dtype), gn.to(out_dtype)
@@ -499,7 +532,7 @@ def nfp_pooled_similarity(x: torch.Tensor, cfg: NFPConfig) -> torch.Tensor:
         _reject_cpu(x)
     if x.dim() == 4:
         _check_geometry(x.shape[2], x.shape[3], cfg)
-    xk, out_dtype, layout = _prepare(x, cfg)
+    xk, out_dtype, layout = _prepare(x, cfg, POOLED_MAP_OPS)
     gn = _NFPPooledMap.apply(xk, cfg, layout)   # fp32
     return gn if gn.dtype == out_dtype else gn.to(out_dtype)
 
