@@ -298,9 +298,9 @@ __device__ __forceinline__ void chan_grad(float c, float n, const float (&k)[5],
 
 // ---- kernels ----------------------------------------------------------------------------------
 
-// y (or raw fp32 values for attention / scs) for every pair
-template <typename T, int M>
-__global__ void __launch_bounds__(kThreads) pair_forward_kernel(const T* __restrict__ x, T* __restrict__ y,
+// y (or raw fp32 values for attention / scs) for every pair; y is T (map mode) or fp32 (pooled mode, YT = float)
+template <typename T, typename YT, int M>
+__global__ void __launch_bounds__(kThreads) pair_forward_kernel(const T* __restrict__ x, YT* __restrict__ y,
                                                                 float* __restrict__ raw, KParams P,
                                                                 long long npairs) {
   long long idx = (long long)blockIdx.x * kThreads + threadIdx.x;
@@ -314,14 +314,14 @@ __global__ void __launch_bounds__(kThreads) pair_forward_kernel(const T* __restr
     raw[idx] = s[0];
     raw[npairs + idx] = (sqrtf(s[1]) + P.q) * (sqrtf(s[2]) + P.q);
   } else {
-    y[idx] = from_f32<T>(finalize<M>(s, P));
+    y[idx] = from_f32<YT>(finalize<M>(s, P));
   }
 }
 
 // softmax over the K neighbours of every output pixel (nfp.py:202)
-template <typename T>
+template <typename YT>
 __global__ void __launch_bounds__(kThreads) attention_forward_kernel(const float* __restrict__ raw,
-                                                                     T* __restrict__ y, KParams P) {
+                                                                     YT* __restrict__ y, KParams P) {
   long long pix = (long long)blockIdx.x * kThreads + threadIdx.x;
   const long long HoWo = (long long)P.Ho * P.Wo;
   if (pix >= (long long)P.B * HoWo) return;
@@ -333,7 +333,7 @@ __global__ void __launch_bounds__(kThreads) attention_forward_kernel(const float
   for (int t = 0; t < P.K; ++t) z += expf(d[t * HoWo] - m);
   for (int t = 0; t < P.K; ++t) {
     float v = expf(d[t * HoWo] - m) / z;
-    y[b * P.K * HoWo + t * HoWo + r] = from_f32<T>(P.similarity ? v : -v);
+    y[b * P.K * HoWo + t * HoWo + r] = from_f32<YT>(P.similarity ? v : -v);
   }
 }
 
@@ -351,8 +351,8 @@ __device__ __forceinline__ float scs_dh(float t, float p) {
 
 // Sharpened cosine with the reference's cross-batch broadcast (nfp.py:363-374):
 // out[b] = mean_{b'} h(dot[b'] / den[b]).
-template <typename T>
-__global__ void __launch_bounds__(kThreads) scs_forward_kernel(const float* __restrict__ raw, T* __restrict__ y,
+template <typename YT>
+__global__ void __launch_bounds__(kThreads) scs_forward_kernel(const float* __restrict__ raw, YT* __restrict__ y,
                                                                KParams P, long long npairs) {
   long long idx = (long long)blockIdx.x * kThreads + threadIdx.x;
   if (idx >= npairs) return;
@@ -362,7 +362,7 @@ __global__ void __launch_bounds__(kThreads) scs_forward_kernel(const float* __re
   float acc = 0.f;
   for (int bp = 0; bp < P.B; ++bp) acc += scs_h(raw[bp * per + r] / den, P.p);
   float v = acc / (float)P.B;
-  y[idx] = from_f32<T>(P.similarity ? v : 1.f - v);
+  y[idx] = from_f32<YT>(P.similarity ? v : 1.f - v);
 }
 
 // coefficients of every pair (SoA: coef[u * npairs + idx]); gy is T (map mode) or fp32 (pooled mode, GT = float)
@@ -591,17 +591,17 @@ inline unsigned blocks_for(long long n) { return (unsigned)((n + kThreads - 1) /
 
 inline size_t align256(size_t b) { return (b + 255) & ~(size_t)255; }
 
-template <typename T>
-int forward_t(const KParams& P, int measure, const T* x, T* y, const LaunchCtx& ctx) {
+template <typename T, typename YT>
+int forward_t(const KParams& P, int measure, const T* x, YT* y, const LaunchCtx& ctx) {
   const long long npairs = (long long)P.B * P.K * P.Ho * P.Wo;
   float* raw = (float*)ctx.ws;
   NFP_DISPATCH_MEASURE(measure,
-    (pair_forward_kernel<T, M><<<blocks_for(npairs), kThreads, 0, ctx.stream>>>(x, y, raw, P, npairs)));
+    (pair_forward_kernel<T, YT, M><<<blocks_for(npairs), kThreads, 0, ctx.stream>>>(x, y, raw, P, npairs)));
   if (measure == NFPB200_ATTENTION) {
     long long pix = (long long)P.B * P.Ho * P.Wo;
-    attention_forward_kernel<T><<<blocks_for(pix), kThreads, 0, ctx.stream>>>(raw, y, P);
+    attention_forward_kernel<YT><<<blocks_for(pix), kThreads, 0, ctx.stream>>>(raw, y, P);
   } else if (measure == NFPB200_SCS) {
-    scs_forward_kernel<T><<<blocks_for(npairs), kThreads, 0, ctx.stream>>>(raw, y, P, npairs);
+    scs_forward_kernel<YT><<<blocks_for(npairs), kThreads, 0, ctx.stream>>>(raw, y, P, npairs);
   }
   return (int)cudaGetLastError();
 }
@@ -632,16 +632,16 @@ int backward_t(const KParams& P, int measure, const T* x, const GT* gy, T* gx, c
 size_t generic_workspace_bytes(const KParams& P, int dtype, int measure, int op) {
   const size_t npairs = (size_t)P.B * P.K * P.Ho * P.Wo;
   const size_t nx = (size_t)P.B * P.C * P.H * P.W;
-  const size_t esz = dtype == NFPB200_BF16 ? 2 : 4;
   const size_t fwd = measure == NFPB200_ATTENTION ? 4 * npairs : (measure == NFPB200_SCS ? 8 * npairs : 0);
   const size_t bwd = align256(20 * npairs);
   (void)nx;
+  (void)dtype;   // every pooled map and scratch buffer is fp32
   switch (op) {
     case NFPB200_OP_FORWARD: return fwd;
     case NFPB200_OP_BACKWARD: return bwd;
-    case NFPB200_OP_POOL_FORWARD: return align256(esz * npairs) + fwd;   // [y map][forward scratch]
+    case NFPB200_OP_POOL_FORWARD: return align256(4 * npairs) + fwd;     // [fp32 y map][forward scratch]
     case NFPB200_OP_POOL_BACKWARD: return align256(4 * npairs) + bwd;    // [fp32 gy map][backward scratch]
-    case NFPB200_OP_POOLED_MAP_FORWARD: return align256(esz * npairs) + fwd;
+    case NFPB200_OP_POOLED_MAP_FORWARD: return align256(4 * npairs) + fwd;
     case NFPB200_OP_POOLED_MAP_BACKWARD: return align256(4 * npairs) + bwd;
   }
   return 0;
@@ -667,8 +667,8 @@ int generic_launch_count(const KParams& P, int dtype, int measure, int op) {
 
 int generic_forward(const KParams& P, int dtype, int measure, const void* x, void* y, const LaunchCtx& ctx) {
   if (dtype == NFPB200_BF16)
-    return forward_t<__nv_bfloat16>(P, measure, (const __nv_bfloat16*)x, (__nv_bfloat16*)y, ctx);
-  return forward_t<float>(P, measure, (const float*)x, (float*)y, ctx);
+    return forward_t<__nv_bfloat16, __nv_bfloat16>(P, measure, (const __nv_bfloat16*)x, (__nv_bfloat16*)y, ctx);
+  return forward_t<float, float>(P, measure, (const float*)x, (float*)y, ctx);
 }
 
 int generic_backward(const KParams& P, int dtype, int measure, const void* x, const void* gy, void* gx,
@@ -684,14 +684,16 @@ namespace {
 template <typename T>
 int pool_forward_t(const KParams& P, int measure, const T* x, float* gap_x, float* gap_nfp, const LaunchCtx& ctx) {
   const size_t npairs = (size_t)P.B * P.K * P.Ho * P.Wo;
-  T* ymap = (T*)ctx.ws;
-  LaunchCtx inner{ctx.stream, (char*)ctx.ws + align256(sizeof(T) * npairs), 0};
-  int rc = forward_t<T>(P, measure, x, ymap, inner);
+  // the map stays fp32 also for bf16 x: GAP(NFP(x)) is an fp32 result, and a map rounded to bf16 first would carry a
+  // 2^-9 relative error per element into it (the fused kernels sum the fp32 values)
+  float* ymap = (float*)ctx.ws;
+  LaunchCtx inner{ctx.stream, (char*)ctx.ws + align256(sizeof(float) * npairs), 0};
+  int rc = forward_t<T, float>(P, measure, x, ymap, inner);
   if (rc) return rc;
   const long long px = (long long)P.B * P.C, py = (long long)P.B * P.K;
   if (gap_x)   // null: GAP(NFP(x)) only (nfpb200_pooled_map_forward)
     gap_kernel<T><<<blocks_for(px * 32), kThreads, 0, ctx.stream>>>(x, gap_x, P.H * P.W, px);
-  gap_kernel<T><<<blocks_for(py * 32), kThreads, 0, ctx.stream>>>(ymap, gap_nfp, P.Ho * P.Wo, py);
+  gap_kernel<float><<<blocks_for(py * 32), kThreads, 0, ctx.stream>>>(ymap, gap_nfp, P.Ho * P.Wo, py);
   return (int)cudaGetLastError();
 }
 template <typename T>

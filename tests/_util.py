@@ -163,6 +163,111 @@ def elem_grad_err(got, want, geo, dtype=torch.float32):
     return max(elem_grad_errs(got, want, geo, dtype).values(), default=0.0)
 
 
+# ---- one rounding to a 16-bit float (tests/test_bf16_rounding_*.py) --------------------------------------------------
+# (mantissa bits, exponent of the smallest normal, half-way point above the largest finite value)
+_FMT16 = {torch.bfloat16: (7, -126, (2.0 - 2.0 ** -8) * 2.0 ** 127), torch.float16: (10, -14, 65520.0)}
+
+
+def _f64(v):
+    """float64 CPU tensor of a tensor of any dtype (bf16 / fp16 included, which numpy cannot take) or array."""
+    if isinstance(v, torch.Tensor):
+        return v.detach().cpu().double()
+    return torch.as_tensor(np.asarray(v), dtype=torch.float64)
+
+
+def ulp(dtype, v):
+    """The unit in the last place of float64 values `v` in bf16 or fp16 (subnormals included: the spacing below the
+    smallest normal is that of the smallest binade; 0 gets the smallest subnormal)."""
+    mant, emin, _ = _FMT16[dtype]
+    v = _f64(v)
+    e = torch.floor(torch.log2(v.abs().clamp_min(2.0 ** emin)))
+    return torch.exp2(e - mant)
+
+
+def round_nearest(dtype, v):
+    """float64 `v` rounded once to the nearest bf16 / fp16 value, ties to even, as float64 (+-inf past the largest
+    finite value).  torch's own float64 -> bf16 cast goes through fp32 and can round twice."""
+    v = _f64(v)
+    q = ulp(dtype, v)
+    r = torch.round(v / q) * q   # v / q and the product are exact: q is a power of two
+    return torch.where(v.abs() >= _FMT16[dtype][2], torch.sign(v) * math.inf, r)
+
+
+def image_groups(shape):
+    """{image: mask} over a (B, ...) tensor: the groups of rounding_errs for maps and pooled vectors."""
+    return {b: (torch.arange(shape[0]) == b).view(-1, *([1] * (len(shape) - 1))) for b in range(shape[0])}
+
+
+def region_groups(x, eps=1e-6):
+    """{(image, region): mask} over a (B, C, H, W) input gradient: each image and pixel-norm region of x
+    (pixel_regions), the groups grad_errs scores separately."""
+    lab = pixel_regions(x, eps)[:, None]
+    img = torch.arange(lab.shape[0]).view(-1, 1, 1, 1)
+    out = {}
+    for b in range(lab.shape[0]):
+        for r, name in enumerate(REGION_NAMES):
+            m = (lab == r) & (img == b)
+            if m.any():
+                out[(b, name)] = m
+    return out
+
+
+def rounding_errs(got, want, dtype, tau, groups=None):
+    """{group: worst ratio} of a bf16 / fp16 result `got` against the fp64 oracle `want` (run on the rounded inputs):
+
+        |got - want| / (1/2 ulp(want) (1 + 2^-7) + tau S_g),   S_g = max |want| over the group's finite elements.
+
+    One rounding to nearest of an fp32 evaluation within tau S_g of `want` scores <= 1.  Where |want| is past the
+    format's overflow point the result must be the infinity of the same sign (ratio 0, else inf); an infinite or NaN
+    `got` elsewhere scores inf; NaN in `want` is not compared.  `groups`: {key: mask broadcastable to want}, default
+    image_groups (maps); region_groups(x) for input gradients."""
+    got, want = _f64(got), _f64(want)
+    assert got.shape == want.shape, (got.shape, want.shape)
+    if groups is None:
+        groups = image_groups(want.shape)
+    over = want.abs() >= _FMT16[dtype][2]
+    fin = torch.isfinite(want) & ~over
+    out = {}
+    for key, m in groups.items():
+        m = m.expand_as(want)
+        if not m.any():
+            continue
+        o = m & over
+        if o.any() and not torch.equal(got[o], torch.sign(want[o]) * math.inf):
+            out[key] = math.inf
+            continue
+        f = m & fin
+        if not f.any():
+            out[key] = 0.0
+            continue
+        w, g = want[f], got[f]
+        if not torch.isfinite(g).all():
+            out[key] = math.inf
+            continue
+        S = w.abs().max().item()
+        bound = 0.5 * ulp(dtype, w) * (1 + 2.0 ** -7) + tau * S
+        out[key] = ((g - w).abs() / bound).max().item()
+    return out
+
+
+def rounding_err(got, want, dtype, tau, groups=None):
+    """max of rounding_errs (0.0 when nothing is compared)."""
+    return max(rounding_errs(got, want, dtype, tau, groups).values(), default=0.0)
+
+
+def rn_mismatches(got, want, dtype, tau):
+    """Elements of `got` (a bf16 / fp16 value, widened) that differ from round_nearest(want), other than where `want`
+    lies within tau S (S = max |want| of the image) of a half-way point and `got` is one of the two neighbours:
+    the count of elements a kernel that evaluates in fp32 and rounds once cannot produce."""
+    got, want = _f64(got), _f64(want)
+    q = ulp(dtype, want)
+    lo = torch.floor(want / q) * q
+    S = want.abs().flatten(1).amax(1).view(-1, *([1] * (want.dim() - 1)))
+    near_tie = (want - (lo + 0.5 * q)).abs() <= tau * S
+    ok = (got == round_nearest(dtype, want)) | (near_tie & ((got == lo) | (got == lo + q)))
+    return int((~ok).sum())
+
+
 def worst(errs, k=4):
     """The k largest entries of a grad_errs() table, for assertion messages."""
     return sorted(errs.items(), key=lambda kv: -kv[1])[:k]

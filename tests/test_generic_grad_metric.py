@@ -221,7 +221,7 @@ def _expected_launches(measure, op):
 
 def test_grid_reaches_generic_pairs():
     """Every (measure, geometry, op, dtype) cell of the GPU grid takes generic/pairs, with the expected launch count
-    and a workspace that holds the 5 pair coefficients (backward) and the map (pooled)."""
+    and a workspace that holds the 5 pair coefficients (backward) and the map (pooled), fp32 for either dtype."""
     wrong = []
     ops = (_capi.OP_FORWARD, _capi.OP_BACKWARD, _capi.OP_POOL_FORWARD, _capi.OP_POOL_BACKWARD)
     for m, g in G.GRID:
@@ -237,9 +237,8 @@ def test_grid_reaches_generic_pairs():
             for op in ops:
                 if op >= _capi.OP_POOL_FORWARD and not any(o == "pooled" for o, _, _ in G.runs(m, g)):
                     continue
-                esz = 4 if dt == F32 else 2
-                need = {_capi.OP_FORWARD: 0, _capi.OP_BACKWARD: 20 * npairs, _capi.OP_POOL_FORWARD: esz * npairs,
-                        _capi.OP_POOL_BACKWARD: 4 * npairs + 20 * npairs}[op]   # fp32 map gradient
+                need = {_capi.OP_FORWARD: 0, _capi.OP_BACKWARD: 20 * npairs, _capi.OP_POOL_FORWARD: 4 * npairs,
+                        _capi.OP_POOL_BACKWARD: 4 * npairs + 20 * npairs}[op]   # fp32 map, fp32 map gradient
                 got = (_capi.describe_path(desc, op), _capi.launch_count(desc, op), _capi.workspace_bytes(desc, op))
                 if got[0] != "generic/pairs" or got[1] != _expected_launches(m, op) or got[2] < need:
                     wrong.append((m, G.geom_id(g), op, dt, got))
