@@ -39,10 +39,8 @@
  *     errors, a positive cudaError_t for CUDA failures.  No C++ exception
  *     crosses the boundary.  nfpb200_status_string() renders either.
  *   - re-entrant and thread-safe: no global mutable state besides one-time
- *     cudaFuncSetAttribute calls, the (atomic) diagnostics pointer of
- *     nfpb200_debug_phase_timing, and the NFPB200_* tuning environment variables
- *     (INTEGRATION.md section 5), which are read ONCE, at the first launch that
- *     consults them, and never change behaviour afterwards.
+ *     cudaFuncSetAttribute calls and the (atomic) diagnostics pointer of
+ *     nfpb200_debug_phase_timing.
  *   - sm_100a only.  There is no CPU path in this library.
  */
 #ifndef NFP_B200_H_

@@ -23,8 +23,6 @@
 //           forward = table + forward (2 launches); backward = table + coef + apply (3 launches, x re-read from L2).
 // The window radius is a template parameter: all tap / offset loops are unrolled and the per-thread arrays live in
 // registers.
-#include <stdlib.h>
-
 #include <utility>
 
 #include "nfp_common.cuh"
@@ -689,18 +687,13 @@ inline int gcd_i(int a, int b) { return b ? gcd_i(b, a % b) : a; }
 // halo rows are re-read and their norms recomputed by the neighbouring CTAs: (TH + 2A) / TH of the work)
 BandPlan fused_plan(const KParams& P, int esz) {
   BandPlan bp{false, 0, 0, 0, 0};
-  static const bool off = [] {
-    const char* e = getenv("NFPB200_PLANAR_SCALAR");
-    return e && e[0] == '1';
-  }();
-  if (off) return bp;
   const int rowB = P.W * esz;
   if (((size_t)P.H * rowB) % 16) return bp;  // every channel plane must start 16-byte aligned
   const int g = 16 / gcd_i(16, rowB);
   const int A = (P.R + g - 1) / g * g;
   const int Hg = (P.H + g - 1) / g * g;
   auto bytes = [&](int th) { return (size_t)P.C * (th + 2 * A) * rowB + 16 + (size_t)(th + 2 * A) * P.W * sizeof(float); };
-  static const int th_cap = [] { const char* e = getenv("NFPB200_PLANAR_TH"); return e ? atoi(e) : 8; }();
+  constexpr int th_cap = 8;  // band height before rounding to the row granule
   int TH = (th_cap + g - 1) / g * g;
   if (TH > Hg) TH = Hg;
   while (TH > g && bytes(TH) > kBandSmemMax) TH -= g;

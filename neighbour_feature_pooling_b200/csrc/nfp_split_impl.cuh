@@ -849,40 +849,33 @@ int max_clusters(K kern, int S, size_t smem, int dev) {
   return n;
 }
 
-inline int env_int(const char* name, int dflt) {
-  const char* e = getenv(name);
-  return e ? atoi(e) : dflt;
-}
-
 template <typename T, class C, int MODE>
 Plan plan_for(const KParams& P) {
   Plan best{false, 0, 0, 0, 0, 0, 0, 0};
   constexpr int esz = (int)sizeof(T);
   constexpr bool bwd = (MODE == MODE_BWD || MODE == MODE_POOL_BWD);
   constexpr int item = 2 * C::CPW;  // work item: a pair of channel groups
-  static const int target_bytes = env_int("NFPB200_UNIT_BYTES", 25 * 1024 + 512);
-  static const int want_sub = env_int("NFPB200_SUBCHUNKS", 4);
-  static const int force_s = env_int("NFPB200_CLUSTER", 0);
-  static const int want_lanech = env_int("NFPB200_PASSB_LANECH", 1);
+  constexpr int target_bytes = 25 * 1024 + 512;  // unit size
+  constexpr int want_sub = 4;
+  static_assert(want_sub <= kMaxSub, "sub-chunk barriers");
   if (((size_t)C::K * C::P * esz) % 16) return best;
   long best_cost = -1;
   for (int S = 1; S <= kMaxS; ++S) {
-    if (force_s && S != force_s) continue;
     if (P.C % S) continue;
     const int Cs = P.C / S;
     if (Cs % item) continue;
     const long bytes = (long)Cs * C::P * esz;
     if (bytes % 16) continue;
     if (((size_t)item * C::P * esz) % 16) continue;  // TMA bulk store granularity of the strip form
-    const int lanech = (bwd && C::LANECH && want_lanech && Cs % C::TASK == 0) ? 1 : 0;
+    const int lanech = (bwd && C::LANECH && Cs % C::TASK == 0) ? 1 : 0;
     Lay<T, C, MODE, kNW> L(Cs, lanech != 0);
     if (L.total > kSmemPerSM - 1024) continue;
     long cost = bytes > target_bytes ? 2 * (bytes - target_bytes) : (target_bytes - bytes);
-    if (bwd && C::LANECH && want_lanech && !lanech) cost += 16 * 1024;
+    if (bwd && C::LANECH && !lanech) cost += 16 * 1024;
     if (best_cost >= 0 && cost >= best_cost) continue;
     // sub-chunks: as close to `want_sub` as the channel count allows (whole work items, 16-byte multiples)
     int nsub = 0;
-    for (int n = want_sub < kMaxSub ? want_sub : kMaxSub; n >= 1; --n) {
+    for (int n = want_sub; n >= 1; --n) {
       if (Cs % n) continue;
       const int sc = Cs / n;
       if (sc % item) continue;
@@ -931,10 +924,7 @@ int launch_mode(const KParams& P, SplitArgs a, cudaStream_t stream) {
   }
   const Tables<C>* gt = tables_for<C>(a.pad_mode);
   if (!gt) return NFPB200_EINVAL;
-  static const int use_pdl = env_int("NFPB200_PDL", 1);
-  static const int cap_clusters = env_int("NFPB200_MAX_CLUSTERS", 0);
   int G = max_clusters(kern, pl.S, pl.smem, dev);
-  if (cap_clusters > 0 && G > cap_clusters) G = cap_clusters;
   if (G > P.B) G = P.B;
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3((unsigned)(G * pl.S));
@@ -950,11 +940,9 @@ int launch_mode(const KParams& P, SplitArgs a, cudaStream_t stream) {
     attr[na].val.clusterDim.z = 1;
     ++na;
   }
-  if (use_pdl) {
-    attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[na].val.programmaticStreamSerializationAllowed = 1;
-    ++na;
-  }
+  attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[na].val.programmaticStreamSerializationAllowed = 1;
+  ++na;
   cfg.attrs = attr;
   cfg.numAttrs = na;
   cudaError_t lrc = cudaLaunchKernelEx(&cfg, kern, a, gt);

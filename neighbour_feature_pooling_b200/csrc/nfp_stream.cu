@@ -1,8 +1,5 @@
 // Dispatcher of the streaming fused NFP kernels: geometry check, dtype selection, entry points used
 // by the C ABI (nfp_capi.cu).  The kernels themselves live in nfp_stream_impl.cuh.
-#include <stdlib.h>
-#include <string.h>
-
 #include "nfp_split.h"
 #include "nfp_stream.h"
 
@@ -26,14 +23,10 @@ int op_mode(int op) {
   }
 }
 
-// the cluster-split kernels (nfp_split_impl.cuh) take every problem their planner accepts; the one-CTA-per-image
-// ring kernels (nfp_stream_impl.cuh) remain for the rest and for A/B runs (NFPB200_FUSED_IMPL=stream)
+// the one-CTA-per-image ring kernels (nfp_stream_impl.cuh) serve every fused problem; the cluster-split kernels
+// (nfp_split_impl.cuh) only NFPB200_PATH_SPLIT, and only the problems their planner accepts
 bool split_ok(const KParams& P, int dtype, int mode) {
-  static const bool want_split = [] {
-    const char* e = getenv("NFPB200_FUSED_IMPL");
-    return e && strcmp(e, "split") == 0;
-  }();
-  if (!want_split && !P.force_split) return false;
+  if (!P.force_split) return false;
   if (P.rin) return false;  // multi-radius launches: ring kernels only
   switch (dtype) {
     case NFPB200_F32: return split::plan_f32(P, mode).ok;
@@ -73,9 +66,9 @@ bool stream_supported(const KParams& P, int dtype, int measure, int op) {
   if (!geometry_ok(P, measure)) return false;
   const int mode = op_mode(op);
   if (dtype == NFPB200_F16) {
-    // the ring kernels serve fp16 exactly where they serve bf16 (same element size, same plans); a problem the
-    // cluster-split kernels would take for bf16 (NFPB200_PATH_SPLIT, NFPB200_FUSED_IMPL=split) is not served
-    return !P.force_split && !split_ok(P, NFPB200_BF16, mode) && stream::plan_ok_f16(P, mode);
+    // the ring kernels serve fp16 exactly where they serve bf16 (same element size, same plans); the cluster-split
+    // kernels carry no fp16 instantiation, so NFPB200_PATH_SPLIT is not served
+    return !P.force_split && stream::plan_ok_f16(P, mode);
   }
   if (split_ok(P, dtype, mode)) return true;
   if (P.force_split) return false;
@@ -110,9 +103,9 @@ int stream_pool_forward(const KParams& P, int dtype, const void* x, float* gap_x
   a.x = x; a.gap_x = gap_x; a.gap_nfp = gap_nfp;
   return run(P, dtype, stream::MODE_POOL_FWD, a, ctx.stream);
 }
-// fused nfp_pooling head on the ring kernels (the cluster-split experiment does not carry it)
+// fused nfp_pooling head on the ring kernels (the cluster-split kernels do not carry it)
 bool stream_head_supported(const KParams& P, int dtype, int measure, int op) {
-  return stream_supported(P, dtype, measure, op) && !split_ok(P, dtype, op_mode(op)) && P.K % 4 == 0;
+  return stream_supported(P, dtype, measure, op) && !P.force_split && P.K % 4 == 0;
 }
 int stream_head_forward(const KParams& P, int dtype, const void* x, const float* proj_w, const float* proj_b, float* out,
                         float* gap_x, float* gap_nfp, const LaunchCtx& ctx) {

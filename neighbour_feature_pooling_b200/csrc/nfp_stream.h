@@ -33,8 +33,6 @@ struct StreamArgs {
   int pad_mode, similarity;
   int lanech;    // backward: lane-per-channel pass B (C a multiple of 64, chunks a whole number of 64-channel tasks)
   int x_early;   // backward: x is stable across the preceding launch -> stream it before griddepcontrol.wait
-  int nsm;       // SMs of the device: CTAs with blockIdx >= nsm are the second CTA of their SM
-  int y_delay_ns, y_stages;  // experiment knobs for those second CTAs (NFPB200_Y_DELAY_NS / NFPB200_Y_STAGES)
   int y_f32;     // forward: y is fp32 regardless of T
   int bdirect;   // backward: per-lane partial tables (no shuffle tree over the channel slots), see Smem
   int gy_bufs;   // backward: upstream-gradient buffers in shared memory (1 when every CTA handles a single image)

@@ -227,16 +227,8 @@ __global__ void __launch_bounds__(block_threads(MODE, NW), C::MINB) stream_kerne
         grid_launch_dependents();
       }
       int slot = 0, img = 0;
-      uint32_t phbits = 0;  // per-slot phase parity (the number of active stages may differ between the passes)
+      uint32_t phbits = 0;  // per-slot phase parity (every pass restarts at slot 0)
       const int npass = (BWD && !resident) ? 2 : 1;
-      // second CTA of an SM (blockIdx >= number of SMs): optionally starts later and streams pass A through fewer
-      // stages, so the SM's first CTA gets the larger share of the SM's load bandwidth and the two run out of phase
-      const bool second = (int)blockIdx.x >= a.nsm;
-      const int nactA = (second && !resident && a.y_stages > 0 && a.y_stages < nst) ? a.y_stages : nst;
-      if (second && a.y_delay_ns > 0) {
-        const unsigned long long t0 = globaltimer_ns();
-        while (globaltimer_ns() - t0 < (unsigned long long)a.y_delay_ns) {}
-      }
       auto load_grads = [&](int b, int img) {
         if (MODE == MODE_BWD) {
           const int par = img & 1;
@@ -261,10 +253,9 @@ __global__ void __launch_bounds__(block_threads(MODE, NW), C::MINB) stream_kerne
         int issued = 0;
         for (int pass = 0; pass < npass; ++pass) {
           const unsigned char* src = xb;
-          const int nact = pass == 0 ? nactA : nst;
           slot = 0;
           for (int ch = 0; ch < NCH; ++ch, src += chunk_bytes, ++issued) {
-            if (dep_pending && issued == nactA) {  // the ring is full of the first image's x: now wait, then its gradients
+            if (dep_pending && issued == nst) {  // the ring is full of the first image's x: now wait, then its gradients
               grid_dependency_wait();
               grid_launch_dependents();
               dep_pending = false;
@@ -274,7 +265,7 @@ __global__ void __launch_bounds__(block_threads(MODE, NW), C::MINB) stream_kerne
             mbar_expect_tx(&full[slot], chunk_bytes);
             bulk_g2s(ring + slot * L.slot_stride, src, chunk_bytes, &full[slot]);
             phbits ^= 1u << slot;
-            if (++slot == nact) slot = 0;
+            if (++slot == nst) slot = 0;
           }
         }
         if (dep_pending) {  // fewer chunks than ring stages
@@ -323,8 +314,6 @@ __global__ void __launch_bounds__(block_threads(MODE, NW), C::MINB) stream_kerne
 
   int slot = 0, img = 0;
   uint32_t phbits = 0;  // per-slot phase parity, in step with the producer's
-  const bool second = (int)blockIdx.x >= a.nsm;
-  const int nactA = (second && !resident && a.y_stages > 0 && a.y_stages < nst) ? a.y_stages : nst;
   NFP_STAMP(0);  // consumers ready
   for (int b = blockIdx.x; b < a.B; b += gridDim.x, ++img) {
     const uint32_t phbits0 = phbits;
@@ -509,7 +498,7 @@ __global__ void __launch_bounds__(block_threads(MODE, NW), C::MINB) stream_kerne
             if (lane == 0) mbar_arrive(&empty[slot]);
           }
           phbits ^= 1u << slot;
-          if (++slot == nactA) slot = 0;
+          if (++slot == nst) slot = 0;
         }
 #pragma unroll
         for (int j = 0; j < TW; ++j)
@@ -572,7 +561,7 @@ __global__ void __launch_bounds__(block_threads(MODE, NW), C::MINB) stream_kerne
             if (lane == 0) mbar_arrive(&empty[slot]);
           }
           phbits ^= 1u << slot;
-          if (++slot == nactA) slot = 0;
+          if (++slot == nst) slot = 0;
         }
       }
       if constexpr (NFP_DBG_SKIP_TAIL && !BWD) {
@@ -1067,28 +1056,19 @@ struct Plan {
   size_t smem;
 };
 
-inline int env_int(const char* name, int dflt) {
-  const char* e = getenv(name);
-  return e ? atoi(e) : dflt;
-}
-
 template <typename T, class C, int MODE>
 Plan plan_for(const KParams& P, int num_sms = 148) {
   Plan pl{false, 0, 0, 0, 0, 0, 0, 2, 0, 0};
   constexpr int esz = (int)sizeof(T);
   constexpr bool bwd = (MODE == MODE_BWD || MODE == MODE_POOL_BWD);
-  static const int target_bytes = env_int("NFPB200_CHUNK_BYTES", 16 * 1024);
-  static const int want_ctas = env_int("NFPB200_CTAS_PER_SM", C::MINB);
-  static const int force_stream = env_int("NFPB200_NO_RESIDENT", 0);
+  constexpr int target_bytes = 16 * 1024;  // chunk size
   constexpr int pair = 2 * C::CPW;  // work item: a pair of channel groups
   if (((size_t)pair * C::P * esz) % 16) return pl;   // TMA bulk store / load granularity
   if (((size_t)C::K * C::P * esz) % 16) return pl;
   if (P.Kin && (C::R < 2 || ((size_t)P.Kin * C::P * esz) % 16)) return pl;  // multi-radius: the blocks of gy are bulk-copied
   if (P.C % pair) return pl;
   // backward of the full-row-strip 3x3 shapes: lane-per-channel pass B when C is a whole number of 64-channel tasks
-  // (NFPB200_PASSB_LANECH=0 keeps the strip form for A/B runs)
-  static const int want_lanech = env_int("NFPB200_PASSB_LANECH", 1);
-  pl.lanech = (bwd && C::LANECH && want_lanech && P.C % C::TASK == 0) ? 1 : 0;
+  pl.lanech = (bwd && C::LANECH && P.C % C::TASK == 0) ? 1 : 0;
   // chunk: the largest CC <= target that divides C and is a whole number of group pairs (of tasks)
   const int step = pl.lanech ? C::TASK : pair;
   int best = 0;
@@ -1101,18 +1081,14 @@ Plan plan_for(const KParams& P, int num_sms = 148) {
   if (!best) return pl;
   pl.CC = best;
   pl.NCH = P.C / best;
-  const int max_ctas = want_ctas < 1 ? 1 : (want_ctas > C::MINB ? C::MINB : want_ctas);
-  static const int want_whole = env_int("NFPB200_RESIDENT_IMAGE", 1);
-  for (int ctas = max_ctas; ctas >= 1 && !pl.ok; --ctas) {
+  for (int ctas = C::MINB; ctas >= 1 && !pl.ok; --ctas) {
     // one image per CTA (the whole batch fits the resident CTAs): a single upstream-gradient buffer suffices
     const int gy_bufs = (bwd && P.B <= num_sms * ctas) ? 1 : 2;
     const int budget = (kSmemPerSM + 1024) / ctas - 1024 - 256;  // 228 KB per SM, 1 KB reserved per CTA; 256 B slack
-    static const int max_stages = env_int("NFPB200_MAX_STAGES", 5);  // measured: 4-5 stages beat 6-8 at B = 256
-    int first = max_stages < kMaxStages ? max_stages : kMaxStages;
+    int first = 5;  // measured: 4-5 stages beat 6-8 at B = 256
     // one image per CTA, lane-per-channel pass B: per-lane partial tables (no shuffle tree, one publish round) with the
-    // image streamed twice, instead of the resident image with the two-round publish (NFPB200_BWD_DIRECT=0: off)
-    static const int want_bdirect = env_int("NFPB200_BWD_DIRECT", 1);
-    if (Smem<T, C, MODE, kNW>::BDIRECT_OK && want_bdirect && pl.lanech && gy_bufs == 1 && !force_stream) {
+    // image streamed twice, instead of the resident image with the two-round publish
+    if (Smem<T, C, MODE, kNW>::BDIRECT_OK && pl.lanech && gy_bufs == 1) {
       for (int nst = first; nst >= 3 && !pl.ok; --nst) {
         Smem<T, C, MODE, kNW> L(pl.CC, nst, P.C, P.Kin, pl.lanech, gy_bufs, 1);
         if (L.total > budget) continue;
@@ -1128,7 +1104,7 @@ Plan plan_for(const KParams& P, int num_sms = 148) {
     // backward with the lane-per-channel pass B: if the WHOLE image fits (512x7x7 fp32: 8 slots, 98 KB), keep it -- a
     // warp owns a whole chunk in pass B, so with fewer slots than chunks the last warps wait for a slot to drain and
     // for its refill (an L2 round trip) before they can start
-    if (pl.lanech && want_whole && !force_stream && pl.NCH <= kMaxStages && pl.NCH > first) {
+    if (pl.lanech && pl.NCH <= kMaxStages && pl.NCH > first) {
       Smem<T, C, MODE, kNW> L(pl.CC, pl.NCH, P.C, P.Kin, pl.lanech, gy_bufs);
       if (L.total <= budget) first = pl.NCH;
     }
@@ -1144,7 +1120,7 @@ Plan plan_for(const KParams& P, int num_sms = 148) {
     }
   }
   if (!pl.ok) return pl;
-  pl.resident = (bwd && !force_stream && pl.NCH <= pl.nst) ? 1 : 0;
+  pl.resident = (bwd && pl.NCH <= pl.nst) ? 1 : 0;
   return pl;
 }
 
@@ -1177,16 +1153,10 @@ int launch_mode(const KParams& P, StreamArgs a, cudaStream_t stream) {
   a.nst = pl.nst;
   a.resident = pl.resident;
   a.lanech = pl.lanech;
-  static const int y_delay = env_int("NFPB200_Y_DELAY_NS", 0);
-  static const int y_stages = env_int("NFPB200_Y_STAGES", 0);
-  a.y_delay_ns = y_delay;
-  a.y_stages = y_stages;
-  a.nsm = num_sms;
   const Tables<C>* gt = tables_for<C>(a.pad_mode);
   if (!gt) return NFPB200_EINVAL;
   const int slots = num_sms * pl.ctas_per_sm;
   const int grid = P.B < slots ? P.B : slots;
-  static const int use_pdl = env_int("NFPB200_PDL", 1);
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3((unsigned)grid);
   cfg.blockDim = dim3(block_threads(MODE, kNW));
@@ -1196,7 +1166,7 @@ int launch_mode(const KParams& P, StreamArgs a, cudaStream_t stream) {
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = use_pdl ? 1 : 0;
+  cfg.numAttrs = 1;
   cudaError_t lrc = cudaLaunchKernelEx(&cfg, kern, a, gt);
   if (lrc != cudaSuccess && getenv("NFPB200_VERBOSE")) {
     cudaFuncAttributes fa{};

@@ -28,7 +28,6 @@
 // Bit-reproducible: every sum has a fixed order.  fp32 channels-last inputs are not covered (TF32 would break the 1e-5
 // parity bound): the host side repacks those to NCHW.
 #include <stdio.h>
-#include <stdlib.h>
 
 #include <type_traits>
 
@@ -728,9 +727,8 @@ Plan plan_for(const KParams& P) {
   if (P.C % 64 || P.C < 64) return pl;             // swizzle granule: 8 chunks of 8 channels
   if ((C::K * C::P * 2) % 16) return pl;           // upstream-gradient rows are fetched with 16-byte copies
   if (P.Kin && (C::R < 2 || (P.Kin * C::P * 2) % 16)) return pl;  // multi-radius: both gradient blocks
-  static const int want_two = [] { const char* e = getenv("NFPB200_TOKEN_TWO_CTAS"); return e ? atoi(e) : 1; }();
   // two 8-warp CTAs per SM (one image buffer each) when they fit and there is more than one image per SM to overlap
-  if (want_two && plan_try<C, MODE, kNWSmall>(P, 1, kSmemPerSM / 2 - 1024, pl)) {
+  if (plan_try<C, MODE, kNWSmall>(P, 1, kSmemPerSM / 2 - 1024, pl)) {
     pl.ctas = 2;
     return pl;
   }

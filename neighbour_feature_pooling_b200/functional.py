@@ -16,7 +16,6 @@ CPU tensors are rejected (except the constructor-time shape probes described in
 from __future__ import annotations
 
 import ctypes
-import os
 import math
 from dataclasses import dataclass, replace
 
@@ -114,10 +113,9 @@ def _trace(desc, op, what):
         PATH_TRACE.add(f"{_capi.describe_path(desc, op)} {_DTYPE_NAMES[desc.dtype]} "
                        f"{'channels-last' if desc.layout else 'nchw'} {what}")
 
-# NFPB200_HINT_X_STABLE (include/nfp_b200.h) is opt-in: it pays only when the backward directly follows another fused NFP
-# launch on the stream (-1.9 us per backward in such chains); after any other kernel -- the normal case inside a network --
-# there is nothing to overlap and the reordered prologue costs ~0.9 us.  NFPB200_X_STABLE_HINT=1 switches it on.
-_X_STABLE_HINT = os.environ.get("NFPB200_X_STABLE_HINT", "0") == "1"
+# The backward passes here never set NFPB200_HINT_X_STABLE (include/nfp_b200.h): it pays only when the backward directly
+# follows another fused NFP launch on the stream (-1.9 us per backward in such chains); after any other kernel -- the
+# normal case inside a network -- there is nothing to overlap and the reordered prologue costs ~0.9 us.
 
 
 def _prepare(x: torch.Tensor, cfg: NFPConfig = None, ops=MAP_OPS):
@@ -262,10 +260,6 @@ class _NFPSimilarity(torch.autograd.Function):
     def backward(ctx, gy):
         (x,) = ctx.saved_tensors
         desc = _desc_for(x, ctx.cfg, ctx.layout)
-        # x is a saved forward activation: the launch that precedes this one on the stream did not write it, so the
-        # hint would be valid here; see _X_STABLE_HINT for why it is opt-in
-        if _X_STABLE_HINT:
-            desc.path |= _capi.HINT_X_STABLE
         gy = gy.to(x.dtype).contiguous()
         if gy.data_ptr() % 16:
             gy = gy.clone()
@@ -301,10 +295,6 @@ class _NFPGapPair(torch.autograd.Function):
     def backward(ctx, g_gap_x, g_gap_nfp):
         (x,) = ctx.saved_tensors
         desc = _desc_for(x, ctx.cfg, ctx.layout)
-        # x is a saved forward activation: the launch that precedes this one on the stream did not write it, so the
-        # hint would be valid here; see _X_STABLE_HINT for why it is opt-in
-        if _X_STABLE_HINT:
-            desc.path |= _capi.HINT_X_STABLE
         g_gap_x = g_gap_x.float().contiguous()
         g_gap_nfp = g_gap_nfp.float().contiguous()
         gx = _empty_like_layout(x, ctx.layout)
@@ -340,8 +330,6 @@ class _NFPPooledMap(torch.autograd.Function):
     def backward(ctx, g_gap_nfp):
         (x,) = ctx.saved_tensors
         desc = _desc_for(x, ctx.cfg, ctx.layout)
-        if _X_STABLE_HINT:
-            desc.path |= _capi.HINT_X_STABLE
         g_gap_nfp = g_gap_nfp.float().contiguous()   # fp32 whatever the dtype of x
         gx = _empty_like_layout(x, ctx.layout)
         with torch.cuda.device(x.device):
@@ -386,8 +374,6 @@ class _NFPHead(torch.autograd.Function):
     def backward(ctx, g_out):
         x, w, bvec, gap_x, gap_nfp = ctx.saved_tensors
         desc = _desc_for(x, ctx.cfg, ctx.layout)
-        if _X_STABLE_HINT:
-            desc.path |= _capi.HINT_X_STABLE
         g_out = g_out.float().contiguous()
         gx = _empty_like_layout(x, ctx.layout)
         with torch.cuda.device(x.device):
@@ -450,8 +436,6 @@ class _NFPMultiRadius(torch.autograd.Function):
         (x,) = ctx.saved_tensors
         desc = _desc_for(x, ctx.cfg, ctx.layout)
         desc.inner_R = ctx.inner_R
-        if _X_STABLE_HINT:
-            desc.path |= _capi.HINT_X_STABLE
         gy = gy.to(x.dtype).contiguous()
         if gy.data_ptr() % 16:
             gy = gy.clone()

@@ -5,11 +5,8 @@ fp16 is served by the NCHW streaming-ring kernels ("fused/stream_*") and the cha
 NFPB200_EUNSUPPORTED (-5) and the Python side widens it to fp32."""
 import ctypes
 import itertools
-import json
 import os
 import re
-import subprocess
-import sys
 
 import pytest
 import torch
@@ -151,27 +148,6 @@ def test_f16_y_f32_flag_is_accepted_where_bf16_is():
     for s in SHAPES["ring"][:2] + SHAPES["token"][:2]:
         for dt in (_capi.BF16, _capi.F16):
             assert _query(_desc(dt, s, yf32=True), _capi.OP_FORWARD)[0] == 0
-
-
-_SPLIT_SCRIPT = r"""
-import json, sys
-sys.path.insert(0, sys.argv[1])
-import test_f16_host as T
-t = T.routing_table()
-served = T.check_routing(t)
-split = sum(1 for qb, qh, _, _ in t.values() if qb[0] == 0 and qb[1].startswith("fused/split_"))
-print(json.dumps({"served": served, "split": split}))
-"""
-
-
-def test_f16_under_split_selection():
-    """NFPB200_FUSED_IMPL=split sends bf16 ring problems to the cluster-split kernels: those are -5 for fp16."""
-    env = dict(os.environ, NFPB200_FUSED_IMPL="split")
-    r = subprocess.run([sys.executable, "-c", _SPLIT_SCRIPT, os.path.dirname(os.path.abspath(__file__))],
-                       capture_output=True, text=True, env=env, cwd=ROOT, timeout=600)
-    assert r.returncode == 0, r.stderr
-    got = json.loads(r.stdout.strip().splitlines()[-1])
-    assert got["split"] > 0 and got["served"] > 0, got
 
 
 # ---- _prepare: keep fp16 when the caller's ops take it, widen otherwise ------------------------------------------------

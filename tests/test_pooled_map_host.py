@@ -4,7 +4,6 @@ import copy
 import ctypes
 import io
 import math
-import os
 import pickle
 
 import pytest
@@ -36,12 +35,11 @@ def _rc(d, op):
 
 
 def _partials_floor(d):
-    """B * n_bands * K * 4 bytes: the band partials.  A band has at most round_up(cap, g) rows, cap = NFPB200_PLANAR_TH
-    (default 8) and g the row granule that keeps each bulk copy 16-byte aligned (fused_plan), so
-    n_bands >= ceil(H / round_up(cap, g))."""
+    """B * n_bands * K * 4 bytes: the band partials.  A band has at most round_up(cap, g) rows, cap = 8 and g the row
+    granule that keeps each bulk copy 16-byte aligned (fused_plan), so n_bands >= ceil(H / round_up(cap, g))."""
     K = (2 * d.R + 1) ** 2 - 1
     g = 16 // math.gcd(16, d.W * (2 if d.dtype == _capi.BF16 else 4))
-    th_max = max(-(-int(os.environ.get("NFPB200_PLANAR_TH", "8")) // g) * g, g)
+    th_max = -(-8 // g) * g
     return d.B * -(-d.H // th_max) * K * 4
 
 
