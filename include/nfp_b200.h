@@ -15,6 +15,8 @@
  *   nfpb200_pooled_map_forward  <- adaptive_avg_pool2d(NFPPooling(x), (1, 1)).view(B, -1): every stage of
  *                             MobileNetV3_MultiStageNFP   (models/texture_pooling.py:249-256)
  *   nfpb200_pooled_map_backward <- autograd through those lines
+ *   nfpb200_jvp / nfpb200_backward_backward <- forward-mode AD and double backward through the cosine
+ *                             forward (F.cosine_similarity, nfp.py:150-159), see "second order" below
  *   nfpb200_output_shape   <- Conv2d output-size rule behind NFPPooling.output_size
  *                                                           (nfp.py:125-130, 42-47)
  *   nfpb200_desc_t         <- the constructor arguments     (nfp.py:16-18); inner_R: the two NFP layers of
@@ -130,7 +132,10 @@ enum {
   NFPB200_OP_POOL_FORWARD = 2,
   NFPB200_OP_POOL_BACKWARD = 3,
   NFPB200_OP_POOLED_MAP_FORWARD = 4,  /* ABI v4 */
-  NFPB200_OP_POOLED_MAP_BACKWARD = 5  /* ABI v4 */
+  NFPB200_OP_POOLED_MAP_BACKWARD = 5, /* ABI v4 */
+  /* 6 is not an op (ABI v5 callers have been told so) */
+  NFPB200_OP_JVP = 7,                 /* nfpb200_jvp */
+  NFPB200_OP_BACKWARD_BACKWARD = 8    /* nfpb200_backward_backward */
 };
 
 /* error codes (negative); positive return values are cudaError_t */
@@ -265,6 +270,35 @@ int nfpb200_head_forward(const nfpb200_desc_t* desc, const void* x, const float*
 /* gx = d loss / dx given g_out = d loss / d out (B, C) fp32 and the forward's gap_x / gap_nfp. */
 int nfpb200_head_backward(const nfpb200_desc_t* desc, const void* x, const float* proj_w, const float* proj_b,
                           const float* gap_x, const float* gap_nfp, const float* g_out, void* gx, void* stream);
+
+/* ---- second order of the cosine measure ----------------------------------------------------------------------
+ * What autograd needs past the first derivative: the reference is plain ATen (one-hot convs + F.cosine_similarity),
+ * so a model trained on it may differentiate NFP twice (gradient penalties, input-gradient regularisation, Hessian-vector
+ * products) or run it under torch.autograd.forward_ad.  Two entry points cover both:
+ *   nfpb200_jvp                ydot (B, K, H', W') = the directional derivative of NFP(x) along v (B, C, H, W);
+ *   nfpb200_backward_backward  gx2 (B, C, H, W) = d<v, gx(x, gy)>/dx, gx = nfpb200_backward's result.
+ * The rest of the double backward, d<v, gx>/d gy, is nfpb200_jvp(x, v, NFPB200_JVP_REVERSE).
+ * ATen's cosine_similarity clamps each norm at eps in place, outside autograd: the norm takes the value max(||x||, eps)
+ * but differentiates as ||x||.  Reverse mode therefore keeps the norm's derivative below eps (NFPB200_JVP_REVERSE, and
+ * the backward of the backward), while forward AD gives a clamped norm a zero tangent (NFPB200_JVP_FORWARD_AD).  The
+ * backward of the backward is NaN in every channel of an all-zero pixel and reaches ~1e12 at pixels below eps, as ATen's.
+ * Cosine measure, NCHW and inner_R = 0 only (NFPB200_EUNSUPPORTED otherwise: the caller folds an inner_R gradient onto
+ * the outer taps and repacks NHWC to NCHW); any radius, stride, dilation, padding and padding mode; x, v, gy in the
+ * descriptor's dtype (fp32, bf16, fp16), fp32 arithmetic, results rounded once to nearest.  One path each, whatever
+ * desc->path selects ("second/jvp": 1 launch; "second/pairs": 2 launches, a pair kernel writing 6 fp32 coefficients per
+ * (output pixel, tap) to the workspace and a gather kernel writing gx2).  No atomics: bit-identical from run to run. */
+enum { NFPB200_JVP_FORWARD_AD = 0, NFPB200_JVP_REVERSE = 1 };
+
+/* ydot = J v by `rule` (NFPB200_JVP_*; EINVAL otherwise).  ydot is in desc->dtype, or fp32 with NFPB200_FLAG_Y_F32 and a
+ * bf16 / fp16 x.  No workspace is needed (nfpb200_workspace_bytes reports 0).
+ * Alignment: x, v, ydot, workspace 16 bytes. */
+int nfpb200_jvp(const nfpb200_desc_t* desc, const void* x, const void* v, void* ydot, int32_t rule,
+                void* workspace, size_t workspace_bytes, void* stream);
+
+/* gx2 (B, C, H, W) = d<v, gx(x, gy)>/dx ; gy (B, K, H', W') and v (B, C, H, W) in desc->dtype, gx2 in desc->dtype.
+ * Alignment: x, gy, v, gx2, workspace 16 bytes. */
+int nfpb200_backward_backward(const nfpb200_desc_t* desc, const void* x, const void* gy, const void* v, void* gx2,
+                              void* workspace, size_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }

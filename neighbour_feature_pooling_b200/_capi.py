@@ -30,6 +30,8 @@ HINT_X_STABLE = 0x100   # NFPB200_HINT_X_STABLE, OR-ed into Desc.path for the ba
 FLAG_Y_F32 = 0x200      # NFPB200_FLAG_Y_F32, OR-ed into Desc.path for nfpb200_forward with bf16 / fp16 x: y is fp32
 OP_FORWARD, OP_BACKWARD, OP_POOL_FORWARD, OP_POOL_BACKWARD = 0, 1, 2, 3
 OP_POOLED_MAP_FORWARD, OP_POOLED_MAP_BACKWARD = 4, 5   # GAP(NFP(x)) alone (ABI v4)
+OP_JVP, OP_BACKWARD_BACKWARD = 7, 8                   # second order of the cosine measure (6 is not an op)
+JVP_FORWARD_AD, JVP_REVERSE = 0, 1                    # nfpb200_jvp rule: forward AD / the map nfpb200_backward transposes
 LAYOUT_NCHW, LAYOUT_NHWC = 0, 1
 
 EXPORTS = (
@@ -37,7 +39,7 @@ EXPORTS = (
     "nfpb200_workspace_bytes", "nfpb200_describe_path", "nfpb200_launch_count",
     "nfpb200_forward", "nfpb200_backward", "nfpb200_pool_forward", "nfpb200_pool_backward",
     "nfpb200_debug_phase_timing", "nfpb200_head_supported", "nfpb200_head_forward", "nfpb200_head_backward",
-    "nfpb200_pooled_map_forward", "nfpb200_pooled_map_backward",
+    "nfpb200_pooled_map_forward", "nfpb200_pooled_map_backward", "nfpb200_jvp", "nfpb200_backward_backward",
 )
 
 
@@ -111,6 +113,10 @@ def load():
         lib.nfpb200_pooled_map_forward.argtypes = [dp, vp, vp, vp, ctypes.c_size_t, vp]
         lib.nfpb200_pooled_map_backward.restype = ctypes.c_int
         lib.nfpb200_pooled_map_backward.argtypes = [dp, vp, vp, vp, vp, ctypes.c_size_t, vp]
+        lib.nfpb200_jvp.restype = ctypes.c_int
+        lib.nfpb200_jvp.argtypes = [dp, vp, vp, vp, ctypes.c_int32, vp, ctypes.c_size_t, vp]
+        lib.nfpb200_backward_backward.restype = ctypes.c_int
+        lib.nfpb200_backward_backward.argtypes = [dp, vp, vp, vp, vp, vp, ctypes.c_size_t, vp]
         got = lib.nfpb200_abi_version()
         if got != ABI_VERSION:
             raise RuntimeError(f"libnfp_b200.so ABI version {got}, host code expects {ABI_VERSION}; rebuild")

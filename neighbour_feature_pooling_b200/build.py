@@ -22,7 +22,7 @@ LIB_DIR = os.path.join(PKG_DIR, "lib")
 LIB_PATH = os.path.join(LIB_DIR, "libnfp_b200.so")
 OBJ_DIR = os.path.join(PKG_DIR, "build")
 SOURCES = ["nfp_capi.cu", "nfp_generic.cu", "nfp_stream.cu", "nfp_stream_f32.cu", "nfp_stream_bf16.cu", "nfp_stream_f16.cu",
-           "nfp_split_f32.cu", "nfp_split_bf16.cu", "nfp_planar.cu", "nfp_token.cu"]
+           "nfp_split_f32.cu", "nfp_split_bf16.cu", "nfp_planar.cu", "nfp_token.cu", "nfp_second.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xptxas", "-v", "-I", INCLUDE, "-I", CSRC,

@@ -71,6 +71,15 @@ inline int pool_op_of(int op) {
                                               : (op == NFPB200_OP_POOLED_MAP_BACKWARD ? NFPB200_OP_POOL_BACKWARD : op);
 }
 inline size_t align256(size_t b) { return (b + 255) & ~(size_t)255; }
+inline bool second_op(int op) { return op == NFPB200_OP_JVP || op == NFPB200_OP_BACKWARD_BACKWARD; }
+inline bool valid_op(int op) { return (op >= NFPB200_OP_FORWARD && op <= NFPB200_OP_POOLED_MAP_BACKWARD) || second_op(op); }
+constexpr int kPathSecond = 5;
+
+// The second-order ops have one path each (nfp_second.cu), whatever desc->path asks for: cosine, NCHW, single radius.
+int second_path(const nfpb200_desc_t* d, const KParams& P) {
+  if (d->measure != NFPB200_COSINE || P.layout != NFPB200_LAYOUT_NCHW || P.rin) return NFPB200_EUNSUPPORTED;
+  return kPathSecond;
+}
 
 // fp16 is served by two kernel families only, the ones the live heads use: the NCHW streaming-ring kernels (2) and the
 // channels-last token kernels (4), for every op they carry, on exactly the problems a bf16 descriptor sends to them.
@@ -89,6 +98,7 @@ int choose_path_f16(const nfpb200_desc_t* d, const KParams& P, int op) {
 
 // 4 = token (channels-last), 3 = planar, 2 = fused (cluster-split or streaming-ring kernels), 0 = generic, <0 = error
 int choose_path(const nfpb200_desc_t* d, const KParams& P, int op) {
+  if (second_op(op)) return second_path(d, P);
   if (d->dtype == NFPB200_F16) return choose_path_f16(d, P, op);
   if (pooled_map_op(op)) {
     // the pool ops' choice (token, ring, generic; inner_R refused), with the row-band kernels' pooled mode taking the
@@ -122,6 +132,7 @@ int choose_path(const nfpb200_desc_t* d, const KParams& P, int op) {
 size_t path_workspace_bytes(int path, const nfpb200_desc_t* d, const KParams& P, int op) {
   // pooled-map ops on the ring / token kernels: their GAP(x) output (forward) or zero g_gap_x input (backward), (B, C) fp32
   if (pooled_map_op(op) && (path == 2 || path == 4)) return align256((size_t)P.B * P.C * sizeof(float));
+  if (path == kPathSecond) return second_workspace_bytes(P, op);
   if (path == 3) return planar_workspace_bytes(P, d->dtype, op);
   if (path == 4) return 0;
   return path ? 0 : generic_workspace_bytes(P, d->dtype, d->measure, op);
@@ -182,7 +193,7 @@ int nfpb200_workspace_bytes(const nfpb200_desc_t* desc, int32_t op, size_t* byte
   KParams P;
   int rc = make_params(desc, &P);
   if (rc) return rc;
-  if (!bytes || op < NFPB200_OP_FORWARD || op > NFPB200_OP_POOLED_MAP_BACKWARD) return NFPB200_EINVAL;
+  if (!bytes || !valid_op(op)) return NFPB200_EINVAL;
   int path = choose_path(desc, P, op);
   if (path < 0) return path;
   *bytes = path_workspace_bytes(path, desc, P, op);
@@ -193,11 +204,12 @@ int nfpb200_describe_path(const nfpb200_desc_t* desc, int32_t op, char* buf, siz
   KParams P;
   int rc = make_params(desc, &P);
   if (rc) return rc;
-  if (!buf || buf_bytes == 0 || op < NFPB200_OP_FORWARD || op > NFPB200_OP_POOLED_MAP_BACKWARD) return NFPB200_EINVAL;
+  if (!buf || buf_bytes == 0 || !valid_op(op)) return NFPB200_EINVAL;
   int path = choose_path(desc, P, op);
   if (path < 0) return path;
   snprintf(buf, buf_bytes, "%s",
-           path == 4 ? token_name(P) : path == 3 ? planar_name(P, desc->dtype, op)
+           path == kPathSecond ? (op == NFPB200_OP_JVP ? "second/jvp" : "second/pairs")
+           : path == 4 ? token_name(P) : path == 3 ? planar_name(P, desc->dtype, op)
                      : (path == 2 ? stream_name(P, desc->dtype, desc->measure, pool_op_of(op)) : "generic/pairs"));
   return NFPB200_OK;
 }
@@ -206,10 +218,11 @@ int nfpb200_launch_count(const nfpb200_desc_t* desc, int32_t op, int32_t* launch
   KParams P;
   int rc = make_params(desc, &P);
   if (rc) return rc;
-  if (!launches || op < NFPB200_OP_FORWARD || op > NFPB200_OP_POOLED_MAP_BACKWARD) return NFPB200_EINVAL;
+  if (!launches || !valid_op(op)) return NFPB200_EINVAL;
   int path = choose_path(desc, P, op);
   if (path < 0) return path;
-  if (path == 3) *launches = planar_launch_count(P, desc->dtype, op);
+  if (path == kPathSecond) *launches = op == NFPB200_OP_JVP ? 1 : 2;
+  else if (path == 3) *launches = planar_launch_count(P, desc->dtype, op);
   else if (path == 2 || path == 4) *launches = op == NFPB200_OP_POOLED_MAP_BACKWARD ? 2 : 1;   // + the g_gap_x memset
   else *launches = generic_launch_count(P, desc->dtype, desc->measure, op);
   return NFPB200_OK;
@@ -364,6 +377,24 @@ int nfpb200_head_backward(const nfpb200_desc_t* desc, const void* x, const float
     return token_head_run(P, desc->dtype, NFPB200_OP_POOL_BACKWARD, x, proj_w, proj_b, nullptr, const_cast<float*>(gap_x),
                           const_cast<float*>(gap_nfp), g_out, gx, ctx);
   return stream_head_backward(P, desc->dtype, x, proj_w, proj_b, gap_x, gap_nfp, g_out, gx, ctx);
+}
+
+// ---- second order of the cosine measure --------------------------------------------------------------------------
+int nfpb200_jvp(const nfpb200_desc_t* desc, const void* x, const void* v, void* ydot, int32_t rule, void* workspace,
+                size_t workspace_bytes, void* stream) {
+  if (!x || !v || !ydot) return NFPB200_EINVAL;
+  if (misaligned(x) || misaligned(v) || misaligned(ydot) || misaligned(workspace)) return NFPB200_EALIGN;
+  if (rule != NFPB200_JVP_FORWARD_AD && rule != NFPB200_JVP_REVERSE) return NFPB200_EINVAL;
+  NFP_PROLOGUE(NFPB200_OP_JVP)
+  return second_jvp(P, desc->dtype, x, v, ydot, rule, ctx);
+}
+
+int nfpb200_backward_backward(const nfpb200_desc_t* desc, const void* x, const void* gy, const void* v, void* gx2,
+                              void* workspace, size_t workspace_bytes, void* stream) {
+  if (!x || !gy || !v || !gx2) return NFPB200_EINVAL;
+  if (misaligned(x) || misaligned(gy) || misaligned(v) || misaligned(gx2) || misaligned(workspace)) return NFPB200_EALIGN;
+  NFP_PROLOGUE(NFPB200_OP_BACKWARD_BACKWARD)
+  return second_backward_backward(P, desc->dtype, x, gy, v, gx2, ctx);
 }
 
 }  // extern "C"

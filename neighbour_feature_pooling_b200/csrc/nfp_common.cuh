@@ -60,6 +60,27 @@ __host__ __device__ __forceinline__ void tap_rc(int t, int k, int K, int& a, int
   b = tt - a * k;
 }
 
+// Every padded coordinate p (frame: i*stride + a*dil - pad) that the padding rule maps onto source coordinate r.
+template <class F>
+__device__ __forceinline__ void for_each_preimage(int r, int n, int pad, int mode, F f) {
+  f(r);
+  switch (mode) {
+    case NFPB200_PAD_REFLECT:
+      if (r >= 1 && r <= pad) f(-r);
+      if (r <= n - 2 && n - 1 - r <= pad) f(2 * (n - 1) - r);
+      break;
+    case NFPB200_PAD_REPLICATE:
+      if (r == 0) for (int p = -pad; p < 0; ++p) f(p);
+      if (r == n - 1) for (int p = n; p < n + pad; ++p) f(p);
+      break;
+    case NFPB200_PAD_CIRCULAR:
+      if (r - n >= -pad) f(r - n);
+      if (r + n <= n - 1 + pad) f(r + n);
+      break;
+    default: break;
+  }
+}
+
 template <typename T> __device__ __forceinline__ float to_f32(T v);
 template <> __device__ __forceinline__ float to_f32<float>(float v) { return v; }
 template <> __device__ __forceinline__ float to_f32<__nv_bfloat16>(__nv_bfloat16 v) { return __bfloat162float(v); }
@@ -131,5 +152,11 @@ int planar_backward(const KParams& P, int dtype, const void* x, const void* gy, 
 int planar_pooled_forward(const KParams& P, int dtype, const void* x, float* gap_nfp, const LaunchCtx& ctx);
 int planar_pooled_backward(const KParams& P, int dtype, const void* x, const float* g_gap_nfp, void* gx,
                            const LaunchCtx& ctx);
+
+// second-order kernels of the cosine measure (JVP, backward of the backward; NCHW, any geometry): nfp_second.cu
+size_t second_workspace_bytes(const KParams& P, int op);
+int second_jvp(const KParams& P, int dtype, const void* x, const void* v, void* ydot, int rule, const LaunchCtx& ctx);
+int second_backward_backward(const KParams& P, int dtype, const void* x, const void* gy, const void* v, void* gx2,
+                             const LaunchCtx& ctx);
 
 }  // namespace nfp

@@ -452,27 +452,6 @@ __global__ void __launch_bounds__(kThreads) scs_coef_kernel_b(float* __restrict_
   coef[2 * npairs + idx] = nn > 0.f ? gden * (nc + P.q) / nn : 0.f;
 }
 
-// Every padded coordinate p (frame: i*stride + a*dil - pad) that the padding rule maps onto source coordinate r.
-template <class F>
-__device__ __forceinline__ void for_each_preimage(int r, int n, int pad, int mode, F f) {
-  f(r);
-  switch (mode) {
-    case NFPB200_PAD_REFLECT:
-      if (r >= 1 && r <= pad) f(-r);
-      if (r <= n - 2 && n - 1 - r <= pad) f(2 * (n - 1) - r);
-      break;
-    case NFPB200_PAD_REPLICATE:
-      if (r == 0) for (int p = -pad; p < 0; ++p) f(p);
-      if (r == n - 1) for (int p = n; p < n + pad; ++p) f(p);
-      break;
-    case NFPB200_PAD_CIRCULAR:
-      if (r - n >= -pad) f(r - n);
-      if (r + n <= n - 1 + pad) f(r + n);
-      break;
-    default: break;
-  }
-}
-
 // Gather form of the backward: one thread per (b, channel, INPUT pixel q) collects, in a fixed order, every
 // contribution that lands on q -- as a neighbour tap of an output pixel (d/dn) and as the centre of an output pixel
 // (sum over its taps of d/dc) -- through the inverse of the padding / stride / dilation index map.  No atomics:

@@ -231,6 +231,118 @@ def _stream(device) -> int:
     return torch.cuda.current_stream(device).cuda_stream
 
 
+# ---- second order (cosine measure) -------------------------------------------------------------------------------
+# Every Function below differentiates once through its own C-ABI call.  Past that, for the cosine measure:
+#  * backward under create_graph=True builds its input gradient from _NFPBackward (today's nfpb200_backward, itself
+#    differentiable through nfpb200_backward_backward and nfpb200_jvp) and torch ops, so the gradient can be
+#    differentiated again (gradient penalties, double backward, Hessian-vector products);
+#  * jvp (torch.autograd.forward_ad) is nfpb200_jvp by the forward-AD rule.
+# With create_graph=False the backward issues exactly its first-order call.  Other measures raise on a second derivative.
+_once = torch.autograd.function.once_differentiable
+
+
+def _second_order(cfg) -> bool:
+    """True when this backward must build a differentiable graph and the measure has second-order kernels."""
+    return torch.is_grad_enabled() and cfg.measure == "cosine"
+
+
+def _nchw(t: torch.Tensor) -> torch.Tensor:
+    """t as a contiguous NCHW tensor at a 16-byte aligned address (the second-order kernels' layout)."""
+    t = t.contiguous()
+    return t.clone() if t.data_ptr() % 16 else t
+
+
+def _jvp(x: torch.Tensor, v: torch.Tensor, cfg: NFPConfig, rule: int, y_f32: bool = False) -> torch.Tensor:
+    """d NFP(x) along v (B, K, H', W') by `rule` (_capi.JVP_*): nfpb200_jvp.  fp32 for bf16 / fp16 x when y_f32."""
+    x = _nchw(x)
+    v = _nchw(v.to(x.dtype))
+    desc = _desc_for(x, cfg)
+    y_f32 = y_f32 and x.dtype != torch.float32
+    if y_f32:
+        desc.path |= _capi.FLAG_Y_F32
+    Ho, Wo = _capi.output_shape(desc)
+    yd = torch.empty((x.shape[0], cfg.out_channels, Ho, Wo), dtype=torch.float32 if y_f32 else x.dtype,
+                     device=x.device)
+    with torch.cuda.device(x.device):
+        rc = _capi.load().nfpb200_jvp(ctypes.byref(desc), x.data_ptr(), v.data_ptr(), yd.data_ptr(), rule, None, 0,
+                                      _stream(x.device))
+    _capi.check(rc, "nfpb200_jvp")
+    return yd
+
+
+def _backward_backward(x: torch.Tensor, gy: torch.Tensor, v: torch.Tensor, cfg: NFPConfig) -> torch.Tensor:
+    """d<v, gx(x, gy)>/dx (B, C, H, W) NCHW in the dtype of x: nfpb200_backward_backward."""
+    x = _nchw(x)
+    gy, v = _nchw(gy.to(x.dtype)), _nchw(v.to(x.dtype))
+    desc = _desc_for(x, cfg)
+    gx2 = torch.empty_like(x)
+    with torch.cuda.device(x.device):
+        ws, ws_ptr, ws_n = _workspace(desc, _capi.OP_BACKWARD_BACKWARD, x.device)
+        rc = _capi.load().nfpb200_backward_backward(ctypes.byref(desc), x.data_ptr(), gy.data_ptr(), v.data_ptr(),
+                                                    gx2.data_ptr(), ws_ptr, ws_n, _stream(x.device))
+    _capi.check(rc, "nfpb200_backward_backward")
+    return gx2
+
+
+class _NFPBackward(torch.autograd.Function):
+    """gx = nfpb200_backward(x, gy) as a function of (x, gy) that autograd differentiates once more (cosine measure).
+    Its backward is (nfpb200_backward_backward(x, gy, v), nfpb200_jvp(x, v, reverse rule)); a channels-last x is
+    copied to NCHW for those two calls."""
+
+    @staticmethod
+    def forward(ctx, x, gy, cfg, layout):
+        desc = _desc_for(x, cfg, layout)
+        gyk = gy.clone() if gy.data_ptr() % 16 else gy
+        gx = _empty_like_layout(x, layout)
+        with torch.cuda.device(x.device):
+            ws, ws_ptr, ws_n = _workspace(desc, _capi.OP_BACKWARD, x.device)
+            rc = _capi.load().nfpb200_backward(ctypes.byref(desc), x.data_ptr(), gyk.data_ptr(), gx.data_ptr(),
+                                               ws_ptr, ws_n, _stream(x.device))
+        _capi.check(rc, "nfpb200_backward")
+        ctx.save_for_backward(x, gy)
+        ctx.cfg = cfg
+        return gx
+
+    @staticmethod
+    @_once
+    def backward(ctx, v):
+        x, gy = ctx.saved_tensors
+        x = _nchw(x)
+        gx2 = _backward_backward(x, gy, v, ctx.cfg) if ctx.needs_input_grad[0] else None
+        ggy = _jvp(x, v, ctx.cfg, _capi.JVP_REVERSE) if ctx.needs_input_grad[1] else None
+        return gx2, ggy, None, None
+
+
+def _map_gx(x, gy, cfg, layout):
+    """Differentiable input gradient of the map for upstream gradient gy (B, K, H', W') of any dtype."""
+    return _NFPBackward.apply(x, gy.to(x.dtype).contiguous(), cfg, layout)
+
+
+def _pooled_gx(x, g_gap_x, g_gap_nfp, cfg, layout):
+    """Differentiable d(<g_gap_x, GAP(x)> + <g_gap_nfp, GAP(NFP(x))>)/dx: the map gradient is g_gap_nfp / (H' W')
+    expanded over the map, the GAP(x) gradient g_gap_x / (H W) over the input (g_gap_x None: no GAP(x) term)."""
+    B, C, H, W = x.shape
+    Ho, Wo = conv_output_size(H, cfg), conv_output_size(W, cfg)
+    gy = (g_gap_nfp.float() / (Ho * Wo))[:, :, None, None].expand(B, cfg.out_channels, Ho, Wo)
+    gx = _map_gx(x, gy, cfg, layout)
+    if g_gap_x is not None:
+        gx = (gx + (g_gap_x.float() / (H * W))[:, :, None, None]).to(x.dtype)
+    return gx
+
+
+def _inner_taps(R: int, r: int):
+    """The radius-R tap number of each tap of the radius-r window (both row-major, centre removed; nfp_common.cuh
+    inner_tap): y_r = y_R[:, _inner_taps(R, r)] when both layers pad by their radius."""
+    k, k1 = 2 * R + 1, 2 * r + 1
+    out = []
+    for o1 in range(k1 * k1):
+        if o1 == k1 * k1 // 2:
+            continue
+        o = (o1 // k1 - r + R) * k + (o1 % k1 - r + R)
+        out.append(o if o < k * k // 2 else o - 1)
+    return out
+
+
 class _NFPSimilarity(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, cfg, y_f32=False, layout=0):
@@ -251,13 +363,27 @@ class _NFPSimilarity(torch.autograd.Function):
                                               _stream(x.device))
         _capi.check(rc, "nfpb200_forward")
         ctx.save_for_backward(x)
+        ctx.save_for_forward(x)
         ctx.cfg = cfg
         ctx.layout = layout
+        ctx.y_f32 = y_f32
         return y
 
     @staticmethod
-    @torch.autograd.function.once_differentiable
+    def jvp(ctx, x_t, *_):
+        (x,) = ctx.saved_tensors
+        return _jvp(x, x_t, ctx.cfg, _capi.JVP_FORWARD_AD, ctx.y_f32)
+
+    @staticmethod
     def backward(ctx, gy):
+        if _second_order(ctx.cfg):
+            (x,) = ctx.saved_tensors
+            return _map_gx(x, gy, ctx.cfg, ctx.layout), None, None, None
+        return _NFPSimilarity._backward(ctx, gy)
+
+    @staticmethod
+    @_once
+    def _backward(ctx, gy):
         (x,) = ctx.saved_tensors
         desc = _desc_for(x, ctx.cfg, ctx.layout)
         gy = gy.to(x.dtype).contiguous()
@@ -286,13 +412,26 @@ class _NFPGapPair(torch.autograd.Function):
                                                    gap_nfp.data_ptr(), ws_ptr, ws_n, _stream(x.device))
         _capi.check(rc, "nfpb200_pool_forward")
         ctx.save_for_backward(x)
+        ctx.save_for_forward(x)
         ctx.cfg = cfg
         ctx.layout = layout
         return gap_x, gap_nfp
 
     @staticmethod
-    @torch.autograd.function.once_differentiable
+    def jvp(ctx, x_t, *_):
+        (x,) = ctx.saved_tensors
+        return x_t.float().mean((2, 3)), _jvp(x, x_t, ctx.cfg, _capi.JVP_FORWARD_AD, True).mean((2, 3))
+
+    @staticmethod
     def backward(ctx, g_gap_x, g_gap_nfp):
+        if _second_order(ctx.cfg):
+            (x,) = ctx.saved_tensors
+            return _pooled_gx(x, g_gap_x, g_gap_nfp, ctx.cfg, ctx.layout), None, None
+        return _NFPGapPair._backward(ctx, g_gap_x, g_gap_nfp)
+
+    @staticmethod
+    @_once
+    def _backward(ctx, g_gap_x, g_gap_nfp):
         (x,) = ctx.saved_tensors
         desc = _desc_for(x, ctx.cfg, ctx.layout)
         g_gap_x = g_gap_x.float().contiguous()
@@ -321,13 +460,26 @@ class _NFPPooledMap(torch.autograd.Function):
                                                          ws_ptr, ws_n, _stream(x.device))
         _capi.check(rc, "nfpb200_pooled_map_forward")
         ctx.save_for_backward(x)
+        ctx.save_for_forward(x)
         ctx.cfg = cfg
         ctx.layout = layout
         return gap_nfp
 
     @staticmethod
-    @torch.autograd.function.once_differentiable
+    def jvp(ctx, x_t, *_):
+        (x,) = ctx.saved_tensors
+        return _jvp(x, x_t, ctx.cfg, _capi.JVP_FORWARD_AD, True).mean((2, 3))
+
+    @staticmethod
     def backward(ctx, g_gap_nfp):
+        if _second_order(ctx.cfg):
+            (x,) = ctx.saved_tensors
+            return _pooled_gx(x, None, g_gap_nfp, ctx.cfg, ctx.layout), None, None
+        return _NFPPooledMap._backward(ctx, g_gap_nfp)
+
+    @staticmethod
+    @_once
+    def _backward(ctx, g_gap_nfp):
         (x,) = ctx.saved_tensors
         desc = _desc_for(x, ctx.cfg, ctx.layout)
         g_gap_nfp = g_gap_nfp.float().contiguous()   # fp32 whatever the dtype of x
@@ -362,7 +514,8 @@ class _NFPHead(torch.autograd.Function):
                                                    bvec.data_ptr() if bvec is not None else None, out.data_ptr(),
                                                    gap_x.data_ptr(), gap_nfp.data_ptr(), _stream(x.device))
         _capi.check(rc, "nfpb200_head_forward")
-        ctx.save_for_backward(x, w, bvec if bvec is not None else w.new_empty(0), gap_x, gap_nfp)
+        ctx.save_for_backward(x, w, bvec if bvec is not None else w.new_empty(0), gap_x, gap_nfp, weight, bias)
+        ctx.save_for_forward(x, w, bvec if bvec is not None else w.new_empty(0), gap_x, gap_nfp)
         ctx.cfg = cfg
         ctx.layout = layout
         ctx.has_bias = bias is not None
@@ -370,9 +523,46 @@ class _NFPHead(torch.autograd.Function):
         return out
 
     @staticmethod
-    @torch.autograd.function.once_differentiable
-    def backward(ctx, g_out):
+    def jvp(ctx, x_t, w_t, b_t, *_):
+        # product rule on out = gap_x * (W gap_nfp + b), with dual weight / bias
         x, w, bvec, gap_x, gap_nfp = ctx.saved_tensors
+        proj = gap_nfp @ w.t() + (bvec if ctx.has_bias else 0.0)
+        gap_x_t = x_t.float().mean((2, 3))
+        proj_t = _jvp(x, x_t, ctx.cfg, _capi.JVP_FORWARD_AD, True).mean((2, 3)) @ w.t()
+        if w_t is not None:
+            proj_t = proj_t + gap_nfp @ w_t.float().t()
+        if b_t is not None:
+            proj_t = proj_t + b_t.float()
+        return gap_x_t * proj + gap_x * proj_t
+
+    @staticmethod
+    def backward(ctx, g_out):
+        if _second_order(ctx.cfg):
+            return _NFPHead._backward_graph(ctx, g_out)
+        return _NFPHead._backward(ctx, g_out)
+
+    @staticmethod
+    def _backward_graph(ctx, g_out):
+        """The backward as differentiable pieces: gap_x and gap_nfp are recomputed (the saved ones are not outputs of
+        this Function, so they carry no graph), the projection is torch ops on the caller's weight and bias."""
+        x, weight, bias = ctx.saved_tensors[0], ctx.saved_tensors[5], ctx.saved_tensors[6]
+        g_out = g_out.float()
+        gap_x = x.float().mean((2, 3))
+        gap_nfp = _NFPPooledMap.apply(x, ctx.cfg, ctx.layout)
+        wf = weight.float()
+        proj = gap_nfp @ wf.t()
+        if ctx.has_bias:
+            proj = proj + bias.float()
+        t = g_out * gap_x
+        gx = _pooled_gx(x, g_out * proj, t @ wf, ctx.cfg, ctx.layout)
+        gw = (t.t() @ gap_nfp).to(ctx.param_dtypes[0]) if ctx.needs_input_grad[1] else None
+        gb = t.sum(0).to(ctx.param_dtypes[1]) if (ctx.has_bias and ctx.needs_input_grad[2]) else None
+        return gx, gw, gb, None, None
+
+    @staticmethod
+    @_once
+    def _backward(ctx, g_out):
+        x, w, bvec, gap_x, gap_nfp = ctx.saved_tensors[:5]
         desc = _desc_for(x, ctx.cfg, ctx.layout)
         g_out = g_out.float().contiguous()
         gx = _empty_like_layout(x, ctx.layout)
@@ -427,12 +617,31 @@ class _NFPMultiRadius(torch.autograd.Function):
                                               _stream(x.device))
         _capi.check(rc, "nfpb200_forward (multi-radius)")
         ctx.save_for_backward(x)
-        ctx.cfg, ctx.inner_R, ctx.layout = cfg, inner_R, layout
+        ctx.save_for_forward(x)
+        ctx.cfg, ctx.inner_R, ctx.layout, ctx.y_f32 = cfg, inner_R, layout, y_f32
         return y
 
     @staticmethod
-    @torch.autograd.function.once_differentiable
+    def jvp(ctx, x_t, *_):
+        # the outer map's tangent, and the inner map's as its inner taps
+        (x,) = ctx.saved_tensors
+        yd = _jvp(x, x_t, ctx.cfg, _capi.JVP_FORWARD_AD, ctx.y_f32)
+        return torch.cat([yd[:, _inner_taps(ctx.cfg.R, ctx.inner_R)], yd], dim=1)
+
+    @staticmethod
     def backward(ctx, gy):
+        if _second_order(ctx.cfg):
+            # fold the inner block onto the outer taps it equals (y_r = y_R[inner taps]), then one radius-R backward
+            (x,) = ctx.saved_tensors
+            k_in = len(_inner_taps(ctx.cfg.R, ctx.inner_R))
+            idx = torch.tensor(_inner_taps(ctx.cfg.R, ctx.inner_R), device=gy.device)
+            g = gy[:, k_in:].index_add(1, idx, gy[:, :k_in])
+            return _map_gx(x, g, ctx.cfg, ctx.layout), None, None, None, None
+        return _NFPMultiRadius._backward(ctx, gy)
+
+    @staticmethod
+    @_once
+    def _backward(ctx, gy):
         (x,) = ctx.saved_tensors
         desc = _desc_for(x, ctx.cfg, ctx.layout)
         desc.inner_R = ctx.inner_R
