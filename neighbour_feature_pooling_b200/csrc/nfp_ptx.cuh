@@ -47,6 +47,8 @@ __device__ __forceinline__ void bulk_s2g(void* dst, const void* src, uint32_t by
                "r"(bytes)
                : "memory");
 }
+// warm L2 with the line that holds the global address p: no data to the SM, nothing to wait for
+__device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 template <int N>
 __device__ __forceinline__ void bulk_wait_read() {

@@ -38,6 +38,7 @@ struct StreamArgs {
   int gy_bufs;   // backward: upstream-gradient buffers in shared memory (1 when every CTA handles a single image)
   int kin, rin;  // multi-radius launch (desc.inner_R): y / gy carry kin extra channels per image (the radius-rin map) in front
   int ggx_tma;   // pooled backward: g_gap_x rows are 16-byte aligned and sized -> fetched with one bulk copy per image
+  int pf_imgs;   // leading images per CTA whose inputs are prefetched into L2 before griddepcontrol.wait
   float eps;
   unsigned long long* dbg;  // optional: 8 globaltimer stamps per CTA (first image), see nfpb200_debug_phase_timing
 };

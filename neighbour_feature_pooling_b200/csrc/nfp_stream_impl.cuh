@@ -68,6 +68,10 @@
 #ifndef NFP_DBG_SKIP_EPI
 #define NFP_DBG_SKIP_EPI 0
 #endif
+// same-tree baseline for the L2 prefetch before the dependency wait (results are unchanged either way)
+#ifndef NFP_DBG_NO_L2_PREFETCH
+#define NFP_DBG_NO_L2_PREFETCH 0
+#endif
 
 namespace nfp {
 namespace stream {
@@ -85,6 +89,9 @@ __host__ __device__ constexpr int block_threads(int mode, int nw) {
 constexpr int kNW = 8;                  // consumer warps
 constexpr int kSmemPerSM = 227 * 1024;
 constexpr int kLeadPad = 128;           // zeroed bytes in front of the ring (halo reads of the first plane)
+// pause between two rounds of L2 prefetch lines (32 KB per CTA) before the dependency wait.  B200, 512x7x7 fp32 step
+// at 128 / 256 / 512 ns: 21.05 / 20.95 / 20.79 us, but 512 slows the 2x2 and the 7x7 bf16 maps
+constexpr unsigned kPrefetchPauseNs = 256;
 
 // Shared-memory layout (byte offsets).  Fixed regions first, then a union: the per-warp partial
 // tables of pass A are dead once the image's table is summed, the backward scratch / store staging
@@ -185,6 +192,7 @@ __global__ void __launch_bounds__(block_threads(MODE, NW), C::MINB) stream_kerne
   uint64_t* gyfull = empty + kMaxStages;
   uint64_t* gyempty = gyfull + 2;
   uint64_t* tabfull = gyempty + 2;
+  volatile uint32_t* dep_done = reinterpret_cast<volatile uint32_t*>(tabfull + 1);  // the producer's wait returned
   float* tfull = reinterpret_cast<float*>(smem_raw + L.tfull);
   float* inv = reinterpret_cast<float*>(smem_raw + L.inv);
   float* wtab = reinterpret_cast<float*>(smem_raw + L.wtab);
@@ -205,6 +213,7 @@ __global__ void __launch_bounds__(block_threads(MODE, NW), C::MINB) stream_kerne
       mbar_init(&gyempty[s], 1);
     }
     mbar_init(tabfull, 1);
+    *dep_done = 0u;
     fence_mbar_init();
   }
   __syncthreads();
@@ -224,6 +233,7 @@ __global__ void __launch_bounds__(block_threads(MODE, NW), C::MINB) stream_kerne
       bool dep_pending = BWD && a.x_early;
       if (!dep_pending) {
         grid_dependency_wait();
+        *dep_done = 1u;
         grid_launch_dependents();
       }
       int slot = 0, img = 0;
@@ -294,6 +304,39 @@ __global__ void __launch_bounds__(block_threads(MODE, NW), C::MINB) stream_kerne
     if (a.lanech) {  // no pads between the slots: one behind the last
       uint32_t* zp = reinterpret_cast<uint32_t*>(ring + nst * L.slot_stride);
       for (int i = tid; i < 32; i += NT) zp[i] = 0u;
+    }
+  }
+  // While the preceding grid still runs, warm L2 with the inputs of this CTA's first a.pf_imgs images, in the order
+  // they are consumed, so that their HBM stream overlaps that grid's tail.  A prefetch moves no data into the SM:
+  // everything this grid consumes is still read after griddepcontrol.wait, from L2 -- the point of coherence every
+  // write of the preceding grid goes through -- so the data consumed is the same, also when x or gy is an output of
+  // the preceding grid.  Every address is inside the caller's buffers.  The consumer threads issue one line each per
+  // round and pause between rounds; they stop as soon as the producer's wait has returned: from then on the ring
+  // loads stream the image in order, and prefetching further ahead would only make the first chunks land later (an
+  // unpaced prefetch of the whole image costs 0.6 us per fp32 launch after a non-NFP kernel, where nothing overlaps;
+  // a bulk prefetch from the producer, cp.async.bulk.prefetch.L2, queues ahead of the ring loads in the TMA unit and
+  // costs 1.4 us).  With the x-stable hint the producer streams x before its wait itself.
+  if (!NFP_DBG_NO_L2_PREFETCH && !(BWD && a.x_early)) {
+    bool stop = false;
+    auto prefetch_range = [&](const void* base, size_t bytes) {
+      const unsigned char* p = reinterpret_cast<const unsigned char*>(base);
+      for (size_t off = 0; off < bytes && !stop; off += (size_t)NT * 128) {
+        if (*dep_done) {
+          stop = true;
+          break;
+        }
+        if (off + (size_t)tid * 128 < bytes) prefetch_l2(p + off + (size_t)tid * 128);
+        if (tid == 0 && off + (size_t)NT * 128 >= bytes) prefetch_l2(p + bytes - 1);  // last line, base not 128-aligned
+        __nanosleep(kPrefetchPauseNs);
+      }
+    };
+    int n = 0;
+    for (int b = blockIdx.x; b < a.B && n < a.pf_imgs && !stop; b += gridDim.x, ++n) {
+      if (MODE == MODE_BWD)
+        prefetch_range(reinterpret_cast<const unsigned char*>(a.gy) + (size_t)b * (K + a.kin) * P * ESZ,
+                       (size_t)(K + a.kin) * P * ESZ);
+      if (MODE == MODE_POOL_BWD && a.g_gap_x) prefetch_range(a.g_gap_x + (size_t)b * a.C, (size_t)a.C * 4);
+      prefetch_range(reinterpret_cast<const unsigned char*>(a.x) + (size_t)b * a.C * P * ESZ, (size_t)a.C * P * ESZ);
     }
   }
   // PDL: nothing below may touch global memory the preceding grid still uses -- except, with the x-stable hint, the
@@ -1128,6 +1171,7 @@ template <typename T, class C, int MODE>
 int launch_mode(const KParams& P, StreamArgs a, cudaStream_t stream) {
   constexpr int kMaxDev = 64;
   static int sm_count[kMaxDev] = {0};
+  static int l2_bytes[kMaxDev] = {0};
   int dev = 0;
   cudaError_t e = cudaGetDevice(&dev);
   if (e != cudaSuccess) return (int)e;
@@ -1141,6 +1185,10 @@ int launch_mode(const KParams& P, StreamArgs a, cudaStream_t stream) {
     int n = 0;
     e = cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
     if (e != cudaSuccess) return (int)e;
+    int l2 = 0;
+    e = cudaDeviceGetAttribute(&l2, cudaDevAttrL2CacheSize, dev);
+    if (e != cudaSuccess) return (int)e;
+    l2_bytes[dev] = l2;
     sm_count[dev] = n;
   }
   const int num_sms = sm_count[dev];
@@ -1157,6 +1205,15 @@ int launch_mode(const KParams& P, StreamArgs a, cudaStream_t stream) {
   if (!gt) return NFPB200_EINVAL;
   const int slots = num_sms * pl.ctas_per_sm;
   const int grid = P.B < slots ? P.B : slots;
+  // L2 prefetch before the dependency wait (stream_kernel's consumer prologue): at most the leading images of every
+  // CTA whose inputs fit in half the L2 over the whole grid -- all of them at B = 256 on 512x7x7 -- so that a large
+  // batch does not flush the working set of the launch it overlaps
+  size_t pf_bytes = (size_t)P.C * C::P * sizeof(T);
+  if (MODE == MODE_BWD) pf_bytes += (size_t)(C::K + P.Kin) * C::P * sizeof(T);
+  if (MODE == MODE_POOL_BWD && a.g_gap_x) pf_bytes += (size_t)P.C * 4;
+  const size_t pf_fit = (size_t)l2_bytes[dev] / 2 / ((size_t)grid * pf_bytes);
+  const int per_cta = (P.B + grid - 1) / grid;
+  a.pf_imgs = pf_fit < (size_t)per_cta ? (int)pf_fit : per_cta;
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3((unsigned)grid);
   cfg.blockDim = dim3(block_threads(MODE, kNW));
